@@ -15,12 +15,14 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def golden():
-    """Vectors produced by the unmodified reference Numba code (oracle/make_golden.py)."""
-    z = np.load(os.path.join(ROOT, "tests", "golden", "reference_numba_golden.npz"))
+    """Vectors produced by the unmodified reference Numba code (oracle/make_golden.py); the c3 group is
+    stored in a file of its own to keep each file under 1 MB."""
     groups = {}
-    for key in z.files:
-        g, name = key.split("/")
-        groups.setdefault(g, {})[name] = z[key]
+    for f in ("reference_numba_golden.npz", "reference_numba_golden_c3.npz"):
+        z = np.load(os.path.join(ROOT, "tests", "golden", f))
+        for key in z.files:
+            g, name = key.split("/")
+            groups.setdefault(g, {})[name] = z[key]
     return groups
 
 

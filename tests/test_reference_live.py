@@ -1,45 +1,44 @@
-"""The UNMODIFIED reference Numba code, imported live (``/root/reference`` in the build container, the
-bytecode staged in ``oracle/_ref`` on the GPU box), as the checker:
+"""The outputs of the UNMODIFIED reference Numba code, stored in ``tests/golden`` by ``oracle/make_golden.py``,
+as the checker of a whole behaviour step.  The golden ``c3`` group was computed on
+``W.heterogeneous_boxes(2048, seed=W.SEED_BASE + 103)``: the workload is regenerated here, and the fixture
+checks that its inputs (previous velocities and step included, through the stored accelerations) are the
+stored ones bit for bit.  The reference's force and torque are its stored components through the behaviour
+tail (``hydro_oracle.numpy_tail``, hydrodynamics_behavior.py:212-224).
 
-  * CPU: the C restatement ``oracle/hydro_oracle.c`` against it on a fresh C3 sample (beyond the committed
-    golden vectors), the harness's vectorised geometry against real wrapper instances, and the staged
-    bytecode against the live tree;
-  * GPU (``-m gpu``): the CUDA path through the C ABI against it on >= 10^4 bodies, both precisions.
+  * CPU: the C restatement ``oracle/hydro_oracle.c`` stepped on that workload against them;
+  * GPU (``-m gpu``): the CUDA path through the C ABI against them, both precisions.
 """
-import os
-import subprocess
-import sys
-
 import numpy as np
 import pytest
 
-from oracle import ref_numba as R
 from silver2_isaacsim_b200 import workloads as W
 from tests import scoring
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-needs_ref = pytest.mark.skipif(not R.available(), reason="reference neither present nor staged (oracle/stage_reference.py)")
-
 
 @pytest.fixture(scope="module")
-def ref_step():
-    """(workload, force, torque, components, raised) of one behaviour step through the real reference."""
-    wl = W.heterogeneous_boxes(12_000, seed=W.SEED_BASE + 77)
-    # a few wet bodies at rest: the reference raises there (SURVEY.md A.8)
+def ref_step(golden):
+    """(workload, force, torque, components, raised) of one behaviour step of the reference."""
+    from oracle.hydro_oracle import COMPONENT_NAMES, numpy_tail
+
+    d = golden["c3"]
+    wl = W.heterogeneous_boxes(len(d["pos"]), seed=W.SEED_BASE + 103)
+    f8 = lambda a: a.astype(np.float64)
+    inputs = {"ctor": wl.ctor_rows(), "mass": wl.masses(), "pos": f8(wl.pos), "quat": f8(wl.quat_xyzw),
+              "v": f8(wl.lin_vel), "w": f8(wl.ang_vel), "a": (f8(wl.lin_vel) - f8(wl.prev_lin)) / wl.dt,
+              "al": (f8(wl.ang_vel) - f8(wl.prev_ang)) / wl.dt}
+    for k, x in inputs.items():
+        assert np.array_equal(x, d[k]), f"the regenerated workload's {k} is not what the golden c3 group stores"
+    comp = {name: d[name] for name in COMPONENT_NAMES + ("sub_ratio",)}
+    F, T, _ = numpy_tail(comp, d["pos"], d["mass"])
+    raised = d["raised"].copy()
+    # a few wet bodies at rest: the reference raises there (SURVEY.md A.8; golden edge case GV5 records it)
+    assert golden["edge"]["raised"][4] and not golden["edge"]["v"][4].any()
     wl.lin_vel[:3] = 0.0
     wl.pos[:3, 2] = -5.0
-    st = R.ReferenceStepper(wl.ctor_rows(), wl.masses())
-    F, T, comp, raised = st.step(wl.pos, wl.quat_xyzw, wl.lin_vel, wl.ang_vel, wl.prev_lin, wl.prev_ang, wl.dt)
+    raised[:3] = True
     return wl, F, T, comp, raised
 
 
-@needs_ref
-def test_harness_geometry_is_the_wrappers():
-    wl = W.heterogeneous_boxes(500, seed=5)
-    R.check_geometry(wl.ctor_rows(), sample=64)
-
-
-@needs_ref
 def test_c_oracle_against_the_live_reference(oracle, ref_step):
     wl, F, T, comp, raised = ref_step
     ref = oracle.step(wl.ctor_rows(), wl.masses(), wl.pos, wl.quat_xyzw, wl.lin_vel, wl.ang_vel, wl.prev_lin,
@@ -57,57 +56,7 @@ def test_c_oracle_against_the_live_reference(oracle, ref_step):
     assert np.abs(comp["sub_ratio"][ok] - ref.components["sub_ratio"][ok]).max() < 1e-12
 
 
-@needs_ref
-@pytest.mark.skipif(not (R.live_available() and R.staged_available()), reason="needs both the live tree and oracle/_ref")
-def test_staged_bytecode_equals_live_tree(tmp_path):
-    """oracle/_ref/*.pyc is the reference: same numbers, bit for bit, as importing /root/reference."""
-    code = (
-        "import sys, numpy as np; sys.path.insert(0, %r)\n"
-        "from oracle import ref_numba as R\n"
-        "from silver2_isaacsim_b200 import workloads as W\n"
-        "wl = W.heterogeneous_boxes(300, seed=9)\n"
-        "a = (wl.lin_vel.astype(np.float64) - wl.prev_lin) / wl.dt; al = (wl.ang_vel.astype(np.float64) - wl.prev_ang) / wl.dt\n"
-        "out, raised = R.components_via_wrapper(wl.ctor_rows(), wl.pos.astype(np.float64), wl.quat_xyzw.astype(np.float64),\n"
-        "                                       wl.lin_vel.astype(np.float64), wl.ang_vel.astype(np.float64), a, al)\n"
-        "np.save(sys.argv[1], out); print(R.source())\n" % ROOT)
-    outs = {}
-    for name, root in (("live", R.REFERENCE_ROOT), ("staged", "/nonexistent")):
-        env = dict(os.environ, H2O_REFERENCE_ROOT=root)
-        f = str(tmp_path / (name + ".npy"))
-        res = subprocess.run([sys.executable, "-c", code, f], env=env, capture_output=True, text=True, timeout=300)
-        assert res.returncode == 0, res.stderr[-1500:]
-        assert res.stdout.strip().endswith(name)
-        outs[name] = np.load(f)
-    assert outs["live"].tobytes() == outs["staged"].tobytes()
-
-
-def test_warp_fixture_is_what_the_reference_warp_source_computes(golden_warp):
-    """tests/golden/reference_warp_golden.npz == the reference's Warp kernel source run now (through the shim or a
-    real ``warp``), bit for bit on a sample of every group; N launches of dim 1 == one launch of dim N."""
-    from oracle import ref_warp
-
-    if not ref_warp.available():
-        pytest.skip("reference tree not present")
-    for g in ("c2", "c3", "edge"):
-        d = golden_warp[g]
-        sel = np.arange(len(d["pos"]))[:: max(1, len(d["pos"]) // 64)]
-        out, raised = ref_warp.components_via_wrapper(d["ctor"][sel], d["pos"][sel], d["quat"][sel], d["v"][sel],
-                                                      d["w"][sel], d["a"][sel], d["al"][sel])
-        assert (raised == d["raised"][sel]).all()
-        for name in ref_warp.NAMES:
-            if ref_warp.load()[3] == "shim":
-                assert out[name].tobytes() == d[name][sel].tobytes(), (g, name)
-            else:  # a real warp: same source, Warp's own float32 code generation
-                np.testing.assert_allclose(out[name], d[name][sel], rtol=3e-5, atol=1e-5)
-    d = golden_warp["batched"]
-    b = ref_warp.components_batched(d["ctor"], d["pos"][:96], d["quat"][:96], d["v"][:96], d["w"][:96], d["a"][:96],
-                                    d["al"][:96])
-    for name in ref_warp.NAMES:
-        np.testing.assert_allclose(b[name], d[name][:96], rtol=3e-5, atol=1e-5)
-
-
 # --------------------------------------------------------------------------------------------- GPU
-@needs_ref
 @pytest.mark.gpu
 @pytest.mark.parametrize("mode", ["fp32", "fp64"])
 def test_cuda_path_against_the_live_reference(ref_step, mode):
@@ -130,8 +79,8 @@ def test_cuda_path_against_the_live_reference(ref_step, mode):
     F, T = F.double().cpu().numpy(), T.double().cpu().numpy()
     ok = ~raised
     if mode == "fp32":
-        scoring.assert_fp32(F[ok], F_ref[ok], "force vs the live reference")
-        scoring.assert_fp32(T[ok], T_ref[ok], "torque vs the live reference")
+        scoring.assert_fp32(F[ok], F_ref[ok], "force vs the reference")
+        scoring.assert_fp32(T[ok], T_ref[ok], "torque vs the reference")
     else:
         scale = scoring.force_scale(wl.coeff_per_body(), wl.rho, wl.g)
         # 1e-11: the reference's own fastmath noise floor sits at ~1e-13 .. 2e-12 on barely wet bodies

@@ -6,7 +6,7 @@ for k in os.environ.get("KS", "1,0,1048576,65536,8192,1024,128,16,1").split(",")
     if k == "1" and "done1" in globals():
         k_env = "2"  # k = 1 means "never"; every body = every 2nd... use a dedicated value below
     env = dict(os.environ, H2O_NO_FALLBACK=k)
-    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "20", "--warmup", "5", "--no-cpu-baseline",
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1200", "--warmup", "5", "--no-cpu-baseline",
                           "--no-extra", "--no-e2e", "--regions", "60"], env=env, capture_output=True, text=True)
     d = json.loads(res.stdout.strip().splitlines()[-1])
     t = d["extra"]["timing"]
