@@ -7,7 +7,11 @@ both replayed from one captured CUDA graph of 100 steps.  After every replay one
 column order of the reference's LogVelocity behaviour (log_velocity.py:17-20), and the real-time
 factor is reported like its BenchmarkRtf (benchmark_rtf.py:37-71).
 
-    python examples/buoy_validation.py [--steps 6000] [--n 1] [--csv /tmp/buoy.csv]
+With --wave-amplitude > 0 the buoy floats in a regular deep-water wave of that amplitude and --wave-period,
+evaluated by the engine at the buoy on every step; the CSV then has one more column, the surface
+elevation at the buoy.
+
+    python examples/buoy_validation.py [--steps 6000] [--n 1] [--csv /tmp/buoy.csv] [--wave-amplitude 0.2 --wave-period 8]
 """
 import argparse
 import os
@@ -17,13 +21,15 @@ import numpy as np
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from silver2_isaacsim_b200 import HydroEngine, workloads as W      # noqa: E402
+from silver2_isaacsim_b200 import HydroEngine, waves, workloads as W  # noqa: E402
 from silver2_isaacsim_b200.trace import RtfMeter, VelocityTrace    # noqa: E402
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--steps", type=int, default=6000)
 ap.add_argument("--n", type=int, default=1, help="identical buoys stepped side by side")
 ap.add_argument("--csv", default="/tmp/buoy_velocity_log.csv")
+ap.add_argument("--wave-amplitude", type=float, default=0.0, help="regular deep-water wave amplitude (m); 0 = still water")
+ap.add_argument("--wave-period", type=float, default=8.0, help="wave period (s)")
 args = ap.parse_args()
 
 dev = torch.device("cuda:0")
@@ -35,15 +41,20 @@ rep = lambda a: torch.as_tensor(np.repeat(np.asarray(a, dtype=np.float64), args.
 pos, quat, v, w = rep(wl.pos), rep(wl.quat_xyzw), rep(wl.lin_vel), rep(wl.ang_vel)
 F, T = eng.bind(pos, quat, v, w)
 eng.set_rollout_mode(free_bodies=True, gravity=wl.g)   # every captured step: forces, then the stepper
+in_waves = args.wave_amplitude > 0
+if in_waves:
+    eng.set_wave_field(waves.regular(args.wave_amplitude, args.wave_period))
 
 GRAPH = 100
 eng.capture_rollout(GRAPH, wl.dt)
-trace, rtf = VelocityTrace(args.csv), RtfMeter(report_every=1000)
+trace = VelocityTrace(args.csv, extra_columns=("surface_elevation",) if in_waves else ())
+rtf = RtfMeter(report_every=1000)
 for k in range(args.steps // GRAPH):
     eng.launch_rollout()
     torch.cuda.synchronize()
     rtf.on_physics_step(wl.dt, GRAPH)
-    trace.sample(pos.cpu(), v.cpu(), w.cpu())           # one row per replayed graph
+    extra = (float(eng.sample_waves(pos[:1])[0, 0]),) if in_waves else ()   # elevation at the buoy, current clock
+    trace.sample(pos.cpu(), v.cpu(), w.cpu(), extra=extra)  # one row per replayed graph
 r = rtf.report()
 z = float(pos[0, 2])
 print(f"{args.n} buoy(s), {r['steps']} steps of {wl.dt * 1e3:.2f} ms: RTF {r['rtf']:.1f}x, {r['steps_per_s']:.0f} steps/s; "

@@ -106,6 +106,43 @@ H2O_API int h2o_set_added_mass_dense(h2o_handle h, int n_types, const double* ma
  * water surface (the reference's is the plane z = 0).  NULL / 0 = the reference's behaviour. */
 H2O_API int h2o_set_environment(h2o_handle h, const double current_xyz[3], double surface_z);
 
+/* Built-in linear (Airy) wave field (SURVEY.md 8(f4)), evaluated on the device at every body's centre on every
+ * step.  comps is n_components x 5 host doubles (a, kx, ky, omega, phase), depth the water depth h (+inf = deep
+ * water).  For component j, with k_j = |(kx_j, ky_j)|, at body position p and clock value t:
+ *   theta_j = kx_j p_x + ky_j p_y - omega_j t + phase_j                        (always float64)
+ *   elevation  eta = sum_j a_j cos theta_j: the body's p_z is measured against the waterline surface_z + eta
+ *              (+ eta[i] when a height field is also set, h2o_set_surface_heights)
+ *   orbital velocity at z = clamp(p_z - surface_z, -h, 0) (measured from the mean level):
+ *              u_h = sum_j a_j omega_j C_j(z) cos theta_j (kx_j, ky_j) / k_j,   u_z = sum_j a_j omega_j S_j(z) sin theta_j
+ *              finite depth: C_j = cosh(k_j (z + h)) / sinh(k_j h),  S_j = sinh(k_j (z + h)) / sinh(k_j h)
+ *              deep water:   C_j = S_j = exp(k_j z)
+ * The orbital velocity adds to the uniform current: drag, damping and lift see v - (current + u), formed
+ * exactly as the uniform current alone is.  As with the current: accelerations stay differences of BODY
+ * velocities, the carried previous velocity stays the body velocity, and no fluid-acceleration
+ * (Froude-Krylov inertia) term is added.
+ * Precision: fp64 mode evaluates everything in double.  fp32 mode keeps the phase in double and evaluates
+ * sine, cosine and the depth decay in float (field within 2e-6 of sum a_j resp. sum a_j omega_j).  eta enters
+ * the waterline as a double, like surface_z; current + u is summed in double, rounded once to the handle dtype
+ * and subtracted there.
+ * Clock: one double in engine-owned device memory.  Every step evaluates the field at the clock's value, then
+ * the clock advances by dt in stream order (no host synchronisation; also inside captured rollouts and the host
+ * pipeline); a step with dt <= 1e-6 leaves it alone.  h2o_rollout_persistent over K steps uses t, t + dt, ...
+ * and leaves the clock bit-identical to K single steps.  The clock starts at 0 and is kept when the field is
+ * replaced or removed.
+ * At most 64 components; n_components == 0 removes the field.  H2O_ERR_BAD_ARGUMENT for non-finite values,
+ * a < 0, omega <= 0, |k| == 0 or depth <= 0 (other than +inf).  The table is copied to engine-owned device
+ * memory.  Steps with a wave field run on the per-body kernel; h2o_components ignores the field (as it ignores
+ * a height field).  Like every h2o_set_* call this drops a captured rollout. */
+H2O_API int h2o_set_wave_field(h2o_handle h, int n_components, const double* comps, double depth);
+/* The wave clock, stream-ordered.  The read synchronises the stream.  Neither drops a captured rollout: the graph
+ * reads the clock from device memory, so a write between replays moves the field the replay sees. */
+H2O_API int h2o_wave_time_write(h2o_handle h, double t, h2o_stream stream);
+H2O_API int h2o_wave_time_read(h2o_handle h, double* t, h2o_stream stream);
+/* Evaluate the field at the clock's current value with the evaluator and precision policy of the step:
+ * points is a DEVICE array (m,3) in the handle dtype (world positions; the velocity depth is measured from
+ * surface_z), out a DEVICE array (m,4) float64 of rows [eta, ux, uy, uz] (zeros without a field). */
+H2O_API int h2o_wave_sample(h2o_handle h, const void* points, int64_t m, double* out, h2o_stream stream);
+
 /* Same twelve scalars, same order as the reference wrapper ctor
  * (numba_hydrodynamics_wrapper.py:9-10): width, depth, height, linear_drag_coefficient,
  * angular_drag_coefficient, linear_damping, angular_damping, water_density, gravity,

@@ -37,6 +37,7 @@ import torch
 
 from . import params as P
 from .engine import HydroEngine
+from .waves import WaveField
 
 
 class BatchedHydrodynamicsBehavior:
@@ -48,7 +49,7 @@ class BatchedHydrodynamicsBehavior:
     def __init__(self, prim_names: Sequence[str], view, device: str = "cuda:0",
                  config_path: Optional[str] = None, dtype: torch.dtype = torch.float32,
                  bodies_per_robot: int = 0, robot_offsets: Optional[Sequence[int]] = None,
-                 warp_compat: bool = False):
+                 warp_compat: bool = False, waves: Optional[WaveField] = None):
         self.prim_names = list(prim_names)
         self._view = view
         self._device = device
@@ -56,6 +57,7 @@ class BatchedHydrodynamicsBehavior:
         self._config_path = config_path
         self._bodies_per_robot = int(bodies_per_robot)
         self._warp_compat = bool(warp_compat)
+        self._waves = waves  # built-in wave field, installed by _setup with its clock at 0
         # robots of unequal size, e.g. [0, 19, 20] for one SILVER2 + the Obsea buoy (the main scene)
         self._robot_offsets = None if robot_offsets is None else [int(o) for o in robot_offsets]
         self._engine: Optional[HydroEngine] = None
@@ -110,6 +112,9 @@ class BatchedHydrodynamicsBehavior:
         self._engine.set_params_per_body(np.asarray(rows, dtype=np.float64))
         if self._warp_compat:
             self._engine.set_warp_compat(True)
+        if self._waves is not None:
+            self._engine.set_wave_field(self._waves)
+            self._engine.set_wave_time(0.0)
         if self._robot_offsets is not None:
             self._engine.set_articulation_offsets(self._robot_offsets)
         else:

@@ -76,6 +76,10 @@ struct h2o_engine {
     int32_t* am_slot_type = nullptr;
     int am_types = 0, am_slots = 0;
     const void* surface_eta = nullptr;  // (n,) per-body surface heights, borrowed, or nullptr = flat
+    double* wave_tab = nullptr;    // (MAX_WAVE_COMPONENTS, WAVE_STRIDE) wave table, first n_waves rows in use
+    double* wave_clock = nullptr;  // the wave field's clock (one double, device)
+    int n_waves = 0;               // 0 = no wave field
+    double wave_depth = INFINITY;
     long long* robot_offsets = nullptr;  // (n_robots_var + 1,) body offsets of unequal robots, or nullptr
     long long n_robots_var = 0;
     int max_ctas_per_sm = 0;   // 0 = as many as fit
@@ -117,6 +121,13 @@ static void invalidate_graph(h2o_engine* e)
     if (e->graph) { cudaGraphDestroy(e->graph); e->graph = nullptr; }
     e->graph_steps = 0;
     e->graph_launches_per_replay = 0;
+}
+
+static WaveArgs wave_args(const h2o_engine* e)
+{
+    WaveArgs w;
+    w.tab = e->wave_tab; w.clock = e->wave_clock; w.depth = e->wave_depth; w.n = e->n_waves;
+    return w;
 }
 
 static h2o_engine* check(h2o_handle h)
@@ -277,6 +288,8 @@ static int launch_direct(h2o_engine* e, const StepArgs& a, long long body_begin,
     const long long cnt = a.n - body_begin;
     if (cnt <= 0) return H2O_OK;
     const int grid = int((cnt + 255) / 256);
+    const WaveArgs wv = wave_args(e);
+    const size_t smem = wave_smem_bytes(wv.n);
     if (e->dry_run) {
         e->launches += 1;
         return H2O_OK;
@@ -286,15 +299,16 @@ static int launch_direct(h2o_engine* e, const StepArgs& a, long long body_begin,
         memset(&cfg, 0, sizeof cfg);
         cfg.gridDim = dim3(grid);
         cfg.blockDim = dim3(256);
+        cfg.dynamicSmemBytes = smem;
         cfg.stream = stream;
         cudaLaunchAttribute attr[1];
         attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, step_direct_kernel<S, kLayout, kParam, kStats>, a, body_begin));
+        CUDA_TRY(cudaLaunchKernelEx(&cfg, step_direct_kernel<S, kLayout, kParam, kStats>, a, body_begin, wv));
     } else {
-        step_direct_kernel<S, kLayout, kParam, kStats><<<grid, 256, 0, stream>>>(a, body_begin);
+        step_direct_kernel<S, kLayout, kParam, kStats><<<grid, 256, smem, stream>>>(a, body_begin, wv);
     }
     CUDA_TRY(cudaGetLastError());
     e->launches += 1;
@@ -335,7 +349,7 @@ static int step_typed2(h2o_engine* e, StepArgs& a, cudaStream_t stream)
     if (e->kernel_choice == H2O_KERNEL_TILE) use_tile = true;
     else if (e->kernel_choice == H2O_KERNEL_AUTO) use_tile = a.n >= (long long)e->sm_count * 256;
     if (TB == 0 || !ptr_ok || a.n < TB) use_tile = false;
-    if (a.am_dense || a.surface_eta || a.warp_compat) use_tile = false;  // f3 / f4 modes: direct kernel (+ robot_wrench_kernel)
+    if (a.am_dense || a.surface_eta || e->n_waves || a.warp_compat) use_tile = false;  // f3 / f4 modes: direct kernel (+ robot_wrench_kernel)
 
     long long done_bodies = 0;
     if (use_tile) {
@@ -423,10 +437,25 @@ static int step_typed(h2o_engine* e, int layout, StepArgs& a, cudaStream_t strea
 #undef H2O_DISPATCH
 }
 
-// Core step on device pointers (no validation beyond configuration).
+// With a wave field: the clock advances by dt, n times, after the work already in `stream` (counted as a launch).
+static int advance_clock(h2o_engine* e, double dt, int n, cudaStream_t stream)
+{
+    if (e->dry_run) {
+        e->launches += 1;
+        return H2O_OK;
+    }
+    advance_clock_kernel<<<1, 1, 0, stream>>>(e->wave_clock, dt, n);
+    CUDA_TRY(cudaGetLastError());
+    e->launches += 1;
+    return H2O_OK;
+}
+
+// Core step on device pointers (no validation beyond configuration).  tick: advance the wave clock after the
+// step's kernels (the chunked host pipeline advances it once after all chunks instead).
 static int step_device(h2o_engine* e, int layout, const void* pos, const void* quat, const void* lin,
                        const void* ang, double dt, void* f, void* t, void* w, long long n,
-                       long long first_body, void* prev, const void* coeff_base, cudaStream_t stream)
+                       long long first_body, void* prev, const void* coeff_base, cudaStream_t stream,
+                       bool tick = true)
 {
     if (e->param_mode < 0) return fail(H2O_ERR_NOT_CONFIGURED, "no parameters set (h2o_set_params_*)");
     if (!(dt > 1e-6)) return H2O_OK;  // hydrodynamics_behavior.py:139
@@ -459,7 +488,9 @@ static int step_device(h2o_engine* e, int layout, const void* pos, const void* q
     a.warp_compat = e->warp_compat;
     a.redo_bitmap = e->redo_bitmap;
     a.surface_eta = e->surface_eta ? static_cast<const char*>(e->surface_eta) + size_t(first_body) * e->esz : nullptr;
-    return e->dtype == H2O_F32 ? step_typed<float>(e, layout, a, stream) : step_typed<double>(e, layout, a, stream);
+    const int rc = e->dtype == H2O_F32 ? step_typed<float>(e, layout, a, stream) : step_typed<double>(e, layout, a, stream);
+    if (rc || !e->n_waves || !tick) return rc;
+    return advance_clock(e, dt, 1, stream);
 }
 
 static const void* coeff_at(h2o_engine* e, long long first_body)
@@ -522,6 +553,9 @@ int h2o_create(h2o_handle* out, int64_t n_bodies, int dtype, int device)
     if (cudaMalloc(&e->prev, size_t(n_bodies) * 6 * e->esz) != cudaSuccess ||
         cudaMalloc(reinterpret_cast<void**>(&e->stats), N_STATS * sizeof(double)) != cudaSuccess ||
         cudaMalloc(reinterpret_cast<void**>(&e->redo_bitmap), bitmap_bytes) != cudaSuccess ||
+        cudaMalloc(reinterpret_cast<void**>(&e->wave_tab), MAX_WAVE_COMPONENTS * WAVE_STRIDE * sizeof(double)) != cudaSuccess ||
+        cudaMalloc(reinterpret_cast<void**>(&e->wave_clock), sizeof(double)) != cudaSuccess ||
+        cudaMemset(e->wave_clock, 0, sizeof(double)) != cudaSuccess ||
         cudaMemset(e->redo_bitmap, 0, bitmap_bytes) != cudaSuccess ||
         cudaMemset(e->prev, 0, size_t(n_bodies) * 6 * e->esz) != cudaSuccess ||
         cudaMemset(e->stats, 0, N_STATS * sizeof(double)) != cudaSuccess) {
@@ -529,6 +563,8 @@ int h2o_create(h2o_handle* out, int64_t n_bodies, int dtype, int device)
         if (e->prev) cudaFree(e->prev);
         if (e->stats) cudaFree(e->stats);
         if (e->redo_bitmap) cudaFree(e->redo_bitmap);
+        if (e->wave_tab) cudaFree(e->wave_tab);
+        if (e->wave_clock) cudaFree(e->wave_clock);
         delete e;
         return fail(H2O_ERR_CUDA, "allocating the engine state for %lld bodies failed: %s", (long long)n_bodies,
                     cudaGetErrorString(why));
@@ -560,6 +596,8 @@ int h2o_destroy(h2o_handle h)
     if (e->prev) cudaFree(e->prev);
     if (e->stats) cudaFree(e->stats);
     if (e->redo_bitmap) cudaFree(e->redo_bitmap);
+    if (e->wave_tab) cudaFree(e->wave_tab);
+    if (e->wave_clock) cudaFree(e->wave_clock);
     e->magic = 0;
     delete e;
     return H2O_OK;
@@ -591,6 +629,81 @@ int h2o_set_surface_heights(h2o_handle h, const void* eta_dev)
     if (!e) return H2O_ERR_BAD_HANDLE;
     { DeviceGuard gi(e->device); invalidate_graph(e); }
     e->surface_eta = eta_dev;
+    return H2O_OK;
+}
+
+int h2o_set_wave_field(h2o_handle h, int n_components, const double* comps, double depth)
+{
+    h2o_engine* e = check(h);
+    if (!e) return H2O_ERR_BAD_HANDLE;
+    { DeviceGuard gi(e->device); invalidate_graph(e); }
+    if (n_components == 0) {
+        e->n_waves = 0;
+        return H2O_OK;
+    }
+    if (n_components < 0 || n_components > MAX_WAVE_COMPONENTS)
+        return fail(H2O_ERR_BAD_ARGUMENT, "n_components %d out of range [0,%d]", n_components, MAX_WAVE_COMPONENTS);
+    if (!comps) return fail(H2O_ERR_BAD_ARGUMENT, "comps is NULL");
+    if (!(depth > 0.0))  // also refuses NaN and -inf; +inf = deep water
+        return fail(H2O_ERR_BAD_ARGUMENT, "depth must be > 0 (+inf = deep water), got %g", depth);
+    std::vector<double> tab(size_t(n_components) * WAVE_STRIDE);
+    for (int j = 0; j < n_components; ++j) {
+        const double* c = comps + 5 * j;
+        for (int k = 0; k < 5; ++k)
+            if (!std::isfinite(c[k])) return fail(H2O_ERR_BAD_ARGUMENT, "component %d: non-finite value", j);
+        if (c[0] < 0.0) return fail(H2O_ERR_BAD_ARGUMENT, "component %d: amplitude %g < 0", j, c[0]);
+        if (c[1] == 0.0 && c[2] == 0.0) return fail(H2O_ERR_BAD_ARGUMENT, "component %d: wave vector is zero", j);
+        if (!(c[3] > 0.0)) return fail(H2O_ERR_BAD_ARGUMENT, "component %d: omega %g <= 0", j, c[3]);
+        wave_table_row(c, depth, tab.data() + size_t(j) * WAVE_STRIDE);
+    }
+    DeviceGuard g(e->device);
+    e->n_waves = 0;  // no field until the upload below succeeds
+    CUDA_TRY(cudaMemcpy(e->wave_tab, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice));
+    e->n_waves = n_components;
+    e->wave_depth = depth;
+    return H2O_OK;
+}
+
+int h2o_wave_time_write(h2o_handle h, double t, h2o_stream stream)
+{
+    h2o_engine* e = check(h);
+    if (!e) return H2O_ERR_BAD_HANDLE;
+    if (!std::isfinite(t)) return fail(H2O_ERR_BAD_ARGUMENT, "wave time must be finite");
+    DeviceGuard g(e->device);
+    set_clock_kernel<<<1, 1, 0, static_cast<cudaStream_t>(stream)>>>(e->wave_clock, t);
+    CUDA_TRY(cudaGetLastError());
+    return H2O_OK;
+}
+
+int h2o_wave_time_read(h2o_handle h, double* t, h2o_stream stream)
+{
+    h2o_engine* e = check(h);
+    if (!e) return H2O_ERR_BAD_HANDLE;
+    if (!t) return fail(H2O_ERR_BAD_ARGUMENT, "t is NULL");
+    DeviceGuard g(e->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    CUDA_TRY(cudaMemcpyAsync(t, e->wave_clock, sizeof(double), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    return H2O_OK;
+}
+
+int h2o_wave_sample(h2o_handle h, const void* points, int64_t m, double* out, h2o_stream stream)
+{
+    h2o_engine* e = check(h);
+    if (!e) return H2O_ERR_BAD_HANDLE;
+    if (m < 0) return fail(H2O_ERR_BAD_ARGUMENT, "m must be >= 0");
+    if (m == 0) return H2O_OK;
+    if (!points || !out) return fail(H2O_ERR_BAD_ARGUMENT, "NULL points / out");
+    DeviceGuard g(e->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int grid = int((m + 255) / 256);
+    const size_t smem = (size_t(e->n_waves) * WAVE_STRIDE + 1) * sizeof(double);
+    if (e->dtype == H2O_F32)
+        wave_sample_kernel<float><<<grid, 256, smem, s>>>(wave_args(e), e->surface_z, static_cast<const float*>(points), m, out);
+    else
+        wave_sample_kernel<double><<<grid, 256, smem, s>>>(wave_args(e), e->surface_z, static_cast<const double*>(points), m,
+                                                           out);
+    CUDA_TRY(cudaGetLastError());
     return H2O_OK;
 }
 
@@ -1150,7 +1263,9 @@ int h2o_rollout_persistent(h2o_handle h, int n_steps, double dt, double gravity,
     if (trace_every < 0 || (trace_every > 0 && !trace_out))
         return fail(H2O_ERR_BAD_ARGUMENT, "trace_every > 0 needs a trace buffer of (n_steps / trace_every, n_bodies, 9)");
     if (e->am_dense || e->surface_eta)
-        return fail(H2O_ERR_NOT_CONFIGURED, "persistent rollouts keep the wrapper's added-mass diagonal and a flat surface");
+        return fail(H2O_ERR_NOT_CONFIGURED,
+                    "persistent rollouts keep the wrapper's added-mass diagonal and take no caller height field "
+                    "(the built-in wave field works)");
     if (!(dt > 1e-6)) return H2O_OK;  // hydrodynamics_behavior.py:139
     DeviceGuard g(e->device);
     RolloutArgs a;
@@ -1170,6 +1285,8 @@ int h2o_rollout_persistent(h2o_handle h, int n_steps, double dt, double gravity,
     for (int k = 0; k < 3; ++k) a.current[k] = e->current[k];
     a.surface_z = e->surface_z;
     a.no_fallback = e->no_fallback;
+    a.waves = wave_args(e);
+    const size_t smem = wave_smem_bytes(e->n_waves);
     // small batches: one warp per CTA so that the warps spread over the SMs (a lone warp per scheduler
     // issues back to back); large batches: ordinary 128-thread CTAs
     const int block = e->n <= (long long)e->sm_count * 4 * 32 ? 32 : 128;
@@ -1177,15 +1294,16 @@ int h2o_rollout_persistent(h2o_handle h, int n_steps, double dt, double gravity,
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const bool st = e->stats_on;
     if (e->dtype == H2O_F32) {
-        if (st) rollout_persistent_kernel<float, true><<<grid, block, 0, s>>>(a);
-        else rollout_persistent_kernel<float, false><<<grid, block, 0, s>>>(a);
+        if (st) rollout_persistent_kernel<float, true><<<grid, block, smem, s>>>(a);
+        else rollout_persistent_kernel<float, false><<<grid, block, smem, s>>>(a);
     } else {
-        if (st) rollout_persistent_kernel<double, true><<<grid, block, 0, s>>>(a);
-        else rollout_persistent_kernel<double, false><<<grid, block, 0, s>>>(a);
+        if (st) rollout_persistent_kernel<double, true><<<grid, block, smem, s>>>(a);
+        else rollout_persistent_kernel<double, false><<<grid, block, smem, s>>>(a);
     }
     CUDA_TRY(cudaGetLastError());
     e->launches += 1;
     e->last_kernel = H2O_KERNEL_DIRECT;
+    if (e->n_waves) return advance_clock(e, dt, n_steps, s);
     return H2O_OK;
 }
 
@@ -1396,7 +1514,7 @@ static int step_host_impl(h2o_engine* e, int layout, const void* const in[4], vo
         char* dT = static_cast<char*>(e->hp_dev[5]) + size_t(b0) * 3 * e->esz;
         char* dW = bpr ? static_cast<char*>(e->hp_dev[6]) + size_t(b0 / bpr) * 6 * e->esz : nullptr;
         int rc = step_device(e, layout, dchunk[0], dchunk[1], dchunk[2], dchunk[3], dt, dF, dT, dW, cnt, b0,
-                             static_cast<char*>(e->prev) + size_t(b0) * 6 * e->esz, coeff_at(e, b0), s);
+                             static_cast<char*>(e->prev) + size_t(b0) * 6 * e->esz, coeff_at(e, b0), s, false);
         if (rc) return rc;
         CUDA_TRY(cudaMemcpyAsync(static_cast<char*>(dst[0]) + size_t(b0) * 3 * e->esz, dF, size_t(cnt) * 3 * e->esz,
                                  cudaMemcpyDefault, s));
@@ -1407,6 +1525,10 @@ static int step_host_impl(h2o_engine* e, int layout, const void* const in[4], vo
                                      size_t(cnt / bpr) * 6 * e->esz, cudaMemcpyDefault, s));
     }
     for (int i = 0; i < HOST_PIPE_STREAMS; ++i) CUDA_TRY(cudaStreamSynchronize(e->hp_stream[i]));
+    if (e->n_waves) {  // every chunk has read the clock: one advance for the whole step
+        if (int rc = advance_clock(e, dt, 1, e->hp_stream[0])) return rc;
+        CUDA_TRY(cudaStreamSynchronize(e->hp_stream[0]));
+    }
     for (int i = 0; i < 3; ++i) {
         if (!stage_out[i]) continue;
         const size_t bytes = i == 2 ? size_t(e->n / std::max(1, e->bodies_per_robot)) * 6 * e->esz

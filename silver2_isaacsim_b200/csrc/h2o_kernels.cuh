@@ -29,6 +29,7 @@
 #include <stdint.h>
 
 #include "h2o_model.cuh"
+#include "h2o_waves.cuh"
 
 // study knob (-DH2O_SKIP_ALL=true): the warp-uniform surface-logic skip of the robot-mode kernels in EVERY tile kernel
 // (the 80-register default kernel spills on it; used with regime-sorted inputs to bound what an in-tile sort could give)
@@ -90,6 +91,16 @@ struct StepArgs {
                              // Numba path: every body through the float64 world-frame formulation, direct kernel only
     int no_fallback;         // study knob H2O_NO_FALLBACK: 1 = keep the fast-path result of flagged bodies,
                              // k = 2^j > 1 = re-evaluate exactly every k-th body instead (cost measurements)
+};
+
+// Optional built-in wave field (h2o_set_wave_field): n rows of WAVE_STRIDE doubles, the water depth (+inf = deep)
+// and the engine's clock (one double, device).  n == 0 = none.  A parameter of the per-body kernels only (the tile
+// kernel, which has no wave code, keeps its StepArgs).
+struct WaveArgs {
+    const double* tab;
+    const double* clock;
+    double depth;
+    int n;
 };
 
 // ---------------------------------------------------------------------------
@@ -352,10 +363,11 @@ __device__ __noinline__ ExactStepOut body_step_exact_from_global(
     for (int j = 0; j < N_COEFF; ++j) cl[j] = c[j];
     return exact_eval_f32(r, cl, quat_wxyz, rho, grav, inv_dt, surface_z, cx, cy, cz, am_dense);
 }
-// prev_row: nullptr = the body's row of a.prev (still the OLD velocities), else a saved copy of that row
+// prev_row: nullptr = the body's row of a.prev (still the OLD velocities), else a saved copy of that row.
+// surface_z, cx, cy, cz: the waterline and the flow (rounded to float) the fast path saw for this body.
 template <int kLayout, int kParam>
-__device__ __forceinline__ ExactStepOut redo_exact(const StepArgs& a, long long i, double surface_z,
-                                                   const float* prev_row = nullptr)
+__device__ __forceinline__ ExactStepOut redo_exact(const StepArgs& a, long long i, double surface_z, float cx, float cy,
+                                                   float cz, const float* prev_row = nullptr)
 {
     const float* am = a.am_dense ? reinterpret_cast<const float*>(a.am_dense) + 36 * a.am_slot_type[(a.first_body + i) % a.am_n_slots]
                                  : nullptr;
@@ -364,12 +376,11 @@ __device__ __forceinline__ ExactStepOut redo_exact(const StepArgs& a, long long 
             reinterpret_cast<const float*>(a.pos), reinterpret_cast<const float*>(a.quat),
             reinterpret_cast<const float*>(a.lin), reinterpret_cast<const float*>(a.ang), prev_row,
             reinterpret_cast<const float*>(a.coeff), a.slot_type, i, a.first_body, a.n_slots, a.quat_wxyz, a.rho, a.grav,
-            a.inv_dt, surface_z, float(a.current[0]), float(a.current[1]), float(a.current[2]), am);
+            a.inv_dt, surface_z, cx, cy, cz, am);
     return body_step_exact_from_global<kLayout, kParam, false>(
         reinterpret_cast<const float*>(a.pos), reinterpret_cast<const float*>(a.quat), reinterpret_cast<const float*>(a.lin),
         reinterpret_cast<const float*>(a.ang), reinterpret_cast<const float*>(a.prev), reinterpret_cast<const float*>(a.coeff),
-        a.slot_type, i, a.first_body, a.n_slots, a.quat_wxyz, a.rho, a.grav, a.inv_dt, surface_z, float(a.current[0]),
-        float(a.current[1]), float(a.current[2]), am);
+        a.slot_type, i, a.first_body, a.n_slots, a.quat_wxyz, a.rho, a.grav, a.inv_dt, surface_z, cx, cy, cz, am);
 }
 
 // Deferred re-evaluation at the end of a tile-kernel CTA: one saved body per lane, and the float64 model split
@@ -509,7 +520,7 @@ __device__ __forceinline__ void accumulate_stats(ThreadStats& st, double fx, dou
 // `i` = body index inside the launch (a.pos etc. are the launch's base pointers).
 template <typename S, int kLayout, int kParam, bool kStats, bool kDefer, bool kWarpSkip = false>
 __device__ __forceinline__ bool step_one_body(const StepArgs& a, long long i, const BodyIn<double, S>& in, S mass,
-                                              double surface_z, S F[3], S T[3], ThreadStats& st, uint32_t& mask)
+                                              const Env& env, S F[3], S T[3], ThreadStats& st, uint32_t& mask)
 {
     bool clamped, still;
     double ratio;
@@ -518,7 +529,8 @@ __device__ __forceinline__ bool step_one_body(const StepArgs& a, long long i, co
         redo = redo && a.no_fallback != 1;
         if (a.no_fallback > 1) redo = ((a.first_body + i) & (long long)(a.no_fallback - 1)) == 0;  // study knob: every k-th body, k = 2^j
         if (redo && !kDefer) {
-            const ExactStepOut o = redo_exact<kLayout, kParam>(a, i, surface_z);
+            const ExactStepOut o =
+                redo_exact<kLayout, kParam>(a, i, env.surface_z, float(env.cx), float(env.cy), float(env.cz));
 #pragma unroll
             for (int k = 0; k < 3; ++k) {
                 F[k] = S(o.F[k]);
@@ -787,7 +799,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) step_tile_kernel(const _
                 uint32_t kp_mask;
                 // robot mode (fleets: usually every body of a warp is fully submerged) skips the keypoint compares warp-wide;
                 // its CTAs run under a 96-register cap, the 80-register default kernel would spill on the branch
-                if (step_one_body<S, kLayout, kParam, kStats, true, (kRobot || H2O_SKIP_ALL)>(a, tile_begin + tid, bin, cl[10], env.surface_z, F, T, st, kp_mask)) {
+                if (step_one_body<S, kLayout, kParam, kStats, true, (kRobot || H2O_SKIP_ALL)>(a, tile_begin + tid, bin, cl[10], env, F, T, st, kp_mask)) {
                     if (sizeof(S) == 4) {
                         const long long bi = tile_begin + tid;
                         const int slot = atomicAdd(redo_count, 1);
@@ -941,7 +953,8 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) step_tile_kernel(const _
                 const long long bi = tile_start(it) + tid;
                 const long long gi = a.first_body + bi;
                 if (tid < TB && ((a.redo_bitmap[gi >> 5] >> (gi & 31)) & 1u)) {
-                    const ExactStepOut o = redo_exact<kLayout, kParam>(a, bi, env.surface_z);
+                    const ExactStepOut o = redo_exact<kLayout, kParam>(a, bi, env.surface_z, float(a.current[0]),
+                                                                       float(a.current[1]), float(a.current[2]));
                     patch(bi, o);
                     BodyPtrs<float> bp;
                     bp.pos = reinterpret_cast<const float*>(a.pos); bp.quat = reinterpret_cast<const float*>(a.quat);
@@ -965,14 +978,30 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) step_tile_kernel(const _
 // step_direct_kernel: one thread per body, plain global loads/stores.
 // Processes bodies [body_begin, n).  Robot wrench (if requested) is produced by
 // robot_wrench_kernel below from the written force/torque arrays.
+// Dynamic shared memory: wave_smem_bytes(w.n) (the wave table and the clock value; 0 without waves).
 // ---------------------------------------------------------------------------
+inline size_t wave_smem_bytes(int n_waves) { return n_waves > 0 ? (size_t(n_waves) * WAVE_STRIDE + 1) * sizeof(double) : 0; }
+
+// Every thread of the CTA: stage the wave table, then the clock value behind it; the caller synchronises.
+__device__ __forceinline__ void stage_waves(double* dst, const double* tab, const double* clock, int n_waves)
+{
+    for (int k = threadIdx.x; k < n_waves * WAVE_STRIDE; k += blockDim.x) dst[k] = tab[k];
+    if (threadIdx.x == 0) dst[n_waves * WAVE_STRIDE] = *clock;
+}
+
 template <typename S, int kLayout, int kParam, bool kStats>
-__global__ void __launch_bounds__(256) step_direct_kernel(const __grid_constant__ StepArgs a, long long body_begin)
+__global__ void __launch_bounds__(256) step_direct_kernel(const __grid_constant__ StepArgs a, long long body_begin,
+                                                          const __grid_constant__ WaveArgs wv)
 {
     __shared__ S table[(kParam == PARAM_TABLE) ? MAX_TABLE_TYPES * N_COEFF : 1];
     __shared__ unsigned char slot_map[(kParam == PARAM_TABLE) ? MAX_TABLE_SLOTS : 1];
+    extern __shared__ double wave_smem[];
     pdl_launch_dependents();   // no-ops unless launched with the PDL attribute
     pdl_wait_prerequisites();
+    if (wv.n) {
+        stage_waves(wave_smem, wv.tab, wv.clock, wv.n);
+        __syncthreads();
+    }
     if (kParam == PARAM_TABLE) {
         const S* g = reinterpret_cast<const S*>(a.coeff);
         for (int i = threadIdx.x; i < a.n_types * N_COEFF; i += blockDim.x) table[i] = g[i];
@@ -1003,6 +1032,12 @@ __global__ void __launch_bounds__(256) step_direct_kernel(const __grid_constant_
         }
         BodyIn<double, S> bin;
         Env env{a.current[0], a.current[1], a.current[2], a.surface_z};
+        if (wv.n) {
+            const WaveSample w = wave_eval<sizeof(S) == 4>(wave_smem, wv.n, wv.depth, double(r.px), double(r.py),
+                                                           double(r.pz) - a.surface_z, wave_smem[wv.n * WAVE_STRIDE]);
+            env.surface_z += w.eta;
+            env.cx += w.ux; env.cy += w.uy; env.cz += w.uz;
+        }
         if (a.surface_eta) env.surface_z += double(reinterpret_cast<const S*>(a.surface_eta)[i]);
         make_body_in<S>(r, cl, a.quat_wxyz, a.rho, a.grav, S(a.inv_dt), env, bin);
         if (a.am_dense)
@@ -1033,7 +1068,7 @@ __global__ void __launch_bounds__(256) step_direct_kernel(const __grid_constant_
             if (kStats) accumulate_stats(st, double(F[0]), double(F[1]), double(F[2]), double(o.ratio), (o.flags & 1) != 0,
                                          (o.flags & 2) != 0, true);
         } else {
-            step_one_body<S, kLayout, kParam, kStats, false>(a, i, bin, cl[10], env.surface_z, F, T, st, kp_mask);
+            step_one_body<S, kLayout, kParam, kStats, false>(a, i, bin, cl[10], env, F, T, st, kp_mask);
         }
         S* of = reinterpret_cast<S*>(a.out_force) + 3 * i;
         S* ot = reinterpret_cast<S*>(a.out_torque) + 3 * i;
@@ -1310,11 +1345,19 @@ struct RolloutArgs {
     double dt, gravity, rho, grav;
     double current[3], surface_z;
     int no_fallback;
+    WaveArgs waves;  // evaluated at each step's position and at t, t + dt, ... from the clock
 };
 
+// Dynamic shared memory: wave_smem_bytes(a.waves.n).
 template <typename S, bool kStats>
 __global__ void rollout_persistent_kernel(const __grid_constant__ RolloutArgs a)
 {
+    extern __shared__ double wave_smem[];
+    const WaveArgs& wv = a.waves;
+    if (wv.n) {
+        stage_waves(wave_smem, wv.tab, wv.clock, wv.n);
+        __syncthreads();
+    }
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     ThreadStats st;
     if (i < a.n) {
@@ -1334,10 +1377,19 @@ __global__ void rollout_persistent_kernel(const __grid_constant__ RolloutArgs a)
         r.vx = V[0]; r.vy = V[1]; r.vz = V[2];
         r.wx = W[0]; r.wy = W[1]; r.wz = W[2];
         r.pvx = PV[0]; r.pvy = PV[1]; r.pvz = PV[2]; r.pwx = PV[3]; r.pwy = PV[4]; r.pwz = PV[5];
-        const Env env{a.current[0], a.current[1], a.current[2], a.surface_z};
+        const Env env0{a.current[0], a.current[1], a.current[2], a.surface_z};
         const S inv_dt = S(1.0 / a.dt);
         S F[3] = {S(0), S(0), S(0)}, T[3] = {S(0), S(0), S(0)};
+        double t = wv.n ? wave_smem[wv.n * WAVE_STRIDE] : 0.0;
         for (int step = 0; step < a.n_steps; ++step) {
+            Env env = env0;
+            if (wv.n) {
+                const WaveSample w = wave_eval<sizeof(S) == 4>(wave_smem, wv.n, wv.depth, double(r.px),
+                                                               double(r.py), double(r.pz) - a.surface_z, t);
+                env.surface_z += w.eta;
+                env.cx += w.ux; env.cy += w.uy; env.cz += w.uz;
+                t += a.dt;  // the same sequence of additions as advance_clock_kernel over single steps
+            }
             BodyIn<double, S> bin;
             make_body_in<S>(r, cl, a.quat_wxyz, a.rho, a.grav, inv_dt, env, bin);
             bool clamped, still;
@@ -1357,8 +1409,8 @@ __global__ void rollout_persistent_kernel(const __grid_constant__ RolloutArgs a)
                     float cf[N_COEFF];
 #pragma unroll
                     for (int k = 0; k < N_COEFF; ++k) cf[k] = float(cl[k]);
-                    const ExactStepOut o = body_step_exact_f32(rf, cf, a.quat_wxyz, a.rho, a.grav, 1.0 / a.dt, a.surface_z,
-                                                               float(a.current[0]), float(a.current[1]), float(a.current[2]));
+                    const ExactStepOut o = body_step_exact_f32(rf, cf, a.quat_wxyz, a.rho, a.grav, 1.0 / a.dt, env.surface_z,
+                                                               float(env.cx), float(env.cy), float(env.cz));
 #pragma unroll
                     for (int k = 0; k < 3; ++k) {
                         F[k] = S(o.F[k]);
@@ -1403,6 +1455,38 @@ __global__ void rollout_persistent_kernel(const __grid_constant__ RolloutArgs a)
         ot[0] = T[0]; ot[1] = T[1]; ot[2] = T[2];
     }
     if (kStats && a.stats) flush_stats(st, a.stats);
+}
+
+// ---------------------------------------------------------------------------
+// Wave clock and sampling (h2o_set_wave_field).  The clock is one double in engine-owned device memory; a step
+// evaluates the field at its value and then advance_clock_kernel adds dt to it n times (n = 1 after a step,
+// n = K after a K-step persistent rollout), in stream order, so that captured graphs and the host pipeline
+// see the same clock as eager steps.
+// ---------------------------------------------------------------------------
+__global__ void advance_clock_kernel(double* clock, double dt, int n)
+{
+    double t = *clock;
+    for (int k = 0; k < n; ++k) t += dt;
+    *clock = t;
+}
+__global__ void set_clock_kernel(double* clock, double t) { *clock = t; }
+
+// points (m,3) in the engine dtype -> out (m,4) float64 [eta, ux, uy, uz] at the clock's value: the evaluator and
+// precision policy of the step kernels.  Dynamic shared memory: (wv.n * WAVE_STRIDE + 1) doubles.
+template <typename S>
+__global__ void __launch_bounds__(256) wave_sample_kernel(const __grid_constant__ WaveArgs wv, double surface_z,
+                                                          const S* points, long long m, double* out)
+{
+    extern __shared__ double wave_smem[];
+    stage_waves(wave_smem, wv.tab, wv.clock, wv.n);
+    __syncthreads();
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    const S* p = points + 3 * i;
+    const WaveSample w = wave_eval<sizeof(S) == 4>(wave_smem, wv.n, wv.depth, double(p[0]), double(p[1]),
+                                                   double(p[2]) - surface_z, wave_smem[wv.n * WAVE_STRIDE]);
+    double* o = out + 4 * i;
+    o[0] = w.eta; o[1] = w.ux; o[2] = w.uy; o[3] = w.uz;
 }
 
 }  // namespace h2o

@@ -1,0 +1,113 @@
+// h2o_waves.cuh -- built-in linear (Airy) wave field, evaluated at a point and a clock value.
+//
+// One evaluator for every caller: the per-body step kernel, the persistent rollout kernel and the
+// h2o_wave_sample entry point on the device, tests/host_emul/waves_emul.cpp on the host.  Semantics are
+// pinned in include/h2o.h (h2o_set_wave_field): for component j
+//   theta_j = kx_j p_x + ky_j p_y - omega_j t + phase_j                      (always float64)
+//   eta     = sum a_j cos theta_j
+//   u_h     = sum a_j omega_j C_j(z) cos theta_j  k_j / |k_j|,   u_z = sum a_j omega_j S_j(z) sin theta_j
+// at z = clamp(p_z - surface_z, -h, 0), with C_j = cosh(k_j (z + h)) / sinh(k_j h),
+// S_j = sinh(k_j (z + h)) / sinh(k_j h) (finite depth) or C_j = S_j = exp(k_j z) (deep water).
+// The hyperbolic ratios are evaluated as (e^{kz} +- e^{-k(z + 2h)}) / (1 - e^{-2kh}): no overflow at
+// any k h, and the denominator comes from the table (computed once on the host with expm1).
+#pragma once
+
+#include "h2o_model.cuh"
+
+namespace h2o {
+
+constexpr int MAX_WAVE_COMPONENTS = 64;
+// one component of the engine's device table (doubles): what the caller gave + constants derived once
+enum : int {
+    WAVE_KX = 0, WAVE_KY, WAVE_OMEGA, WAVE_PHASE, WAVE_A,
+    WAVE_A_OMEGA,  // a * omega
+    WAVE_K,        // |k|
+    WAVE_KHAT_X, WAVE_KHAT_Y,  // k / |k|
+    WAVE_INV_DEN,  // 1 / (1 - e^{-2 k h}); 1 in deep water
+    WAVE_STRIDE
+};
+
+struct WaveSample {
+    double eta, ux, uy, uz;
+};
+
+// theta is formed with separately rounded products and sums, in the order written above, on every
+// platform (no FMA contraction), so that it is the same double the NumPy reference forms: at t ~ 1e5 s
+// one ulp of theta is ~1e-11 of the amplitude.
+H2O_HD double wave_mul(double a, double b)
+{
+#if defined(__CUDA_ARCH__)
+    return __dmul_rn(a, b);
+#else
+    volatile double r = a * b;
+    return r;
+#endif
+}
+H2O_HD double wave_add(double a, double b)
+{
+#if defined(__CUDA_ARCH__)
+    return __dadd_rn(a, b);
+#else
+    volatile double r = a + b;
+    return r;
+#endif
+}
+
+H2O_HD void wave_table_row(const double comp[5], double depth, double row[WAVE_STRIDE])
+{
+    const double a = comp[0], kx = comp[1], ky = comp[2], omega = comp[3], phase = comp[4];
+    const double k = sqrt(kx * kx + ky * ky);
+    row[WAVE_KX] = kx; row[WAVE_KY] = ky; row[WAVE_OMEGA] = omega; row[WAVE_PHASE] = phase; row[WAVE_A] = a;
+    row[WAVE_A_OMEGA] = a * omega;
+    row[WAVE_K] = k;
+    row[WAVE_KHAT_X] = kx / k; row[WAVE_KHAT_Y] = ky / k;
+    row[WAVE_INV_DEN] = depth < INFINITY ? -1.0 / expm1(-2.0 * k * depth) : 1.0;
+}
+
+// kF32: the fp32-mode policy.  The phase stays float64 and is reduced to [-pi, pi] in float64; sine, cosine and
+// the depth decay are then evaluated in float (device: MUFU approximations, |error| < 2^-21 on [-pi, pi]), and
+// the sums are kept in float64.  The field then stays within 2e-6 of sum a_j (elevation) and of
+// sum a_j omega_j (velocity) of the float64 values (tests/test_waves.py).
+template <bool kF32>
+H2O_HD WaveSample wave_eval(const double* tab, int n, double depth, double px, double py, double z_rel, double t)
+{
+    const bool deep = !(depth < INFINITY);
+    double z = z_rel < 0.0 ? z_rel : 0.0;
+    if (!deep && z < -depth) z = -depth;
+    WaveSample s{0.0, 0.0, 0.0, 0.0};
+    for (int j = 0; j < n; ++j) {
+        const double* c = tab + WAVE_STRIDE * j;
+        const double th = wave_add(wave_add(wave_add(wave_mul(c[WAVE_KX], px), wave_mul(c[WAVE_KY], py)),
+                                            -wave_mul(c[WAVE_OMEGA], t)),
+                                   c[WAVE_PHASE]);
+        const double k = c[WAVE_K];
+        double cs, sn, ez, ezb;
+        if (kF32) {
+            const double r = th - 6.283185307179586 * rint(th * 0.15915494309189535);
+            float sf, cf, e0, e1;
+#if defined(__CUDA_ARCH__)
+            __sincosf(float(r), &sf, &cf);
+            e0 = __expf(float(k * z));
+            e1 = deep ? 0.0f : __expf(float(-k * (z + 2.0 * depth)));
+#else
+            sf = sinf(float(r)); cf = cosf(float(r));
+            e0 = expf(float(k * z));
+            e1 = deep ? 0.0f : expf(float(-k * (z + 2.0 * depth)));
+#endif
+            cs = cf; sn = sf; ez = e0; ezb = e1;
+        } else {
+            sn = sin(th); cs = cos(th);
+            ez = exp(k * z);
+            ezb = deep ? 0.0 : exp(-k * (z + 2.0 * depth));
+        }
+        const double C = (ez + ezb) * c[WAVE_INV_DEN], S = (ez - ezb) * c[WAVE_INV_DEN];
+        const double uh = c[WAVE_A_OMEGA] * C * cs;
+        s.eta += c[WAVE_A] * cs;
+        s.ux += uh * c[WAVE_KHAT_X];
+        s.uy += uh * c[WAVE_KHAT_Y];
+        s.uz += c[WAVE_A_OMEGA] * S * sn;
+    }
+    return s;
+}
+
+}  // namespace h2o

@@ -13,6 +13,7 @@ zero-copy as DLPack descriptors; the arithmetic lives in ``csrc/``.
 from __future__ import annotations
 
 import ctypes
+import math
 from typing import Optional, Sequence, Tuple
 
 import numpy as np
@@ -21,6 +22,7 @@ from torch.utils import dlpack as _dlpack
 
 from . import _lib as L
 from . import params as P
+from . import waves as W
 
 _TORCH_DTYPES = {torch.float32: L.H2O_F32, torch.float64: L.H2O_F64}
 _NP_DTYPES = {L.H2O_F32: np.float32, L.H2O_F64: np.float64}
@@ -123,6 +125,46 @@ class HydroEngine:
             raise ValueError(f"eta must be a contiguous ({self.n_bodies},) {self.dtype} tensor on {self.device}")
         L.check(self._lib.h2o_set_surface_heights(self._h, ctypes.c_void_p(eta.data_ptr())))
         self._eta = eta  # keep the borrowed memory alive
+
+    def set_wave_field(self, field: Optional["W.WaveField"]):
+        """Built-in linear wave field (``waves.regular`` / ``waves.jonswap`` / ``waves.WaveField``), evaluated on the
+        GPU at every body's centre on every step at the engine's wave clock, which then advances by ``dt``.  The
+        waterline becomes ``surface_z + eta`` and drag, damping and lift see ``v - (current + u)`` (semantics in
+        include/h2o.h).  ``None`` removes the field.  Steps then run on the per-body kernel; ``rollout_persistent``
+        and captured rollouts follow the field; ``components`` ignores it."""
+        if field is None:
+            L.check(self._lib.h2o_set_wave_field(self._h, 0, None, math.inf))
+            return
+        if not isinstance(field, W.WaveField):
+            raise TypeError("field must be a waves.WaveField (waves.regular, waves.jonswap) or None")
+        comps = np.ascontiguousarray(field.components, dtype=np.float64)
+        L.check(self._lib.h2o_set_wave_field(self._h, int(comps.shape[0]),
+                                             comps.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), float(field.depth)))
+
+    @property
+    def wave_time(self) -> float:
+        """The wave clock (s): read after the work queued so far on the current stream (synchronises it)."""
+        t = ctypes.c_double()
+        L.check(self._lib.h2o_wave_time_read(self._h, ctypes.byref(t), _stream_ptr(self.device)))
+        return t.value
+
+    def set_wave_time(self, t: float):
+        """Set the wave clock, in stream order.  A captured rollout is kept: it reads the clock from device memory."""
+        t = float(t)
+        if not math.isfinite(t):
+            raise ValueError("wave time must be finite")
+        L.check(self._lib.h2o_wave_time_write(self._h, t, _stream_ptr(self.device)))
+
+    def sample_waves(self, points) -> torch.Tensor:
+        """Wave field at ``points`` (m,3) world positions and the current clock, with the step's evaluator and
+        precision: a (m,4) float64 CUDA tensor of rows ``eta, ux, uy, uz`` (zeros without a field)."""
+        pts = self._as_dev(points)
+        if pts.ndim != 2 or pts.shape[1] != 3:
+            raise ValueError(f"points must be (m,3), got {tuple(pts.shape)}")
+        out = torch.empty(pts.shape[0], 4, dtype=torch.float64, device=self.device)
+        L.check(self._lib.h2o_wave_sample(self._h, ctypes.c_void_p(pts.data_ptr()), int(pts.shape[0]),
+                                          ctypes.c_void_p(out.data_ptr()), _stream_ptr(self.device)))
+        return out
 
     def set_added_mass_dense(self, matrices=None, slot_type=None):
         """Dense 6x6 body-frame added-mass matrices (the argument ``calculate_added_mass`` takes,

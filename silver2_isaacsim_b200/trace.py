@@ -2,7 +2,7 @@
 
 ``VelocityTrace``  writes the CSV of the reference's ``LogVelocity`` behaviour
                    (/root/reference/src/scripts/physics/log_velocity.py:17-53): same header, same
-                   z / x / y column order, one row per sample of one body.
+                   z / x / y column order, one row per sample of one body (optional extra columns after them).
 ``RtfMeter``       accumulates simulated vs wall time like ``BenchmarkRtf``
                    (/root/reference/src/scripts/physics/benchmark_rtf.py:37-71): real-time factor and
                    steps per second, with a live line every ``report_every`` steps.
@@ -12,7 +12,7 @@ from __future__ import annotations
 import csv
 import datetime
 import time
-from typing import Optional
+from typing import Optional, Sequence
 
 LOG_HEADER = ["timestamp",
               "z_position", "linear_velocity_z", "angular_velocity_z",
@@ -21,16 +21,18 @@ LOG_HEADER = ["timestamp",
 
 
 class VelocityTrace:
-    def __init__(self, path: str, body: int = 0):
-        self.path, self.body = path, body
+    def __init__(self, path: str, body: int = 0, extra_columns: Sequence[str] = ()):
+        self.path, self.body, self.n_extra = path, body, len(extra_columns)
         with open(path, "w", newline="") as f:
-            csv.writer(f).writerow(LOG_HEADER)
+            csv.writer(f).writerow(LOG_HEADER + list(extra_columns))
 
-    def sample(self, position, linear_vel, angular_vel, timestamp: Optional[str] = None):
-        """Append one row for body ``self.body`` (tensors or arrays of shape (N,3))."""
+    def sample(self, position, linear_vel, angular_vel, timestamp: Optional[str] = None, extra: Sequence[float] = ()):
+        """Append one row for body ``self.body`` (tensors or arrays of shape (N,3)), then the ``extra`` values."""
+        if len(extra) != self.n_extra:
+            raise ValueError(f"expected {self.n_extra} extra values, got {len(extra)}")
         p, v, w = (x[self.body].tolist() for x in (position, linear_vel, angular_vel))
         row = [timestamp or datetime.datetime.now().isoformat(),
-               p[2], v[2], w[2], p[0], v[0], w[0], p[1], v[1], w[1]]  # log_velocity.py:38-49
+               p[2], v[2], w[2], p[0], v[0], w[0], p[1], v[1], w[1]] + [float(x) for x in extra]  # log_velocity.py:38-49
         with open(self.path, "a", newline="") as f:
             csv.writer(f).writerow(row)
 

@@ -1,0 +1,139 @@
+"""Linear (Airy) wave fields for the engine's built-in wave evaluator (``HydroEngine.set_wave_field``).
+
+A field is a sum of components ``(a, kx, ky, omega, phase)`` over water of depth ``h`` (``inf`` = deep
+water); ``include/h2o.h`` (``h2o_set_wave_field``) pins the formulas.  This module builds fields
+(``regular``, ``jonswap``), solves the dispersion relation and evaluates a field in float64
+(``evaluate``, the reference the GPU evaluator is tested against).  NumPy only.
+"""
+from __future__ import annotations
+
+import math
+from dataclasses import dataclass
+
+import numpy as np
+
+MAX_COMPONENTS = 64  # h2o_set_wave_field
+
+
+def _check_depth(depth) -> float:
+    depth = float(depth)
+    if not depth > 0.0:  # also NaN and -inf
+        raise ValueError(f"depth must be > 0 (inf = deep water), got {depth}")
+    return depth
+
+
+@dataclass(frozen=True)
+class WaveField:
+    """``components``: (n, 5) float64 rows ``a, kx, ky, omega, phase``; ``depth``: water depth (``inf`` = deep)."""
+
+    components: np.ndarray
+    depth: float = math.inf
+
+    def __post_init__(self):
+        c = np.array(self.components, dtype=np.float64)  # a private copy
+        if c.ndim != 2 or c.shape[1] != 5:
+            raise ValueError("components must be an (n, 5) array of a, kx, ky, omega, phase")
+        if len(c) > MAX_COMPONENTS:
+            raise ValueError(f"at most {MAX_COMPONENTS} components, got {len(c)}")
+        if not np.isfinite(c).all():
+            raise ValueError("components must be finite")
+        if (c[:, 0] < 0).any():
+            raise ValueError("amplitudes must be >= 0")
+        if ((c[:, 1] == 0) & (c[:, 2] == 0)).any():
+            raise ValueError("every wave vector (kx, ky) must be non-zero")
+        if not (c[:, 3] > 0).all():
+            raise ValueError("angular frequencies must be > 0")
+        c.setflags(write=False)
+        object.__setattr__(self, "components", c)
+        object.__setattr__(self, "depth", _check_depth(self.depth))
+
+    @property
+    def n_components(self) -> int:
+        return len(self.components)
+
+
+def wavenumber(omega, depth=math.inf, g: float = 9.81):
+    """Wavenumber k of the linear dispersion relation ``omega^2 = g k tanh(k h)`` (Newton's method on
+    ``x tanh x = omega^2 h / g``, x = k h; deep water: ``omega^2 / g``).  ``omega`` may be an array."""
+    w = np.asarray(omega, dtype=np.float64)
+    if not (np.isfinite(w).all() and (w > 0).all()):
+        raise ValueError("omega must be finite and > 0")
+    if not g > 0:
+        raise ValueError("g must be > 0")
+    h = _check_depth(depth)
+    k_deep = w * w / g
+    if math.isinf(h):
+        return k_deep if k_deep.ndim else float(k_deep)
+    y = k_deep * h
+    x = y / np.sqrt(np.tanh(y ** 0.75)) ** (4.0 / 3.0)  # Fenton & McKee (1990): within ~1 % everywhere
+    for _ in range(50):
+        th = np.tanh(x)
+        dx = (x * th - y) / (th + x * (1.0 - th * th))
+        x = x - dx
+        if (np.abs(dx) <= 4e-16 * x).all():
+            break
+    k = x / h
+    return k if k.ndim else float(k)
+
+
+def regular(amplitude: float, period: float, direction: float = 0.0, phase: float = 0.0, depth=math.inf,
+            g: float = 9.81) -> WaveField:
+    """One regular wave of amplitude ``amplitude`` (m) and period ``period`` (s) travelling towards
+    ``direction`` (radians from +x)."""
+    if not period > 0:
+        raise ValueError("period must be > 0")
+    omega = 2.0 * math.pi / period
+    k = wavenumber(omega, depth, g)
+    return WaveField(np.array([[amplitude, k * math.cos(direction), k * math.sin(direction), omega, phase]]), depth)
+
+
+def jonswap(hs: float, tp: float, gamma: float = 3.3, n_components: int = 32, direction: float = 0.0, seed: int = 0,
+            depth=math.inf, g: float = 9.81) -> WaveField:
+    """Unidirectional JONSWAP sea: ``n_components`` equal-width frequency bins over [0.5, 3] x the peak
+    frequency ``1 / tp``, amplitude ``sqrt(2 S(f) df)`` at each bin centre, seeded uniform random phases.
+    The spectrum is scaled so that the components carry exactly the variance ``(hs / 4)^2``."""
+    if not (hs > 0 and tp > 0 and gamma >= 1):
+        raise ValueError("need hs > 0, tp > 0 and gamma >= 1")
+    if not 1 <= int(n_components) <= MAX_COMPONENTS:
+        raise ValueError(f"n_components must be in [1, {MAX_COMPONENTS}]")
+    n = int(n_components)
+    fp = 1.0 / tp
+    f_lo, f_hi = 0.5 * fp, 3.0 * fp
+    df = (f_hi - f_lo) / n
+    f = f_lo + (np.arange(n) + 0.5) * df
+    sigma = np.where(f <= fp, 0.07, 0.09)
+    shape = f ** -5.0 * np.exp(-1.25 * (fp / f) ** 4) * gamma ** np.exp(-((f - fp) ** 2) / (2.0 * sigma ** 2 * fp ** 2))
+    var = shape * df
+    a = np.sqrt(2.0 * var * (hs / 4.0) ** 2 / var.sum())
+    omega = 2.0 * math.pi * f
+    k = wavenumber(omega, depth, g)
+    phase = np.random.default_rng(seed).uniform(0.0, 2.0 * math.pi, n)
+    comps = np.stack([a, k * math.cos(direction), k * math.sin(direction), omega, phase], axis=1)
+    return WaveField(comps, depth)
+
+
+def evaluate(field: WaveField, points, t: float, surface_z: float = 0.0) -> np.ndarray:
+    """Float64 reference of the field at ``points`` (m, 3) and clock ``t``: (m, 4) rows ``eta, ux, uy, uz``.
+    The phase is formed in the order the GPU evaluator forms it, ``((kx px + ky py) - omega t) + phase``."""
+    p = np.asarray(points, dtype=np.float64).reshape(-1, 3)
+    c = field.components
+    a, kx, ky, w, ph = (c[:, j][None, :] for j in range(5))
+    k = np.hypot(kx, ky)
+    h = field.depth
+    z = np.minimum(p[:, 2:3] - surface_z, 0.0)
+    if math.isinf(h):
+        C = S = np.exp(k * z)
+    else:
+        z = np.maximum(z, -h)
+        inv = -1.0 / np.expm1(-2.0 * k * h)
+        e0, e1 = np.exp(k * z), np.exp(-k * (z + 2.0 * h))
+        C, S = (e0 + e1) * inv, (e0 - e1) * inv   # cosh(k(z+h)) / sinh(kh), sinh(k(z+h)) / sinh(kh)
+    th = ((kx * p[:, 0:1] + ky * p[:, 1:2]) - w * t) + ph
+    cs, sn = np.cos(th), np.sin(th)
+    uh = a * w * C * cs
+    out = np.empty((len(p), 4))
+    out[:, 0] = (a * cs).sum(axis=1)
+    out[:, 1] = (uh * (kx / k)).sum(axis=1)
+    out[:, 2] = (uh * (ky / k)).sum(axis=1)
+    out[:, 3] = (a * w * S * sn).sum(axis=1)
+    return out
