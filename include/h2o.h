@@ -143,6 +143,44 @@ H2O_API int h2o_wave_time_read(h2o_handle h, double* t, h2o_stream stream);
  * surface_z), out a DEVICE array (m,4) float64 of rows [eta, ux, uy, uz] (zeros without a field). */
 H2O_API int h2o_wave_sample(h2o_handle h, const void* points, int64_t m, double* out, h2o_stream stream);
 
+/* Per-env water conditions for vectorised scenes (SURVEY.md 8(f4)).  Envs are contiguous, equal runs of bodies:
+ * body i (global index) belongs to env e = i / bodies_per_env, and E = n_bodies / bodies_per_env.  cond_dev is a
+ * DEVICE array (E, 8) of float64 on the handle's device, 8-byte aligned, one row per env:
+ *   cond[e] = [cx, cy, cz, dz, s, tau, x0, y0]
+ *   cx, cy, cz  current added to the global current       dz      water-level offset added to surface_z
+ *   s           wave scale (multiplies eta and u)         tau     wave time offset (s)
+ *   x0, y0      env origin
+ * For a body of env e at p with clock value t, every operation a separately rounded float64 operation:
+ *   mean level  L_e = surface_z + dz
+ *   theta_j   = ((kx_j (p_x - x0) + ky_j (p_y - y0)) - omega_j (t + tau)) + phase_j
+ *   velocity depth z = clamp(p_z - L_e, -h, 0)
+ *   waterline = L_e + s eta            (+ eta[i] when a height field is also set, h2o_set_surface_heights)
+ *   flow      = (current + c_e) + s u  (fp32 mode: summed in double, rounded once to the handle dtype)
+ * Without a wave field: waterline L_e, flow current + c_e.  The precision policies of h2o_set_wave_field hold.
+ * The identity row [0,0,0,0,1,0,0,0] makes every operation exact: results are bit-identical to a handle without
+ * conditions on the same kernel.
+ * The array is borrowed, not copied: every later step reads it (a persistent rollout reads each row once at kernel
+ * start), so the caller may update it in place between steps or graph replays with no recapture.  It must stay
+ * allocated while set.  bodies_per_env == 0 or cond_dev == NULL removes the conditions.  H2O_ERR_BAD_SHAPE when
+ * bodies_per_env does not divide n_bodies, H2O_ERR_ALIGNMENT / H2O_ERR_BAD_DEVICE for a misaligned pointer or one
+ * not on the handle's device.  Steps with conditions run on the per-body kernel, as with a wave field;
+ * h2o_rollout_persistent accepts them; h2o_components ignores them.  Like every h2o_set_* call this drops a
+ * captured rollout; a refused call leaves it intact. */
+H2O_API int h2o_set_env_conditions(h2o_handle h, int64_t bodies_per_env, const double* cond_dev);
+/* Masked reset of the carried state (the per-env _reset, hydrodynamics_behavior.py:240-245), one stream-ordered
+ * kernel without host synchronisation: env_mask_dev is a DEVICE array of E bytes; the carried [v, omega] of every
+ * body of an env with mask[e] != 0 becomes zero.  restart_waves != 0 also writes cond[e][5] = -clock (read from the
+ * device clock) for those envs, in the borrowed array, so that their next step sees their sea at env time exactly 0.
+ * Other bodies and rows are left bit-unchanged.  Does not drop a captured rollout.  H2O_ERR_NOT_CONFIGURED without
+ * conditions. */
+H2O_API int h2o_reset_envs(h2o_handle h, const uint8_t* env_mask_dev, int restart_waves, h2o_stream stream);
+/* h2o_wave_sample seen from envs: point k is evaluated for env env_index[k] (DEVICE int32 array (m,)) at the
+ * clock's current value, through the step's evaluator.  out rows are [s eta, s ux, s uy, s uz]: the field alone
+ * (c_e and dz are not added); zero rows without a wave field; a NaN row for an index outside [0, E).
+ * H2O_ERR_NOT_CONFIGURED without conditions. */
+H2O_API int h2o_wave_sample_env(h2o_handle h, const void* points, const int32_t* env_index, int64_t m, double* out,
+                                h2o_stream stream);
+
 /* Same twelve scalars, same order as the reference wrapper ctor
  * (numba_hydrodynamics_wrapper.py:9-10): width, depth, height, linear_drag_coefficient,
  * angular_drag_coefficient, linear_damping, angular_damping, water_density, gravity,

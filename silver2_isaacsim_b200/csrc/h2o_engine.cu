@@ -80,6 +80,8 @@ struct h2o_engine {
     double* wave_clock = nullptr;  // the wave field's clock (one double, device)
     int n_waves = 0;               // 0 = no wave field
     double wave_depth = INFINITY;
+    const double* env_cond = nullptr;  // (n / bodies_per_env, ENV_STRIDE) per-env conditions, borrowed, or nullptr
+    long long bodies_per_env = 0;
     long long* robot_offsets = nullptr;  // (n_robots_var + 1,) body offsets of unequal robots, or nullptr
     long long n_robots_var = 0;
     int max_ctas_per_sm = 0;   // 0 = as many as fit
@@ -128,6 +130,13 @@ static WaveArgs wave_args(const h2o_engine* e)
     WaveArgs w;
     w.tab = e->wave_tab; w.clock = e->wave_clock; w.depth = e->wave_depth; w.n = e->n_waves;
     return w;
+}
+
+static EnvArgs env_args(const h2o_engine* e)
+{
+    EnvArgs v;
+    v.cond = e->env_cond; v.bodies_per_env = e->bodies_per_env;
+    return v;
 }
 
 static h2o_engine* check(h2o_handle h)
@@ -289,6 +298,7 @@ static int launch_direct(h2o_engine* e, const StepArgs& a, long long body_begin,
     if (cnt <= 0) return H2O_OK;
     const int grid = int((cnt + 255) / 256);
     const WaveArgs wv = wave_args(e);
+    const EnvArgs ev = env_args(e);
     const size_t smem = wave_smem_bytes(wv.n);
     if (e->dry_run) {
         e->launches += 1;
@@ -306,9 +316,9 @@ static int launch_direct(h2o_engine* e, const StepArgs& a, long long body_begin,
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, step_direct_kernel<S, kLayout, kParam, kStats>, a, body_begin, wv));
+        CUDA_TRY(cudaLaunchKernelEx(&cfg, step_direct_kernel<S, kLayout, kParam, kStats>, a, body_begin, wv, ev));
     } else {
-        step_direct_kernel<S, kLayout, kParam, kStats><<<grid, 256, smem, stream>>>(a, body_begin, wv);
+        step_direct_kernel<S, kLayout, kParam, kStats><<<grid, 256, smem, stream>>>(a, body_begin, wv, ev);
     }
     CUDA_TRY(cudaGetLastError());
     e->launches += 1;
@@ -349,7 +359,8 @@ static int step_typed2(h2o_engine* e, StepArgs& a, cudaStream_t stream)
     if (e->kernel_choice == H2O_KERNEL_TILE) use_tile = true;
     else if (e->kernel_choice == H2O_KERNEL_AUTO) use_tile = a.n >= (long long)e->sm_count * 256;
     if (TB == 0 || !ptr_ok || a.n < TB) use_tile = false;
-    if (a.am_dense || a.surface_eta || e->n_waves || a.warp_compat) use_tile = false;  // f3 / f4 modes: direct kernel (+ robot_wrench_kernel)
+    if (a.am_dense || a.surface_eta || e->n_waves || e->env_cond || a.warp_compat)
+        use_tile = false;  // f3 / f4 modes: direct kernel (+ robot_wrench_kernel)
 
     long long done_bodies = 0;
     if (use_tile) {
@@ -703,6 +714,76 @@ int h2o_wave_sample(h2o_handle h, const void* points, int64_t m, double* out, h2
     else
         wave_sample_kernel<double><<<grid, 256, smem, s>>>(wave_args(e), e->surface_z, static_cast<const double*>(points), m,
                                                            out);
+    CUDA_TRY(cudaGetLastError());
+    return H2O_OK;
+}
+
+int h2o_set_env_conditions(h2o_handle h, int64_t bodies_per_env, const double* cond_dev)
+{
+    h2o_engine* e = check(h);
+    if (!e) return H2O_ERR_BAD_HANDLE;
+    const bool remove = bodies_per_env == 0 || !cond_dev;
+    if (!remove) {  // every check before the captured rollout is dropped: a refused call leaves it intact
+        if (bodies_per_env < 0) return fail(H2O_ERR_BAD_ARGUMENT, "bodies_per_env must be >= 0");
+        if (e->n % bodies_per_env != 0)
+            return fail(H2O_ERR_BAD_SHAPE, "bodies_per_env %lld does not divide n_bodies %lld", (long long)bodies_per_env,
+                        (long long)e->n);
+        if (reinterpret_cast<uintptr_t>(cond_dev) & 7u) return fail(H2O_ERR_ALIGNMENT, "cond is not 8-byte aligned");
+        cudaPointerAttributes attr;
+        if (cudaPointerGetAttributes(&attr, cond_dev) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(H2O_ERR_BAD_DEVICE, "cond is not a CUDA pointer");
+        }
+        if ((attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged) || attr.device != e->device)
+            return fail(H2O_ERR_BAD_DEVICE, "cond must be device memory on device %d", e->device);
+    }
+    { DeviceGuard gi(e->device); invalidate_graph(e); }
+    e->env_cond = remove ? nullptr : cond_dev;
+    e->bodies_per_env = remove ? 0 : bodies_per_env;
+    return H2O_OK;
+}
+
+int h2o_reset_envs(h2o_handle h, const uint8_t* env_mask_dev, int restart_waves, h2o_stream stream)
+{
+    h2o_engine* e = check(h);
+    if (!e) return H2O_ERR_BAD_HANDLE;
+    if (!e->env_cond) return fail(H2O_ERR_NOT_CONFIGURED, "no env conditions set (h2o_set_env_conditions)");
+    if (!env_mask_dev) return fail(H2O_ERR_BAD_ARGUMENT, "env_mask is NULL");
+    DeviceGuard g(e->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int grid = int((e->n + 255) / 256);
+    // the borrowed array is the caller's writable tensor; only restart_waves writes to it (column ENV_TAU)
+    double* cond = const_cast<double*>(e->env_cond);
+    if (e->dtype == H2O_F32)
+        reset_envs_kernel<float><<<grid, 256, 0, s>>>(static_cast<float*>(e->prev), e->n, cond, e->bodies_per_env,
+                                                      env_mask_dev, restart_waves != 0, e->wave_clock);
+    else
+        reset_envs_kernel<double><<<grid, 256, 0, s>>>(static_cast<double*>(e->prev), e->n, cond, e->bodies_per_env,
+                                                       env_mask_dev, restart_waves != 0, e->wave_clock);
+    CUDA_TRY(cudaGetLastError());
+    return H2O_OK;
+}
+
+int h2o_wave_sample_env(h2o_handle h, const void* points, const int32_t* env_index, int64_t m, double* out,
+                        h2o_stream stream)
+{
+    h2o_engine* e = check(h);
+    if (!e) return H2O_ERR_BAD_HANDLE;
+    if (!e->env_cond) return fail(H2O_ERR_NOT_CONFIGURED, "no env conditions set (h2o_set_env_conditions)");
+    if (m < 0) return fail(H2O_ERR_BAD_ARGUMENT, "m must be >= 0");
+    if (m == 0) return H2O_OK;
+    if (!points || !env_index || !out) return fail(H2O_ERR_BAD_ARGUMENT, "NULL points / env_index / out");
+    DeviceGuard g(e->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int grid = int((m + 255) / 256);
+    const size_t smem = (size_t(e->n_waves) * WAVE_STRIDE + 1) * sizeof(double);
+    const long long n_envs = e->n / e->bodies_per_env;
+    if (e->dtype == H2O_F32)
+        wave_sample_env_kernel<float><<<grid, 256, smem, s>>>(wave_args(e), env_args(e), n_envs, e->surface_z,
+                                                              static_cast<const float*>(points), env_index, m, out);
+    else
+        wave_sample_env_kernel<double><<<grid, 256, smem, s>>>(wave_args(e), env_args(e), n_envs, e->surface_z,
+                                                               static_cast<const double*>(points), env_index, m, out);
     CUDA_TRY(cudaGetLastError());
     return H2O_OK;
 }
@@ -1286,6 +1367,7 @@ int h2o_rollout_persistent(h2o_handle h, int n_steps, double dt, double gravity,
     a.surface_z = e->surface_z;
     a.no_fallback = e->no_fallback;
     a.waves = wave_args(e);
+    a.envs = env_args(e);
     const size_t smem = wave_smem_bytes(e->n_waves);
     // small batches: one warp per CTA so that the warps spread over the SMs (a lone warp per scheduler
     // issues back to back); large batches: ordinary 128-thread CTAs
@@ -1293,13 +1375,17 @@ int h2o_rollout_persistent(h2o_handle h, int n_steps, double dt, double gravity,
     const int grid = int((e->n + block - 1) / block);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const bool st = e->stats_on;
+    const bool env = e->env_cond != nullptr;
+#define H2O_ROLLOUT(S, ST, ENV) \
+    if (st == ST && env == ENV) rollout_persistent_kernel<S, ST, ENV><<<grid, block, smem, s>>>(a)
     if (e->dtype == H2O_F32) {
-        if (st) rollout_persistent_kernel<float, true><<<grid, block, smem, s>>>(a);
-        else rollout_persistent_kernel<float, false><<<grid, block, smem, s>>>(a);
+        H2O_ROLLOUT(float, true, true); H2O_ROLLOUT(float, true, false);
+        H2O_ROLLOUT(float, false, true); H2O_ROLLOUT(float, false, false);
     } else {
-        if (st) rollout_persistent_kernel<double, true><<<grid, block, smem, s>>>(a);
-        else rollout_persistent_kernel<double, false><<<grid, block, smem, s>>>(a);
+        H2O_ROLLOUT(double, true, true); H2O_ROLLOUT(double, true, false);
+        H2O_ROLLOUT(double, false, true); H2O_ROLLOUT(double, false, false);
     }
+#undef H2O_ROLLOUT
     CUDA_TRY(cudaGetLastError());
     e->launches += 1;
     e->last_kernel = H2O_KERNEL_DIRECT;

@@ -103,6 +103,14 @@ struct WaveArgs {
     int n;
 };
 
+// Optional per-env water conditions (h2o_set_env_conditions): the borrowed (E, ENV_STRIDE) float64 array, read by
+// every launch, and the env size; body i (global index) belongs to env i / bodies_per_env.  cond == nullptr = none.
+// Like WaveArgs, a parameter of the per-body kernels only.
+struct EnvArgs {
+    const double* cond;
+    long long bodies_per_env;
+};
+
 // ---------------------------------------------------------------------------
 // PTX wrappers: mbarrier + bulk async copies (TMA engine, SASS UBLKCP)
 // ---------------------------------------------------------------------------
@@ -991,7 +999,8 @@ __device__ __forceinline__ void stage_waves(double* dst, const double* tab, cons
 
 template <typename S, int kLayout, int kParam, bool kStats>
 __global__ void __launch_bounds__(256) step_direct_kernel(const __grid_constant__ StepArgs a, long long body_begin,
-                                                          const __grid_constant__ WaveArgs wv)
+                                                          const __grid_constant__ WaveArgs wv,
+                                                          const __grid_constant__ EnvArgs ev)
 {
     __shared__ S table[(kParam == PARAM_TABLE) ? MAX_TABLE_TYPES * N_COEFF : 1];
     __shared__ unsigned char slot_map[(kParam == PARAM_TABLE) ? MAX_TABLE_SLOTS : 1];
@@ -1032,11 +1041,13 @@ __global__ void __launch_bounds__(256) step_direct_kernel(const __grid_constant_
         }
         BodyIn<double, S> bin;
         Env env{a.current[0], a.current[1], a.current[2], a.surface_z};
-        if (wv.n) {
-            const WaveSample w = wave_eval<sizeof(S) == 4>(wave_smem, wv.n, wv.depth, double(r.px), double(r.py),
-                                                           double(r.pz) - a.surface_z, wave_smem[wv.n * WAVE_STRIDE]);
-            env.surface_z += w.eta;
-            env.cx += w.ux; env.cy += w.uy; env.cz += w.uz;
+        if (wv.n || ev.cond) {
+            EnvRow row{};
+            if (ev.cond) row = env_row(ev.cond, (a.first_body + i) / ev.bodies_per_env);
+            const Water w = water_at<sizeof(S) == 4>(a.current, a.surface_z, ev.cond != nullptr, row, wave_smem, wv.n,
+                                                     wv.depth, wv.n ? wave_smem[wv.n * WAVE_STRIDE] : 0.0, double(r.px),
+                                                     double(r.py), double(r.pz));
+            env = Env{w.cx, w.cy, w.cz, w.surface_z};
         }
         if (a.surface_eta) env.surface_z += double(reinterpret_cast<const S*>(a.surface_eta)[i]);
         make_body_in<S>(r, cl, a.quat_wxyz, a.rho, a.grav, S(a.inv_dt), env, bin);
@@ -1346,10 +1357,12 @@ struct RolloutArgs {
     double current[3], surface_z;
     int no_fallback;
     WaveArgs waves;  // evaluated at each step's position and at t, t + dt, ... from the clock
+    EnvArgs envs;    // each body's env row is read once, at kernel start
 };
 
-// Dynamic shared memory: wave_smem_bytes(a.waves.n).
-template <typename S, bool kStats>
+// Dynamic shared memory: wave_smem_bytes(a.waves.n).  kEnv: a.envs.cond is set (a separate instantiation, so that
+// the env row held in registers costs nothing without conditions).
+template <typename S, bool kStats, bool kEnv>
 __global__ void rollout_persistent_kernel(const __grid_constant__ RolloutArgs a)
 {
     extern __shared__ double wave_smem[];
@@ -1377,17 +1390,17 @@ __global__ void rollout_persistent_kernel(const __grid_constant__ RolloutArgs a)
         r.vx = V[0]; r.vy = V[1]; r.vz = V[2];
         r.wx = W[0]; r.wy = W[1]; r.wz = W[2];
         r.pvx = PV[0]; r.pvy = PV[1]; r.pvz = PV[2]; r.pwx = PV[3]; r.pwy = PV[4]; r.pwz = PV[5];
-        const Env env0{a.current[0], a.current[1], a.current[2], a.surface_z};
+        EnvRow row{};
+        if (kEnv) row = env_row(a.envs.cond, i / a.envs.bodies_per_env);
         const S inv_dt = S(1.0 / a.dt);
         S F[3] = {S(0), S(0), S(0)}, T[3] = {S(0), S(0), S(0)};
         double t = wv.n ? wave_smem[wv.n * WAVE_STRIDE] : 0.0;
         for (int step = 0; step < a.n_steps; ++step) {
-            Env env = env0;
-            if (wv.n) {
-                const WaveSample w = wave_eval<sizeof(S) == 4>(wave_smem, wv.n, wv.depth, double(r.px),
-                                                               double(r.py), double(r.pz) - a.surface_z, t);
-                env.surface_z += w.eta;
-                env.cx += w.ux; env.cy += w.uy; env.cz += w.uz;
+            Env env{a.current[0], a.current[1], a.current[2], a.surface_z};
+            if (wv.n || kEnv) {
+                const Water w = water_at<sizeof(S) == 4>(a.current, a.surface_z, kEnv, row, wave_smem,
+                                                         wv.n, wv.depth, t, double(r.px), double(r.py), double(r.pz));
+                env = Env{w.cx, w.cy, w.cz, w.surface_z};
                 t += a.dt;  // the same sequence of additions as advance_clock_kernel over single steps
             }
             BodyIn<double, S> bin;
@@ -1487,6 +1500,48 @@ __global__ void __launch_bounds__(256) wave_sample_kernel(const __grid_constant_
                                                    double(p[2]) - surface_z, wave_smem[wv.n * WAVE_STRIDE]);
     double* o = out + 4 * i;
     o[0] = w.eta; o[1] = w.ux; o[2] = w.uy; o[3] = w.uz;
+}
+
+// Per-env sampling (h2o_wave_sample_env): point k seen from env env_index[k] -> out row [s eta, s u] (the field
+// alone, through water_at); an index outside [0, n_envs) gives a NaN row.  Dynamic shared memory as above.
+template <typename S>
+__global__ void __launch_bounds__(256) wave_sample_env_kernel(const __grid_constant__ WaveArgs wv,
+                                                              const __grid_constant__ EnvArgs ev, long long n_envs,
+                                                              double surface_z, const S* points,
+                                                              const int32_t* env_index, long long m, double* out)
+{
+    extern __shared__ double wave_smem[];
+    stage_waves(wave_smem, wv.tab, wv.clock, wv.n);
+    __syncthreads();
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    double* o = out + 4 * i;
+    const long long e = env_index[i];
+    if (e < 0 || e >= n_envs) {
+        o[0] = o[1] = o[2] = o[3] = __longlong_as_double(0x7ff8000000000000ll);
+        return;
+    }
+    const S* p = points + 3 * i;
+    const double zero[3] = {0.0, 0.0, 0.0};
+    const Water w = water_at<sizeof(S) == 4>(zero, surface_z, true, env_row(ev.cond, e), wave_smem, wv.n, wv.depth,
+                                             wave_smem[wv.n * WAVE_STRIDE], double(p[0]), double(p[1]), double(p[2]));
+    o[0] = w.field.eta; o[1] = w.field.ux; o[2] = w.field.uy; o[3] = w.field.uz;
+}
+
+// Masked env reset (h2o_reset_envs), one thread per body: the carried [v, omega] of every body of a masked env
+// becomes 0; with restart, the env's first body also sets the env's tau to -clock, so that its next step sees its
+// sea at env time clock + tau = 0 exactly.
+template <typename S>
+__global__ void __launch_bounds__(256) reset_envs_kernel(S* prev, long long n, double* cond, long long bodies_per_env,
+                                                         const uint8_t* mask, int restart, const double* clock)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const long long e = i / bodies_per_env;
+    if (!mask[e]) return;
+#pragma unroll
+    for (int k = 0; k < 6; ++k) prev[6 * i + k] = S(0);
+    if (restart && i == e * bodies_per_env) cond[ENV_STRIDE * e + ENV_TAU] = -*clock;
 }
 
 }  // namespace h2o

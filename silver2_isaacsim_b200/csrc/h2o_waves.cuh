@@ -10,6 +10,8 @@
 // S_j = sinh(k_j (z + h)) / sinh(k_j h) (finite depth) or C_j = S_j = exp(k_j z) (deep water).
 // The hyperbolic ratios are evaluated as (e^{kz} +- e^{-k(z + 2h)}) / (1 - e^{-2kh}): no overflow at
 // any k h, and the denominator comes from the table (computed once on the host with expm1).
+// water_at composes the field with the global environment and a per-env conditions row
+// (h2o_set_env_conditions) into the waterline and flow a body sees.
 #pragma once
 
 #include "h2o_model.cuh"
@@ -108,6 +110,73 @@ H2O_HD WaveSample wave_eval(const double* tab, int n, double depth, double px, d
         s.uz += c[WAVE_A_OMEGA] * S * sn;
     }
     return s;
+}
+
+// ---------------------------------------------------------------------------
+// Per-env water conditions (h2o_set_env_conditions): one float64 row per env of bodies_per_env contiguous
+// bodies, cond[e] = [cx, cy, cz, dz, s, tau, x0, y0].
+// ---------------------------------------------------------------------------
+enum : int {
+    ENV_CX = 0, ENV_CY, ENV_CZ,  // current added to the global current
+    ENV_DZ,                      // water-level offset added to surface_z
+    ENV_SCALE,                   // wave scale s
+    ENV_TAU,                     // wave time offset (s)
+    ENV_X0, ENV_Y0,              // env origin
+    ENV_STRIDE
+};
+
+struct EnvRow {
+    double c[ENV_STRIDE];
+};
+
+H2O_HD EnvRow env_row(const double* cond, long long e)
+{
+    EnvRow r;
+    for (int k = 0; k < ENV_STRIDE; ++k) r.c[k] = cond[ENV_STRIDE * e + k];
+    return r;
+}
+
+// What a body sees: the waterline (before a caller height array is added), the flow, and the env's field alone
+// (s * eta, s * u; zeros without a wave field).
+struct Water {
+    double surface_z, cx, cy, cz;
+    WaveSample field;
+};
+
+// The one composition of the global environment (current, surface_z), the env row (has_row), the wave table and
+// the clock value t for a body at p, used by every step kernel, the sampler and the host emulator.  With a row,
+// every operation is a separately rounded float64 operation in the order include/h2o.h gives:
+//   L = surface_z + dz,  field = s * wave_eval(p_x - x0, p_y - y0, p_z - L, t + tau),
+//   waterline = L + s eta,  flow = (current + c) + s u.
+// The identity row [0,0,0,0,1,0,0,0] makes each of them exact, so it reproduces the row-less result bit for bit.
+template <bool kF32>
+H2O_HD Water water_at(const double current[3], double surface_z, bool has_row, const EnvRow& row, const double* tab,
+                      int n_waves, double depth, double t, double px, double py, double pz)
+{
+    Water w{surface_z, current[0], current[1], current[2], {0.0, 0.0, 0.0, 0.0}};
+    const double* c = row.c;
+    if (has_row) {
+        w.surface_z = wave_add(surface_z, c[ENV_DZ]);
+        w.cx = wave_add(current[0], c[ENV_CX]);
+        w.cy = wave_add(current[1], c[ENV_CY]);
+        w.cz = wave_add(current[2], c[ENV_CZ]);
+        px = wave_add(px, -c[ENV_X0]);
+        py = wave_add(py, -c[ENV_Y0]);
+        t = wave_add(t, c[ENV_TAU]);
+    }
+    if (n_waves) {
+        w.field = wave_eval<kF32>(tab, n_waves, depth, px, py, pz - w.surface_z, t);  // the one call site
+        if (has_row) {
+            const double s = c[ENV_SCALE];
+            w.field = WaveSample{wave_mul(s, w.field.eta), wave_mul(s, w.field.ux), wave_mul(s, w.field.uy),
+                                 wave_mul(s, w.field.uz)};
+        }
+        w.surface_z = wave_add(w.surface_z, w.field.eta);
+        w.cx = wave_add(w.cx, w.field.ux);
+        w.cy = wave_add(w.cy, w.field.uy);
+        w.cz = wave_add(w.cz, w.field.uz);
+    }
+    return w;
 }
 
 }  // namespace h2o

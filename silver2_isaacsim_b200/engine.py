@@ -155,16 +155,89 @@ class HydroEngine:
             raise ValueError("wave time must be finite")
         L.check(self._lib.h2o_wave_time_write(self._h, t, _stream_ptr(self.device)))
 
-    def sample_waves(self, points) -> torch.Tensor:
+    def sample_waves(self, points, env=None) -> torch.Tensor:
         """Wave field at ``points`` (m,3) world positions and the current clock, with the step's evaluator and
-        precision: a (m,4) float64 CUDA tensor of rows ``eta, ux, uy, uz`` (zeros without a field)."""
+        precision: a (m,4) float64 CUDA tensor of rows ``eta, ux, uy, uz`` (zeros without a field).  With ``env``
+        (one env index per point, or one for all), each point is seen from that env: rows ``s eta, s u`` at
+        ``p - origin`` and ``clock + tau`` (``waves.evaluate_env``); an index outside ``[0, E)`` gives a NaN row."""
         pts = self._as_dev(points)
         if pts.ndim != 2 or pts.shape[1] != 3:
             raise ValueError(f"points must be (m,3), got {tuple(pts.shape)}")
         out = torch.empty(pts.shape[0], 4, dtype=torch.float64, device=self.device)
-        L.check(self._lib.h2o_wave_sample(self._h, ctypes.c_void_p(pts.data_ptr()), int(pts.shape[0]),
-                                          ctypes.c_void_p(out.data_ptr()), _stream_ptr(self.device)))
+        if env is None:
+            L.check(self._lib.h2o_wave_sample(self._h, ctypes.c_void_p(pts.data_ptr()), int(pts.shape[0]),
+                                              ctypes.c_void_p(out.data_ptr()), _stream_ptr(self.device)))
+            return out
+        idx = torch.as_tensor(env, device=self.device)
+        if idx.dtype.is_floating_point or idx.dtype == torch.bool:
+            raise ValueError("env must hold integer env indices")
+        idx = idx.reshape(-1).long().clamp(-1, 2 ** 31 - 1).to(torch.int32)  # no wrap-around into [0, E)
+        if idx.numel() == 1:
+            idx = idx.expand(pts.shape[0])
+        idx = idx.contiguous()
+        if tuple(idx.shape) != (pts.shape[0],):
+            raise ValueError(f"env must be one index or one per point ({pts.shape[0]}), got {tuple(idx.shape)}")
+        L.check(self._lib.h2o_wave_sample_env(self._h, ctypes.c_void_p(pts.data_ptr()), ctypes.c_void_p(idx.data_ptr()),
+                                              int(pts.shape[0]), ctypes.c_void_p(out.data_ptr()),
+                                              _stream_ptr(self.device)))
         return out
+
+    def set_env_conditions(self, cond: Optional[torch.Tensor], bodies_per_env: int = 0):
+        """Per-env water conditions: ``cond`` is a contiguous (E,8) float64 tensor on the engine's device
+        (``waves.env_conditions`` builds one), rows ``cx, cy, cz, dz, s, tau, x0, y0`` for envs of
+        ``bodies_per_env`` contiguous bodies (E = n_bodies / bodies_per_env).  The env's current adds to the global
+        one, its level to ``surface_z``; its sea is the wave field scaled by ``s`` at ``p - origin`` and
+        ``clock + tau`` (include/h2o.h).  The tensor is borrowed, not copied: in-place edits reach the next step and
+        the next replay of a captured rollout.  ``None`` removes the conditions.  Steps then run on the per-body
+        kernel; ``rollout_persistent`` follows them; ``components`` ignores them."""
+        if cond is None:
+            L.check(self._lib.h2o_set_env_conditions(self._h, 0, None))
+            self._cond = None
+            return
+        bpe = int(bodies_per_env)
+        if not isinstance(cond, torch.Tensor):
+            raise ValueError("cond must be a torch tensor (waves.env_conditions gives the NumPy rows)")
+        if bpe < 1:
+            raise ValueError(f"bodies_per_env must be >= 1, got {bodies_per_env}")
+        if self.n_bodies % bpe:  # the library reports BAD_SHAPE
+            L.check(self._lib.h2o_set_env_conditions(self._h, bpe, ctypes.c_void_p(cond.data_ptr())))
+        n_envs = self.n_bodies // bpe
+        if (cond.dtype != torch.float64 or cond.device != self.device or tuple(cond.shape) != (n_envs, W.COND_COLS)
+                or not cond.is_contiguous()):
+            raise ValueError(f"cond must be a contiguous ({n_envs},{W.COND_COLS}) torch.float64 tensor on {self.device}, "
+                             f"got {tuple(cond.shape)} {cond.dtype} on {cond.device}")
+        L.check(self._lib.h2o_set_env_conditions(self._h, bpe, ctypes.c_void_p(cond.data_ptr())))
+        self._cond = cond  # keep the borrowed memory alive
+
+    @property
+    def env_conditions(self) -> Optional[torch.Tensor]:
+        """The borrowed (E,8) conditions tensor, or ``None``."""
+        return getattr(self, "_cond", None)
+
+    def reset_envs(self, envs, restart_waves: bool = False):
+        """Forget the previous-step velocities of the bodies of some envs (the per-env ``_reset``,
+        hydrodynamics_behavior.py:240-245): ``envs`` is a bool mask (E,) or env ids.  With ``restart_waves`` those
+        envs' ``tau`` becomes ``-clock``, so that their next step sees their sea at env time 0.  Stream-ordered, no
+        host synchronisation (except to range-check env ids held on the device); a captured rollout is kept."""
+        cond = self.env_conditions
+        if cond is None:  # the library reports NOT_CONFIGURED
+            L.check(self._lib.h2o_reset_envs(self._h, None, int(bool(restart_waves)), _stream_ptr(self.device)))
+        n_envs = cond.shape[0]
+        envs = torch.as_tensor(envs)
+        if envs.dtype == torch.bool:
+            if tuple(envs.shape) != (n_envs,):
+                raise ValueError(f"a mask must be ({n_envs},), got {tuple(envs.shape)}")
+            mask = envs.to(device=self.device, dtype=torch.uint8).contiguous()
+        elif not envs.dtype.is_floating_point:
+            ids = envs.reshape(-1).long()
+            if ids.numel() and (int(ids.min()) < 0 or int(ids.max()) >= n_envs):
+                raise ValueError(f"env ids must be in [0, {n_envs})")
+            mask = torch.zeros(n_envs, dtype=torch.uint8, device=self.device)
+            mask[ids.to(self.device)] = 1
+        else:
+            raise ValueError("envs must be a bool mask or integer env ids")
+        L.check(self._lib.h2o_reset_envs(self._h, ctypes.c_void_p(mask.data_ptr()), int(bool(restart_waves)),
+                                         _stream_ptr(self.device)))
 
     def set_added_mass_dense(self, matrices=None, slot_type=None):
         """Dense 6x6 body-frame added-mass matrices (the argument ``calculate_added_mass`` takes,

@@ -112,10 +112,22 @@ def jonswap(hs: float, tp: float, gamma: float = 3.3, n_components: int = 32, di
     return WaveField(comps, depth)
 
 
-def evaluate(field: WaveField, points, t: float, surface_z: float = 0.0) -> np.ndarray:
+def _per_point(x, m: int):
+    """A scalar stays a Python float; an array becomes an (m, 1) float64 column."""
+    if np.ndim(x) == 0:
+        return float(x)
+    x = np.asarray(x, dtype=np.float64).reshape(-1)
+    if x.shape != (m,):
+        raise ValueError(f"expected a scalar or {m} values, got {x.shape[0]}")
+    return x[:, None]
+
+
+def evaluate(field: WaveField, points, t, surface_z=0.0) -> np.ndarray:
     """Float64 reference of the field at ``points`` (m, 3) and clock ``t``: (m, 4) rows ``eta, ux, uy, uz``.
-    The phase is formed in the order the GPU evaluator forms it, ``((kx px + ky py) - omega t) + phase``."""
+    The phase is formed in the order the GPU evaluator forms it, ``((kx px + ky py) - omega t) + phase``.
+    ``t`` and ``surface_z`` are scalars or one value per point."""
     p = np.asarray(points, dtype=np.float64).reshape(-1, 3)
+    t, surface_z = _per_point(t, len(p)), _per_point(surface_z, len(p))
     c = field.components
     a, kx, ky, w, ph = (c[:, j][None, :] for j in range(5))
     k = np.hypot(kx, ky)
@@ -137,3 +149,56 @@ def evaluate(field: WaveField, points, t: float, surface_z: float = 0.0) -> np.n
     out[:, 2] = (uh * (ky / k)).sum(axis=1)
     out[:, 3] = (a * w * S * sn).sum(axis=1)
     return out
+
+
+# Columns of a per-env conditions row (HydroEngine.set_env_conditions, h2o_set_env_conditions)
+COND_CX, COND_CY, COND_CZ, COND_DZ, COND_SCALE, COND_TAU, COND_X0, COND_Y0 = range(8)
+COND_COLS = 8
+
+
+def _cond_column(x, n: int, width: int, name: str) -> np.ndarray:
+    a = np.asarray(x, dtype=np.float64)
+    if a.ndim == 0 or a.shape == (width,):
+        a = np.broadcast_to(a, (n, width))
+    elif width == 1 and a.shape == (n,):
+        a = a[:, None]
+    if a.shape != (n, width):
+        shapes = "a scalar or (E,)" if width == 1 else f"a scalar, ({width},) or (E, {width})"
+        raise ValueError(f"{name} must be {shapes} with E = {n}, got {np.shape(x)}")
+    if not np.isfinite(a).all():
+        raise ValueError(f"{name} must be finite")
+    return a
+
+
+def env_conditions(n_envs: int, current=0.0, surface_dz=0.0, wave_scale=1.0, time_offset=0.0, origin=0.0) -> np.ndarray:
+    """Per-env conditions, an (E, 8) float64 array of rows ``cx, cy, cz, dz, s, tau, x0, y0``: the current added to
+    the global one, the water-level offset, the wave scale, the wave time offset (s) and the env origin.  Each
+    argument is a scalar, one value for every env (``current`` (3,), ``origin`` (2,)) or one per env; the
+    defaults make identity rows ``[0, 0, 0, 0, 1, 0, 0, 0]``, which leave every result unchanged."""
+    n = int(n_envs)
+    if n < 1:
+        raise ValueError(f"n_envs must be >= 1, got {n_envs}")
+    cond = np.empty((n, COND_COLS))
+    cond[:, COND_CX:COND_CZ + 1] = _cond_column(current, n, 3, "current")
+    cond[:, COND_DZ] = _cond_column(surface_dz, n, 1, "surface_dz")[:, 0]
+    cond[:, COND_SCALE] = _cond_column(wave_scale, n, 1, "wave_scale")[:, 0]
+    cond[:, COND_TAU] = _cond_column(time_offset, n, 1, "time_offset")[:, 0]
+    cond[:, COND_X0:COND_Y0 + 1] = _cond_column(origin, n, 2, "origin")
+    return cond
+
+
+def evaluate_env(field: WaveField, points, t: float, cond, env_index, surface_z: float = 0.0) -> np.ndarray:
+    """Float64 reference of what env ``env_index[k]`` sees of the field at ``points[k]`` and clock ``t``:
+    ``s * evaluate(field, p - origin, t + tau, surface_z + dz)`` with the env's row of ``cond`` (E, 8), as rows
+    ``s eta, s ux, s uy, s uz`` (the field alone, as ``HydroEngine.sample_waves(points, env)`` returns it)."""
+    p = np.array(points, dtype=np.float64).reshape(-1, 3)
+    cond = np.asarray(cond, dtype=np.float64)
+    if cond.ndim != 2 or cond.shape[1] != COND_COLS:
+        raise ValueError(f"cond must be (E, {COND_COLS}), got {cond.shape}")
+    r = cond[np.asarray(env_index, dtype=np.int64).reshape(-1)]
+    if len(r) != len(p):
+        raise ValueError("need one env index per point")
+    p[:, 0] = p[:, 0] - r[:, COND_X0]
+    p[:, 1] = p[:, 1] - r[:, COND_Y0]
+    out = evaluate(field, p, t + r[:, COND_TAU], surface_z + r[:, COND_DZ])
+    return r[:, COND_SCALE:COND_SCALE + 1] * out
