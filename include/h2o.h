@@ -134,7 +134,8 @@ H2O_API int h2o_set_environment(h2o_handle h, const double current_xyz[3], doubl
  * memory.  Steps with a wave field run on the per-body kernel; h2o_components ignores the field (as it ignores
  * a height field).  Like every h2o_set_* call this drops a captured rollout. */
 H2O_API int h2o_set_wave_field(h2o_handle h, int n_components, const double* comps, double depth);
-/* The wave clock, stream-ordered.  The read synchronises the stream.  Neither drops a captured rollout: the graph
+/* The water clock (read by the wave field and by a time-varying current grid, h2o_set_current_grid),
+ * stream-ordered.  The read synchronises the stream.  Neither drops a captured rollout: the graph
  * reads the clock from device memory, so a write between replays moves the field the replay sees. */
 H2O_API int h2o_wave_time_write(h2o_handle h, double t, h2o_stream stream);
 H2O_API int h2o_wave_time_read(h2o_handle h, double* t, h2o_stream stream);
@@ -180,6 +181,46 @@ H2O_API int h2o_reset_envs(h2o_handle h, const uint8_t* env_mask_dev, int restar
  * H2O_ERR_NOT_CONFIGURED without conditions. */
 H2O_API int h2o_wave_sample_env(h2o_handle h, const void* points, const int32_t* env_index, int64_t m, double* out,
                                 h2o_stream stream);
+
+/* Gridded water current (SURVEY.md 8(f4)): a space-time lattice of velocity vectors, such as an ocean-model or ADCP
+ * field, a seabed boundary layer or a tidal sequence, interpolated on the device at every body on every step.
+ * grid_dev is a C-contiguous DEVICE array of float64 with shape (nt, nz, ny, nx, 3) (dims = [nt, nz, ny, nx]) on the
+ * handle's device, 8-byte aligned; geom = [gx, gy, gz, hx, hy, hz, t0, ht] (host).  Node (f, k, j, i) sits at
+ * x = gx + i hx, y = gy + j hy, z = gz + k hz and at time t0 + f ht.
+ * A body (or sample point) at p with water-clock value t is located, with L = surface_z + dz the env's mean level
+ * (dz = 0, x0 = y0 = tau = 0 without env conditions):
+ *   X = p_x - x0,  Y = p_y - y0  (env-local, as for waves)
+ *   Z = p_z - L                  (from the env's mean level, not from the instantaneous waterline)
+ *   T = t + tau                  (env time: h2o_reset_envs(..., restart_waves=1) also restarts an env's frames)
+ * On each axis of n nodes, origin o and spacing h, at coordinate q: n == 1 gives index 0 and weight 0 (the axis is
+ * constant and no neighbour is read); otherwise u = (q - o) / h clamped to [0, n - 1], i = min(floor(u), n - 2),
+ * w = u - i.  Outside the lattice, and before the first or after the last frame, the value is held at the
+ * boundary.  Each interpolation is lerp(a, b, w) = a + w (b - a), three separately rounded float64 operations,
+ * along x, then y, then z, then t, for each component.  A NaN coordinate gives a NaN value; no input reads outside
+ * the array.  The grid value g joins the flow, every addition a separately rounded float64 operation:
+ *   flow = ((current + c_e) + g) + s u         (without env conditions: (current + g) + u)
+ * fp32 mode sums the flow in double and rounds it once to the handle dtype.  The waterline is unchanged.  So a grid
+ * of zeros gives the results of no grid, and a uniform grid of value g with a zero global current gives, bit for
+ * bit, the results of no grid and h2o_set_environment(current = g) (h2o_rollout_persistent with a grid runs its own
+ * kernel instantiation, whose multiply-add contraction may differ: to rounding there).  Only the model's inputs change, as for waves:
+ * accelerations stay differences of body velocities and no fluid-acceleration term is added.
+ * The array is borrowed, not copied: every later step reads it, so the caller may edit it in place between steps
+ * or graph replays with no recapture (streaming new frames in).  It must stay allocated while set.
+ * grid_dev == NULL removes the grid.  H2O_ERR_BAD_ARGUMENT for a dim < 1, a total size that overflows, non-finite
+ * geometry, a spacing hx, hy, hz <= 0 or ht <= 0 with nt > 1; H2O_ERR_ALIGNMENT / H2O_ERR_BAD_DEVICE for a
+ * misaligned pointer or one not on the handle's device.  Steps with a grid run on the per-body kernel;
+ * h2o_rollout_persistent re-evaluates the grid at every step; h2o_components ignores it.  Like every h2o_set_* call
+ * this drops a captured rollout; a refused call leaves it intact.
+ * Water clock: the clock of h2o_wave_time_write / _read.  It advances by dt after every step (and by K dt after a
+ * persistent rollout of K steps) whenever a wave field or a grid with nt > 1 is set. */
+H2O_API int h2o_set_current_grid(h2o_handle h, const double* grid_dev, const int64_t dims[4], const double geom[8]);
+/* What a step sees at given points and the clock's current value: points is a DEVICE array (m,3) in the handle
+ * dtype, out a DEVICE array (m,4) float64 of rows [waterline, flow_x, flow_y, flow_z] -- the full composition of
+ * global environment, env row, grid and wave field, before a caller height array (h2o_set_surface_heights) and
+ * before the fp32 rounding.  env_index (DEVICE int32 (m,)) applies env env_index[k]'s row to point k; NULL applies
+ * none; an index outside [0, E) gives a NaN row.  H2O_ERR_NOT_CONFIGURED for env_index without env conditions. */
+H2O_API int h2o_water_sample(h2o_handle h, const void* points, const int32_t* env_index, int64_t m, double* out,
+                             h2o_stream stream);
 
 /* Same twelve scalars, same order as the reference wrapper ctor
  * (numba_hydrodynamics_wrapper.py:9-10): width, depth, height, linear_drag_coefficient,

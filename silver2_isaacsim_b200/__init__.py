@@ -1,11 +1,11 @@
 """B200-native hydrodynamics force engine (drop-in for SILVER2's per-body force path).
 
-Light imports only: ``params`` / ``workloads`` / ``waves`` are NumPy-only; the engine classes are
+Light imports only: ``params`` / ``workloads`` / ``waves`` / ``currents`` are NumPy-only; the engine classes are
 imported lazily because they load the CUDA library (and fail loudly if it is missing).
 """
-from . import params, waves, workloads  # noqa: F401
+from . import currents, params, waves, workloads  # noqa: F401
 
-__all__ = ["params", "waves", "workloads", "HydroEngine", "WarpHydrodynamicsWrapper",
+__all__ = ["currents", "params", "waves", "workloads", "HydroEngine", "WarpHydrodynamicsWrapper",
            "NumbaHydrodynamicsWrapper", "H2OError"]
 
 

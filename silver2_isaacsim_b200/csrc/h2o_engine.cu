@@ -82,6 +82,7 @@ struct h2o_engine {
     double wave_depth = INFINITY;
     const double* env_cond = nullptr;  // (n / bodies_per_env, ENV_STRIDE) per-env conditions, borrowed, or nullptr
     long long bodies_per_env = 0;
+    GridArgs grid{};  // current grid (borrowed values, dims and geometry); grid.vals == nullptr = none
     long long* robot_offsets = nullptr;  // (n_robots_var + 1,) body offsets of unequal robots, or nullptr
     long long n_robots_var = 0;
     int max_ctas_per_sm = 0;   // 0 = as many as fit
@@ -138,6 +139,9 @@ static EnvArgs env_args(const h2o_engine* e)
     v.cond = e->env_cond; v.bodies_per_env = e->bodies_per_env;
     return v;
 }
+
+// The water clock advances after every step when something reads it: a wave field or a time-varying grid.
+static bool clock_runs(const h2o_engine* e) { return e->n_waves || (e->grid.vals && e->grid.nt > 1); }
 
 static h2o_engine* check(h2o_handle h)
 {
@@ -299,6 +303,7 @@ static int launch_direct(h2o_engine* e, const StepArgs& a, long long body_begin,
     const int grid = int((cnt + 255) / 256);
     const WaveArgs wv = wave_args(e);
     const EnvArgs ev = env_args(e);
+    const GridArgs gv = e->grid;
     const size_t smem = wave_smem_bytes(wv.n);
     if (e->dry_run) {
         e->launches += 1;
@@ -316,9 +321,9 @@ static int launch_direct(h2o_engine* e, const StepArgs& a, long long body_begin,
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, step_direct_kernel<S, kLayout, kParam, kStats>, a, body_begin, wv, ev));
+        CUDA_TRY(cudaLaunchKernelEx(&cfg, step_direct_kernel<S, kLayout, kParam, kStats>, a, body_begin, wv, ev, gv));
     } else {
-        step_direct_kernel<S, kLayout, kParam, kStats><<<grid, 256, smem, stream>>>(a, body_begin, wv, ev);
+        step_direct_kernel<S, kLayout, kParam, kStats><<<grid, 256, smem, stream>>>(a, body_begin, wv, ev, gv);
     }
     CUDA_TRY(cudaGetLastError());
     e->launches += 1;
@@ -359,7 +364,7 @@ static int step_typed2(h2o_engine* e, StepArgs& a, cudaStream_t stream)
     if (e->kernel_choice == H2O_KERNEL_TILE) use_tile = true;
     else if (e->kernel_choice == H2O_KERNEL_AUTO) use_tile = a.n >= (long long)e->sm_count * 256;
     if (TB == 0 || !ptr_ok || a.n < TB) use_tile = false;
-    if (a.am_dense || a.surface_eta || e->n_waves || e->env_cond || a.warp_compat)
+    if (a.am_dense || a.surface_eta || e->n_waves || e->env_cond || e->grid.vals || a.warp_compat)
         use_tile = false;  // f3 / f4 modes: direct kernel (+ robot_wrench_kernel)
 
     long long done_bodies = 0;
@@ -448,7 +453,7 @@ static int step_typed(h2o_engine* e, int layout, StepArgs& a, cudaStream_t strea
 #undef H2O_DISPATCH
 }
 
-// With a wave field: the clock advances by dt, n times, after the work already in `stream` (counted as a launch).
+// With a wave field or a time-varying grid: the clock advances by dt, n times, after the work already in `stream` (counted as a launch).
 static int advance_clock(h2o_engine* e, double dt, int n, cudaStream_t stream)
 {
     if (e->dry_run) {
@@ -461,7 +466,7 @@ static int advance_clock(h2o_engine* e, double dt, int n, cudaStream_t stream)
     return H2O_OK;
 }
 
-// Core step on device pointers (no validation beyond configuration).  tick: advance the wave clock after the
+// Core step on device pointers (no validation beyond configuration).  tick: advance the water clock after the
 // step's kernels (the chunked host pipeline advances it once after all chunks instead).
 static int step_device(h2o_engine* e, int layout, const void* pos, const void* quat, const void* lin,
                        const void* ang, double dt, void* f, void* t, void* w, long long n,
@@ -500,7 +505,7 @@ static int step_device(h2o_engine* e, int layout, const void* pos, const void* q
     a.redo_bitmap = e->redo_bitmap;
     a.surface_eta = e->surface_eta ? static_cast<const char*>(e->surface_eta) + size_t(first_body) * e->esz : nullptr;
     const int rc = e->dtype == H2O_F32 ? step_typed<float>(e, layout, a, stream) : step_typed<double>(e, layout, a, stream);
-    if (rc || !e->n_waves || !tick) return rc;
+    if (rc || !clock_runs(e) || !tick) return rc;
     return advance_clock(e, dt, 1, stream);
 }
 
@@ -784,6 +789,71 @@ int h2o_wave_sample_env(h2o_handle h, const void* points, const int32_t* env_ind
     else
         wave_sample_env_kernel<double><<<grid, 256, smem, s>>>(wave_args(e), env_args(e), n_envs, e->surface_z,
                                                                static_cast<const double*>(points), env_index, m, out);
+    CUDA_TRY(cudaGetLastError());
+    return H2O_OK;
+}
+
+int h2o_set_current_grid(h2o_handle h, const double* grid_dev, const int64_t dims[4], const double geom[8])
+{
+    h2o_engine* e = check(h);
+    if (!e) return H2O_ERR_BAD_HANDLE;
+    GridArgs g{};
+    if (grid_dev) {  // every check before the captured rollout is dropped: a refused call leaves it intact
+        if (!dims || !geom) return fail(H2O_ERR_BAD_ARGUMENT, "NULL dims / geom");
+        int64_t total = 3 * int64_t(sizeof(double));
+        for (int k = 0; k < 4; ++k) {
+            if (dims[k] < 1) return fail(H2O_ERR_BAD_ARGUMENT, "dims[%d] = %lld < 1", k, (long long)dims[k]);
+            if (__builtin_mul_overflow(total, dims[k], &total))
+                return fail(H2O_ERR_BAD_ARGUMENT, "grid of %lld x %lld x %lld x %lld x 3 doubles is too large",
+                            (long long)dims[0], (long long)dims[1], (long long)dims[2], (long long)dims[3]);
+        }
+        for (int k = 0; k < 8; ++k)
+            if (!std::isfinite(geom[k])) return fail(H2O_ERR_BAD_ARGUMENT, "geom[%d] is not finite", k);
+        if (!(geom[3] > 0.0 && geom[4] > 0.0 && geom[5] > 0.0))
+            return fail(H2O_ERR_BAD_ARGUMENT, "spacings hx, hy, hz must be > 0");
+        if (dims[0] > 1 && !(geom[7] > 0.0)) return fail(H2O_ERR_BAD_ARGUMENT, "frame interval ht must be > 0 when nt > 1");
+        if (reinterpret_cast<uintptr_t>(grid_dev) & 7u) return fail(H2O_ERR_ALIGNMENT, "grid is not 8-byte aligned");
+        cudaPointerAttributes attr;
+        if (cudaPointerGetAttributes(&attr, grid_dev) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(H2O_ERR_BAD_DEVICE, "grid is not a CUDA pointer");
+        }
+        if ((attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged) || attr.device != e->device)
+            return fail(H2O_ERR_BAD_DEVICE, "grid must be device memory on device %d", e->device);
+        g.vals = grid_dev;
+        g.nt = dims[0]; g.nz = dims[1]; g.ny = dims[2]; g.nx = dims[3];
+        g.gx = geom[0]; g.gy = geom[1]; g.gz = geom[2];
+        g.hx = geom[3]; g.hy = geom[4]; g.hz = geom[5];
+        g.t0 = geom[6]; g.ht = geom[7];
+    }
+    { DeviceGuard gi(e->device); invalidate_graph(e); }
+    e->grid = g;
+    return H2O_OK;
+}
+
+int h2o_water_sample(h2o_handle h, const void* points, const int32_t* env_index, int64_t m, double* out,
+                     h2o_stream stream)
+{
+    h2o_engine* e = check(h);
+    if (!e) return H2O_ERR_BAD_HANDLE;
+    if (env_index && !e->env_cond) return fail(H2O_ERR_NOT_CONFIGURED, "no env conditions set (h2o_set_env_conditions)");
+    if (m < 0) return fail(H2O_ERR_BAD_ARGUMENT, "m must be >= 0");
+    if (m == 0) return H2O_OK;
+    if (!points || !out) return fail(H2O_ERR_BAD_ARGUMENT, "NULL points / out");
+    DeviceGuard g(e->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int grid = int((m + 255) / 256);
+    const size_t smem = (size_t(e->n_waves) * WAVE_STRIDE + 1) * sizeof(double);
+    const long long n_envs = e->env_cond ? e->n / e->bodies_per_env : 0;
+    const double* c = e->current;
+    if (e->dtype == H2O_F32)
+        water_sample_kernel<float><<<grid, 256, smem, s>>>(wave_args(e), env_args(e), e->grid, n_envs, c[0], c[1],
+                                                           c[2], e->surface_z, static_cast<const float*>(points),
+                                                           env_index, m, out);
+    else
+        water_sample_kernel<double><<<grid, 256, smem, s>>>(wave_args(e), env_args(e), e->grid, n_envs, c[0], c[1],
+                                                            c[2], e->surface_z, static_cast<const double*>(points),
+                                                            env_index, m, out);
     CUDA_TRY(cudaGetLastError());
     return H2O_OK;
 }
@@ -1368,6 +1438,7 @@ int h2o_rollout_persistent(h2o_handle h, int n_steps, double dt, double gravity,
     a.no_fallback = e->no_fallback;
     a.waves = wave_args(e);
     a.envs = env_args(e);
+    a.grid = e->grid;
     const size_t smem = wave_smem_bytes(e->n_waves);
     // small batches: one warp per CTA so that the warps spread over the SMs (a lone warp per scheduler
     // issues back to back); large batches: ordinary 128-thread CTAs
@@ -1376,20 +1447,25 @@ int h2o_rollout_persistent(h2o_handle h, int n_steps, double dt, double gravity,
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const bool st = e->stats_on;
     const bool env = e->env_cond != nullptr;
-#define H2O_ROLLOUT(S, ST, ENV) \
-    if (st == ST && env == ENV) rollout_persistent_kernel<S, ST, ENV><<<grid, block, smem, s>>>(a)
+    const bool cg = e->grid.vals != nullptr;
+#define H2O_ROLLOUT(S, ST, ENV, CG) \
+    if (st == ST && env == ENV && cg == CG) rollout_persistent_kernel<S, ST, ENV, CG><<<grid, block, smem, s>>>(a)
+#define H2O_ROLLOUTS(S) \
+    H2O_ROLLOUT(S, true, true, false); H2O_ROLLOUT(S, true, false, false);   \
+    H2O_ROLLOUT(S, false, true, false); H2O_ROLLOUT(S, false, false, false); \
+    H2O_ROLLOUT(S, true, true, true); H2O_ROLLOUT(S, true, false, true);     \
+    H2O_ROLLOUT(S, false, true, true); H2O_ROLLOUT(S, false, false, true)
     if (e->dtype == H2O_F32) {
-        H2O_ROLLOUT(float, true, true); H2O_ROLLOUT(float, true, false);
-        H2O_ROLLOUT(float, false, true); H2O_ROLLOUT(float, false, false);
+        H2O_ROLLOUTS(float);
     } else {
-        H2O_ROLLOUT(double, true, true); H2O_ROLLOUT(double, true, false);
-        H2O_ROLLOUT(double, false, true); H2O_ROLLOUT(double, false, false);
+        H2O_ROLLOUTS(double);
     }
+#undef H2O_ROLLOUTS
 #undef H2O_ROLLOUT
     CUDA_TRY(cudaGetLastError());
     e->launches += 1;
     e->last_kernel = H2O_KERNEL_DIRECT;
-    if (e->n_waves) return advance_clock(e, dt, n_steps, s);
+    if (clock_runs(e)) return advance_clock(e, dt, n_steps, s);
     return H2O_OK;
 }
 
@@ -1611,7 +1687,7 @@ static int step_host_impl(h2o_engine* e, int layout, const void* const in[4], vo
                                      size_t(cnt / bpr) * 6 * e->esz, cudaMemcpyDefault, s));
     }
     for (int i = 0; i < HOST_PIPE_STREAMS; ++i) CUDA_TRY(cudaStreamSynchronize(e->hp_stream[i]));
-    if (e->n_waves) {  // every chunk has read the clock: one advance for the whole step
+    if (clock_runs(e)) {  // every chunk has read the clock: one advance for the whole step
         if (int rc = advance_clock(e, dt, 1, e->hp_stream[0])) return rc;
         CUDA_TRY(cudaStreamSynchronize(e->hp_stream[0]));
     }

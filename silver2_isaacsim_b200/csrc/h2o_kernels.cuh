@@ -111,6 +111,9 @@ struct EnvArgs {
     long long bodies_per_env;
 };
 
+// The optional current grid (h2o_set_current_grid) travels as GridArgs (csrc/h2o_waves.cuh), the third argument of
+// this kind, again of the per-body kernels only.
+
 // ---------------------------------------------------------------------------
 // PTX wrappers: mbarrier + bulk async copies (TMA engine, SASS UBLKCP)
 // ---------------------------------------------------------------------------
@@ -1000,7 +1003,8 @@ __device__ __forceinline__ void stage_waves(double* dst, const double* tab, cons
 template <typename S, int kLayout, int kParam, bool kStats>
 __global__ void __launch_bounds__(256) step_direct_kernel(const __grid_constant__ StepArgs a, long long body_begin,
                                                           const __grid_constant__ WaveArgs wv,
-                                                          const __grid_constant__ EnvArgs ev)
+                                                          const __grid_constant__ EnvArgs ev,
+                                                          const __grid_constant__ GridArgs gv)
 {
     __shared__ S table[(kParam == PARAM_TABLE) ? MAX_TABLE_TYPES * N_COEFF : 1];
     __shared__ unsigned char slot_map[(kParam == PARAM_TABLE) ? MAX_TABLE_SLOTS : 1];
@@ -1041,12 +1045,14 @@ __global__ void __launch_bounds__(256) step_direct_kernel(const __grid_constant_
         }
         BodyIn<double, S> bin;
         Env env{a.current[0], a.current[1], a.current[2], a.surface_z};
-        if (wv.n || ev.cond) {
+        if (wv.n || ev.cond || gv.vals) {
             EnvRow row{};
             if (ev.cond) row = env_row(ev.cond, (a.first_body + i) / ev.bodies_per_env);
+            // the clock: staged with the wave table, else read directly when only the grid needs it
+            const double t = wv.n ? wave_smem[wv.n * WAVE_STRIDE] : (gv.vals ? *wv.clock : 0.0);
             const Water w = water_at<sizeof(S) == 4>(a.current, a.surface_z, ev.cond != nullptr, row, wave_smem, wv.n,
-                                                     wv.depth, wv.n ? wave_smem[wv.n * WAVE_STRIDE] : 0.0, double(r.px),
-                                                     double(r.py), double(r.pz));
+                                                     wv.depth, t, double(r.px), double(r.py), double(r.pz),
+                                                     gv.vals ? &gv : nullptr);
             env = Env{w.cx, w.cy, w.cz, w.surface_z};
         }
         if (a.surface_eta) env.surface_z += double(reinterpret_cast<const S*>(a.surface_eta)[i]);
@@ -1358,11 +1364,13 @@ struct RolloutArgs {
     int no_fallback;
     WaveArgs waves;  // evaluated at each step's position and at t, t + dt, ... from the clock
     EnvArgs envs;    // each body's env row is read once, at kernel start
+    GridArgs grid;   // re-evaluated at each step's position and clock value
 };
 
 // Dynamic shared memory: wave_smem_bytes(a.waves.n).  kEnv: a.envs.cond is set (a separate instantiation, so that
-// the env row held in registers costs nothing without conditions).
-template <typename S, bool kStats, bool kEnv>
+// the env row held in registers costs nothing without conditions).  kGrid: a.grid.vals is set (likewise: rollouts
+// without a grid compile as they did before the grid existed).
+template <typename S, bool kStats, bool kEnv, bool kGrid>
 __global__ void rollout_persistent_kernel(const __grid_constant__ RolloutArgs a)
 {
     extern __shared__ double wave_smem[];
@@ -1394,12 +1402,13 @@ __global__ void rollout_persistent_kernel(const __grid_constant__ RolloutArgs a)
         if (kEnv) row = env_row(a.envs.cond, i / a.envs.bodies_per_env);
         const S inv_dt = S(1.0 / a.dt);
         S F[3] = {S(0), S(0), S(0)}, T[3] = {S(0), S(0), S(0)};
-        double t = wv.n ? wave_smem[wv.n * WAVE_STRIDE] : 0.0;
+        double t = wv.n ? wave_smem[wv.n * WAVE_STRIDE] : (kGrid ? *wv.clock : 0.0);
         for (int step = 0; step < a.n_steps; ++step) {
             Env env{a.current[0], a.current[1], a.current[2], a.surface_z};
-            if (wv.n || kEnv) {
+            if (wv.n || kEnv || kGrid) {
                 const Water w = water_at<sizeof(S) == 4>(a.current, a.surface_z, kEnv, row, wave_smem,
-                                                         wv.n, wv.depth, t, double(r.px), double(r.py), double(r.pz));
+                                                         wv.n, wv.depth, t, double(r.px), double(r.py), double(r.pz),
+                                                         kGrid ? &a.grid : nullptr);
                 env = Env{w.cx, w.cy, w.cz, w.surface_z};
                 t += a.dt;  // the same sequence of additions as advance_clock_kernel over single steps
             }
@@ -1526,6 +1535,41 @@ __global__ void __launch_bounds__(256) wave_sample_env_kernel(const __grid_const
     const Water w = water_at<sizeof(S) == 4>(zero, surface_z, true, env_row(ev.cond, e), wave_smem, wv.n, wv.depth,
                                              wave_smem[wv.n * WAVE_STRIDE], double(p[0]), double(p[1]), double(p[2]));
     o[0] = w.field.eta; o[1] = w.field.ux; o[2] = w.field.uy; o[3] = w.field.uz;
+}
+
+// Water sampling (h2o_water_sample): point k -> out row [waterline, flow x, y, z], the full water_at composition a
+// step forms at the clock's value (global environment, env row of env_index[k] when env_index is set, grid, waves),
+// before a caller height array and the fp32 rounding; an index outside [0, n_envs) gives a NaN row.  Dynamic shared
+// memory: (wv.n * WAVE_STRIDE + 1) doubles (the clock is staged even without waves).
+template <typename S>
+__global__ void __launch_bounds__(256) water_sample_kernel(const __grid_constant__ WaveArgs wv,
+                                                           const __grid_constant__ EnvArgs ev,
+                                                           const __grid_constant__ GridArgs gv, long long n_envs,
+                                                           double cx, double cy, double cz, double surface_z,
+                                                           const S* points, const int32_t* env_index, long long m,
+                                                           double* out)
+{
+    extern __shared__ double wave_smem[];
+    stage_waves(wave_smem, wv.tab, wv.clock, wv.n);
+    __syncthreads();
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    double* o = out + 4 * i;
+    EnvRow row{};
+    if (env_index) {
+        const long long e = env_index[i];
+        if (e < 0 || e >= n_envs) {
+            o[0] = o[1] = o[2] = o[3] = __longlong_as_double(0x7ff8000000000000ll);
+            return;
+        }
+        row = env_row(ev.cond, e);
+    }
+    const S* p = points + 3 * i;
+    const double current[3] = {cx, cy, cz};
+    const Water w = water_at<sizeof(S) == 4>(current, surface_z, env_index != nullptr, row, wave_smem, wv.n, wv.depth,
+                                             wave_smem[wv.n * WAVE_STRIDE], double(p[0]), double(p[1]), double(p[2]),
+                                             gv.vals ? &gv : nullptr);
+    o[0] = w.surface_z; o[1] = w.cx; o[2] = w.cy; o[3] = w.cz;
 }
 
 // Masked env reset (h2o_reset_envs), one thread per body: the carried [v, omega] of every body of a masked env

@@ -10,8 +10,8 @@
 // S_j = sinh(k_j (z + h)) / sinh(k_j h) (finite depth) or C_j = S_j = exp(k_j z) (deep water).
 // The hyperbolic ratios are evaluated as (e^{kz} +- e^{-k(z + 2h)}) / (1 - e^{-2kh}): no overflow at
 // any k h, and the denominator comes from the table (computed once on the host with expm1).
-// water_at composes the field with the global environment and a per-env conditions row
-// (h2o_set_env_conditions) into the waterline and flow a body sees.
+// water_at composes the field with the global environment, a per-env conditions row
+// (h2o_set_env_conditions) and a current grid (h2o_set_current_grid) into the waterline and flow a body sees.
 #pragma once
 
 #include "h2o_model.cuh"
@@ -51,6 +51,16 @@ H2O_HD double wave_add(double a, double b)
     return __dadd_rn(a, b);
 #else
     volatile double r = a + b;
+    return r;
+#endif
+}
+
+H2O_HD double wave_div(double a, double b)
+{
+#if defined(__CUDA_ARCH__)
+    return __ddiv_rn(a, b);
+#else
+    volatile double r = a / b;
     return r;
 #endif
 }
@@ -136,6 +146,98 @@ H2O_HD EnvRow env_row(const double* cond, long long e)
     return r;
 }
 
+// ---------------------------------------------------------------------------
+// Current grid (h2o_set_current_grid): a borrowed, C-contiguous float64 array (nt, nz, ny, nx, 3) of velocity
+// vectors; node (f, k, j, i) sits at (gx + i hx, gy + j hy, gz + k hz) and at time t0 + f ht.  The kernels read
+// it through the read-only path: it is not written during a launch (the caller edits it in stream order only).
+// ---------------------------------------------------------------------------
+struct GridArgs {
+    const double* vals;  // nullptr = no grid
+    long long nt, nz, ny, nx;
+    double gx, gy, gz, hx, hy, hz, t0, ht;
+};
+
+struct GridAxis {
+    long long i;  // lower node
+    double w;     // weight of the upper node
+};
+
+// Coordinate q on an axis of n nodes at o + k h: u = (q - o) / h clamped to [0, n - 1], i = min(floor(u), n - 2),
+// w = u - i; a single node gives index 0 and weight 0 (its neighbour is never read).  q must not be NaN.
+H2O_HD GridAxis grid_axis(double q, long long n, double o, double h)
+{
+    if (n == 1) return GridAxis{0, 0.0};
+    const double top = double(n - 1);
+    double u = wave_div(wave_add(q, -o), h);
+    u = u > 0.0 ? (u < top ? u : top) : 0.0;
+    long long i = (long long)floor(u);
+    if (i > n - 2) i = n - 2;
+    return GridAxis{i, wave_add(u, -double(i))};
+}
+
+H2O_HD double grid_ld(const double* p)
+{
+#if defined(__CUDA_ARCH__)
+    return __ldg(p);
+#else
+    return *p;
+#endif
+}
+
+// a <- a + w (b - a), component by component, three separately rounded operations
+H2O_HD void grid_lerp(double a[3], const double b[3], double w)
+{
+    for (int c = 0; c < 3; ++c) a[c] = wave_add(a[c], wave_mul(w, wave_add(b[c], -a[c])));
+}
+
+// The node at p, interpolated along x (the x-neighbour pair is 6 contiguous doubles), then y, then z.
+H2O_HD void grid_x(const double* p, long long nx, double wx, double v[3])
+{
+    v[0] = grid_ld(p); v[1] = grid_ld(p + 1); v[2] = grid_ld(p + 2);
+    if (nx > 1) {
+        const double b[3] = {grid_ld(p + 3), grid_ld(p + 4), grid_ld(p + 5)};
+        grid_lerp(v, b, wx);
+    }
+}
+H2O_HD void grid_xy(const GridArgs& g, const double* p, double wx, double wy, double v[3])
+{
+    grid_x(p, g.nx, wx, v);
+    if (g.ny > 1) {
+        double b[3];
+        grid_x(p + 3 * g.nx, g.nx, wx, b);
+        grid_lerp(v, b, wy);
+    }
+}
+H2O_HD void grid_xyz(const GridArgs& g, const double* p, double wx, double wy, double wz, double v[3])
+{
+    grid_xy(g, p, wx, wy, v);
+    if (g.nz > 1) {
+        double b[3];
+        grid_xy(g, p + 3 * g.nx * g.ny, wx, wy, b);
+        grid_lerp(v, b, wz);
+    }
+}
+
+// The grid's velocity at grid-frame coordinates (X, Y, Z) and time T: multilinear, along x, then y, then z, then t,
+// held at the boundary outside the lattice and before the first / after the last frame.  Any NaN coordinate gives
+// NaN, with no read.
+H2O_HD void grid_eval(const GridArgs& g, double X, double Y, double Z, double T, double v[3])
+{
+    if (X != X || Y != Y || Z != Z || T != T) {  // NaN
+        v[0] = v[1] = v[2] = nan("");
+        return;
+    }
+    const GridAxis ax = grid_axis(X, g.nx, g.gx, g.hx), ay = grid_axis(Y, g.ny, g.gy, g.hy);
+    const GridAxis az = grid_axis(Z, g.nz, g.gz, g.hz), at = grid_axis(T, g.nt, g.t0, g.ht);
+    const double* p = g.vals + 3 * (((at.i * g.nz + az.i) * g.ny + ay.i) * g.nx + ax.i);
+    grid_xyz(g, p, ax.w, ay.w, az.w, v);
+    if (g.nt > 1) {
+        double b[3];
+        grid_xyz(g, p + 3 * g.nx * g.ny * g.nz, ax.w, ay.w, az.w, b);
+        grid_lerp(v, b, at.w);
+    }
+}
+
 // What a body sees: the waterline (before a caller height array is added), the flow, and the env's field alone
 // (s * eta, s * u; zeros without a wave field).
 struct Water {
@@ -143,15 +245,19 @@ struct Water {
     WaveSample field;
 };
 
-// The one composition of the global environment (current, surface_z), the env row (has_row), the wave table and
-// the clock value t for a body at p, used by every step kernel, the sampler and the host emulator.  With a row,
-// every operation is a separately rounded float64 operation in the order include/h2o.h gives:
-//   L = surface_z + dz,  field = s * wave_eval(p_x - x0, p_y - y0, p_z - L, t + tau),
-//   waterline = L + s eta,  flow = (current + c) + s u.
-// The identity row [0,0,0,0,1,0,0,0] makes each of them exact, so it reproduces the row-less result bit for bit.
+// The one composition of the global environment (current, surface_z), the env row (has_row), the current grid
+// (grid, or nullptr), the wave table and the clock value t for a body at p, used by every step kernel, the samplers
+// and the host emulators.  Every operation with the row or the grid is a separately rounded float64 operation in
+// the order include/h2o.h gives:
+//   L = surface_z + dz,  X = p_x - x0,  Y = p_y - y0,  Z = p_z - L,  T = t + tau,
+//   g = grid_eval(X, Y, Z, T),  field = s * wave_eval(X, Y, Z, T),
+//   waterline = L + s eta,  flow = ((current + c) + g) + s u.
+// The identity row [0,0,0,0,1,0,0,0] makes each row operation exact, so it reproduces the row-less result bit for
+// bit; a grid of zeros does the same for the grid.
 template <bool kF32>
 H2O_HD Water water_at(const double current[3], double surface_z, bool has_row, const EnvRow& row, const double* tab,
-                      int n_waves, double depth, double t, double px, double py, double pz)
+                      int n_waves, double depth, double t, double px, double py, double pz,
+                      const GridArgs* grid = nullptr)
 {
     Water w{surface_z, current[0], current[1], current[2], {0.0, 0.0, 0.0, 0.0}};
     const double* c = row.c;
@@ -164,8 +270,16 @@ H2O_HD Water water_at(const double current[3], double surface_z, bool has_row, c
         py = wave_add(py, -c[ENV_Y0]);
         t = wave_add(t, c[ENV_TAU]);
     }
+    const double z_rel = pz - w.surface_z;
+    if (grid) {
+        double g[3];
+        grid_eval(*grid, px, py, z_rel, t, g);
+        w.cx = wave_add(w.cx, g[0]);
+        w.cy = wave_add(w.cy, g[1]);
+        w.cz = wave_add(w.cz, g[2]);
+    }
     if (n_waves) {
-        w.field = wave_eval<kF32>(tab, n_waves, depth, px, py, pz - w.surface_z, t);  // the one call site
+        w.field = wave_eval<kF32>(tab, n_waves, depth, px, py, z_rel, t);  // the one call site
         if (has_row) {
             const double s = c[ENV_SCALE];
             w.field = WaveSample{wave_mul(s, w.field.eta), wave_mul(s, w.field.ux), wave_mul(s, w.field.uy),

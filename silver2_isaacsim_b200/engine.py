@@ -160,27 +160,80 @@ class HydroEngine:
         precision: a (m,4) float64 CUDA tensor of rows ``eta, ux, uy, uz`` (zeros without a field).  With ``env``
         (one env index per point, or one for all), each point is seen from that env: rows ``s eta, s u`` at
         ``p - origin`` and ``clock + tau`` (``waves.evaluate_env``); an index outside ``[0, E)`` gives a NaN row."""
-        pts = self._as_dev(points)
-        if pts.ndim != 2 or pts.shape[1] != 3:
-            raise ValueError(f"points must be (m,3), got {tuple(pts.shape)}")
-        out = torch.empty(pts.shape[0], 4, dtype=torch.float64, device=self.device)
+        pts, out = self._sample_buffers(points)
         if env is None:
             L.check(self._lib.h2o_wave_sample(self._h, ctypes.c_void_p(pts.data_ptr()), int(pts.shape[0]),
                                               ctypes.c_void_p(out.data_ptr()), _stream_ptr(self.device)))
             return out
+        idx = self._env_index(env, pts.shape[0])
+        L.check(self._lib.h2o_wave_sample_env(self._h, ctypes.c_void_p(pts.data_ptr()), ctypes.c_void_p(idx.data_ptr()),
+                                              int(pts.shape[0]), ctypes.c_void_p(out.data_ptr()),
+                                              _stream_ptr(self.device)))
+        return out
+
+    def sample_water(self, points, env=None) -> torch.Tensor:
+        """What a step sees at ``points`` (m,3) world positions and the current clock: a (m,4) float64 CUDA tensor
+        of rows ``waterline, flow_x, flow_y, flow_z``, the full composition of global environment, env row, current
+        grid and wave field (include/h2o.h, h2o_water_sample), before a caller height array and before the fp32
+        rounding.  ``env`` (one env index per point, or one for all) applies that env's conditions; ``None`` applies
+        none; an index outside ``[0, E)`` gives a NaN row."""
+        pts, out = self._sample_buffers(points)
+        idx = None if env is None else self._env_index(env, pts.shape[0])
+        L.check(self._lib.h2o_water_sample(self._h, ctypes.c_void_p(pts.data_ptr()),
+                                           None if idx is None else ctypes.c_void_p(idx.data_ptr()), int(pts.shape[0]),
+                                           ctypes.c_void_p(out.data_ptr()), _stream_ptr(self.device)))
+        return out
+
+    def _sample_buffers(self, points):
+        pts = self._as_dev(points)
+        if pts.ndim != 2 or pts.shape[1] != 3:
+            raise ValueError(f"points must be (m,3), got {tuple(pts.shape)}")
+        return pts, torch.empty(pts.shape[0], 4, dtype=torch.float64, device=self.device)
+
+    def _env_index(self, env, m: int) -> torch.Tensor:
         idx = torch.as_tensor(env, device=self.device)
         if idx.dtype.is_floating_point or idx.dtype == torch.bool:
             raise ValueError("env must hold integer env indices")
         idx = idx.reshape(-1).long().clamp(-1, 2 ** 31 - 1).to(torch.int32)  # no wrap-around into [0, E)
         if idx.numel() == 1:
-            idx = idx.expand(pts.shape[0])
+            idx = idx.expand(m)
         idx = idx.contiguous()
-        if tuple(idx.shape) != (pts.shape[0],):
-            raise ValueError(f"env must be one index or one per point ({pts.shape[0]}), got {tuple(idx.shape)}")
-        L.check(self._lib.h2o_wave_sample_env(self._h, ctypes.c_void_p(pts.data_ptr()), ctypes.c_void_p(idx.data_ptr()),
-                                              int(pts.shape[0]), ctypes.c_void_p(out.data_ptr()),
-                                              _stream_ptr(self.device)))
-        return out
+        if tuple(idx.shape) != (m,):
+            raise ValueError(f"env must be one index or one per point ({m}), got {tuple(idx.shape)}")
+        return idx
+
+    def set_current_grid(self, values: Optional[torch.Tensor], origin=(0.0, 0.0, 0.0), spacing=(1.0, 1.0, 1.0),
+                         t0: float = 0.0, frame_dt: float = 0.0):
+        """Gridded water current: ``values`` is a contiguous float64 tensor on the engine's device, (nt,nz,ny,nx,3)
+        or (nz,ny,nx,3) (one frame), of velocities at the nodes ``origin + (i, j, k) * spacing`` and times
+        ``t0 + f * frame_dt`` (``currents.CurrentGrid`` builds them).  Every step interpolates it at each body's
+        env-local position, depth below the env's mean level and env time, and adds it to the current
+        (include/h2o.h).  The tensor is borrowed, not copied: in-place edits reach the next step and the next replay
+        of a captured rollout.  ``None`` removes the grid.  Steps then run on the per-body kernel;
+        ``rollout_persistent`` follows it; ``components`` ignores it."""
+        if values is None:
+            L.check(self._lib.h2o_set_current_grid(self._h, None, None, None))
+            self._grid = None
+            return
+        if not isinstance(values, torch.Tensor):
+            raise ValueError("values must be a torch tensor (currents.CurrentGrid gives the NumPy values)")
+        if (values.dtype != torch.float64 or values.device != self.device or values.ndim not in (4, 5)
+                or values.shape[-1] != 3 or not values.is_contiguous()):
+            raise ValueError(f"values must be a contiguous (nt,nz,ny,nx,3) or (nz,ny,nx,3) torch.float64 tensor on "
+                             f"{self.device}, got {tuple(values.shape)} {values.dtype} on {values.device}")
+        if values.numel() == 0:
+            raise ValueError("values must not be empty")
+        if len(origin) != 3 or len(spacing) != 3:
+            raise ValueError("origin and spacing must have 3 values")
+        dims = (ctypes.c_int64 * 4)(*([1] * (5 - values.ndim) + list(values.shape[:-1])))
+        geom = (ctypes.c_double * 8)(*[float(x) for x in (*origin, *spacing)], float(t0), float(frame_dt))
+        L.check(self._lib.h2o_set_current_grid(self._h, ctypes.c_void_p(values.data_ptr()), dims, geom))
+        self._grid = values  # keep the borrowed memory alive
+
+    @property
+    def current_grid(self) -> Optional[torch.Tensor]:
+        """The borrowed current-grid tensor, or ``None``."""
+        return getattr(self, "_grid", None)
 
     def set_env_conditions(self, cond: Optional[torch.Tensor], bodies_per_env: int = 0):
         """Per-env water conditions: ``cond`` is a contiguous (E,8) float64 tensor on the engine's device
