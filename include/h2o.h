@@ -341,7 +341,10 @@ H2O_API int h2o_launch_rollout(h2o_handle h, h2o_stream stream);
  * velocity tensors and the carried velocities hold the final state, out_force / out_torque the last step's
  * wrench.  trace_every > 0: every trace_every-th step a row [p, v, w] (9 scalars, handle dtype) per body
  * goes to trace_out, a device array (n_steps / trace_every, n_bodies, 9) -- the columns of the
- * reference's velocity logger (log_velocity.py:17-20).  dt <= 1e-6 is a successful no-op. */
+ * reference's velocity logger (log_velocity.py:17-20); trace_every > n_steps (no row) is H2O_ERR_BAD_ARGUMENT.
+ * The kernel follows the Numba semantics and has no robot-wrench output, so a handle with h2o_set_warp_compat
+ * on, or bound with an out_robot_wrench, gets H2O_ERR_NOT_CONFIGURED (h2o_capture_rollout honours both), as
+ * does one with dense added mass or a caller height field.  dt <= 1e-6 is a successful no-op. */
 H2O_API int h2o_rollout_persistent(h2o_handle h, int n_steps, double dt, double gravity, int trace_every,
                                    void* trace_out, h2o_stream stream);
 

@@ -13,31 +13,38 @@ from . import hydro_oracle as O
 
 
 def _rot(q):
-    x, y, z, w = q
+    """Rotation matrix (..., 3, 3) of xyzw quaternions (..., 4), not normalised."""
+    x, y, z, w = np.moveaxis(np.asarray(q, dtype=np.float64), -1, 0)
     x2, y2, z2 = x + x, y + y, z + z
-    return np.array([[1 - (y * y2 + z * z2), x * y2 - w * z2, x * z2 + w * y2],
-                     [x * y2 + w * z2, 1 - (x * x2 + z * z2), y * z2 - w * x2],
-                     [x * z2 - w * y2, y * z2 + w * x2, 1 - (x * x2 + y * y2)]])
+    rows = [[1 - (y * y2 + z * z2), x * y2 - w * z2, x * z2 + w * y2],
+            [x * y2 + w * z2, 1 - (x * x2 + z * z2), y * z2 - w * x2],
+            [x * z2 - w * y2, y * z2 + w * x2, 1 - (x * x2 + y * y2)]]
+    return np.stack([np.stack(r, axis=-1) for r in rows], axis=-2)
 
 
 def integrate(p, q, v, w, F, T, mass, dims, dt, gravity):
-    """One semi-implicit Euler step of a free box (xyzw quaternion); returns new (p,q,v,w)."""
+    """One semi-implicit Euler step of a free box (xyzw quaternion); returns new (p,q,v,w).
+
+    One body, or a batch: vectors (..., 3), quaternions (..., 4), mass (...) and dims (..., 3)."""
+    p, q, v, w, F, T, dims = (np.asarray(a, dtype=np.float64) for a in (p, q, v, w, F, T, dims))
+    mass = np.asarray(mass, dtype=np.float64)[..., None]
     v = v + dt * (F / mass + np.array([0.0, 0.0, -gravity]))
     R = _rot(q)
-    dx, dy, dz = dims
-    I = mass * np.array([dy * dy + dz * dz, dx * dx + dz * dz, dx * dx + dy * dy]) / 12.0
-    tb, wb = R.T @ T, R.T @ w
+    dx, dy, dz = np.moveaxis(dims, -1, 0)
+    I = mass * np.stack([dy * dy + dz * dz, dx * dx + dz * dz, dx * dx + dy * dy], axis=-1) / 12.0
+    tb, wb = np.einsum("...ji,...j->...i", R, T), np.einsum("...ji,...j->...i", R, w)
     gyro = np.cross(wb, I * wb)
     wb = wb + dt * (tb - gyro) / I
-    w = R @ wb
+    w = np.einsum("...ij,...j->...i", R, wb)
     p = p + dt * v
-    x, y, z, s = q
+    x, y, z, s = np.moveaxis(q, -1, 0)
+    wx, wy, wz = np.moveaxis(w, -1, 0)
     h = 0.5 * dt
-    nq = np.array([x + h * (w[0] * s + w[1] * z - w[2] * y),
-                   y + h * (w[1] * s + w[2] * x - w[0] * z),
-                   z + h * (w[2] * s + w[0] * y - w[1] * x),
-                   s - h * (w[0] * x + w[1] * y + w[2] * z)])
-    return p, nq / np.linalg.norm(nq), v, w
+    nq = np.stack([x + h * (wx * s + wy * z - wz * y),
+                   y + h * (wy * s + wz * x - wx * z),
+                   z + h * (wz * s + wx * y - wy * x),
+                   s - h * (wx * x + wy * y + wz * z)], axis=-1)
+    return p, nq / np.linalg.norm(nq, axis=-1, keepdims=True), v, w
 
 
 def rollout(ctor, mass, p, q, v, w, dt, steps, gravity=9.81):

@@ -1413,10 +1413,17 @@ int h2o_rollout_persistent(h2o_handle h, int n_steps, double dt, double gravity,
     if (n_steps < 1) return fail(H2O_ERR_BAD_ARGUMENT, "n_steps must be >= 1");
     if (trace_every < 0 || (trace_every > 0 && !trace_out))
         return fail(H2O_ERR_BAD_ARGUMENT, "trace_every > 0 needs a trace buffer of (n_steps / trace_every, n_bodies, 9)");
+    if (trace_every > n_steps)
+        return fail(H2O_ERR_BAD_ARGUMENT, "trace_every (%d) > n_steps (%d): the rollout would write no trace row",
+                    trace_every, n_steps);
     if (e->am_dense || e->surface_eta)
         return fail(H2O_ERR_NOT_CONFIGURED,
                     "persistent rollouts keep the wrapper's added-mass diagonal and take no caller height field "
                     "(the built-in wave field works)");
+    if (e->warp_compat || e->b_w)
+        return fail(H2O_ERR_NOT_CONFIGURED,
+                    "persistent rollouts follow the Numba semantics and write no robot wrench: turn Warp "
+                    "compatibility off and bind without a robot-wrench output, or use h2o_capture_rollout");
     if (!(dt > 1e-6)) return H2O_OK;  // hydrodynamics_behavior.py:139
     DeviceGuard g(e->device);
     RolloutArgs a;

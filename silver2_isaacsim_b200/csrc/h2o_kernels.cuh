@@ -1264,53 +1264,7 @@ struct FreeBodyArgs {
     double dt, gravity;            // gravity acts along -z
 };
 
-// One semi-implicit Euler step of a free box (shared by free_body_kernel and the persistent rollout kernel).
-// State in double, quaternion xyzw; m, dx, dy, dz from the coefficient record.
-struct FreeBodyState {
-    double px, py, pz, qx, qy, qz, qw, vx, vy, vz, wx, wy, wz;
-};
-__device__ __forceinline__ void free_body_update(FreeBodyState& s, double fx, double fy, double fz, double tx, double ty,
-                                                 double tz, double m, double dx, double dy, double dz, double dt,
-                                                 double gravity)
-{
-    const double qx = s.qx, qy = s.qy, qz = s.qz, qw = s.qw;
-    const double im = 1.0 / m;
-    // linear: v += dt (F/m + g)
-    const double vx = s.vx + dt * fx * im;
-    const double vy = s.vy + dt * fy * im;
-    const double vz = s.vz + dt * (fz * im - gravity);
-    // angular, body frame: I w' = tau_b - w_b x (I w_b)
-    const double x2 = qx + qx, y2 = qy + qy, z2 = qz + qz;
-    const double r00 = 1 - (qy * y2 + qz * z2), r01 = qx * y2 - qw * z2, r02 = qx * z2 + qw * y2;
-    const double r10 = qx * y2 + qw * z2, r11 = 1 - (qx * x2 + qz * z2), r12 = qy * z2 - qw * x2;
-    const double r20 = qx * z2 - qw * y2, r21 = qy * z2 + qw * x2, r22 = 1 - (qx * x2 + qy * y2);
-    const double Ix = m * (dy * dy + dz * dz) / 12.0, Iy = m * (dx * dx + dz * dz) / 12.0,
-                 Iz = m * (dx * dx + dy * dy) / 12.0;
-    const double wx = s.wx, wy = s.wy, wz = s.wz;
-    const double tbx = r00 * tx + r10 * ty + r20 * tz, tby = r01 * tx + r11 * ty + r21 * tz,
-                 tbz = r02 * tx + r12 * ty + r22 * tz;
-    double wbx = r00 * wx + r10 * wy + r20 * wz, wby = r01 * wx + r11 * wy + r21 * wz,
-           wbz = r02 * wx + r12 * wy + r22 * wz;
-    const double gx = wby * (Iz * wbz) - wbz * (Iy * wby), gy = wbz * (Ix * wbx) - wbx * (Iz * wbz),
-                 gz = wbx * (Iy * wby) - wby * (Ix * wbx);
-    wbx += dt * (tbx - gx) / Ix;
-    wby += dt * (tby - gy) / Iy;
-    wbz += dt * (tbz - gz) / Iz;
-    const double nwx = r00 * wbx + r01 * wby + r02 * wbz, nwy = r10 * wbx + r11 * wby + r12 * wbz,
-                 nwz = r20 * wbx + r21 * wby + r22 * wbz;
-    // pose with the NEW velocities; q' = q + dt/2 (0,w) * q
-    s.px += dt * vx; s.py += dt * vy; s.pz += dt * vz;
-    const double h = 0.5 * dt;
-    double nqw = qw - h * (nwx * qx + nwy * qy + nwz * qz);
-    double nqx = qx + h * (nwx * qw + nwy * qz - nwz * qy);
-    double nqy = qy + h * (nwy * qw + nwz * qx - nwx * qz);
-    double nqz = qz + h * (nwz * qw + nwx * qy - nwy * qx);
-    const double inv = 1.0 / sqrt(nqx * nqx + nqy * nqy + nqz * nqz + nqw * nqw);
-    s.qx = nqx * inv; s.qy = nqy * inv; s.qz = nqz * inv; s.qw = nqw * inv;
-    s.vx = vx; s.vy = vy; s.vz = vz;
-    s.wx = nwx; s.wy = nwy; s.wz = nwz;
-}
-
+// The step itself is free_body_update (h2o_model.cuh), shared with the persistent rollout kernel.
 template <typename S> __global__ void __launch_bounds__(256) free_body_kernel(const __grid_constant__ FreeBodyArgs a)
 {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;

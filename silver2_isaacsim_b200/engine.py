@@ -551,10 +551,15 @@ class HydroEngine:
     def rollout_persistent(self, n_steps: int, dt: float, gravity: float = 9.81, trace_every: int = 0):
         """``n_steps`` x (fused force step -> free-body stepper) over the bound split-layout tensors in ONE
         kernel launch (state in registers across the steps).  Returns the trace tensor
-        ``(n_steps // trace_every, n_bodies, 9)`` = [p, v, w] rows when ``trace_every > 0``, else ``None``."""
+        ``(n_steps // trace_every, n_bodies, 9)`` = [p, v, w] rows when ``trace_every > 0``, else ``None``; a
+        ``trace_every`` above ``n_steps`` would write no row and raises ``ValueError``.  The rollout follows the
+        Numba semantics and writes no robot wrench: with ``set_warp_compat(True)`` or a bound robot-wrench output
+        it raises (use ``capture_rollout`` in free-body mode there)."""
         trace = None
+        if trace_every > n_steps:
+            raise ValueError(f"trace_every ({trace_every}) > n_steps ({n_steps}) would write no trace row")
         if trace_every > 0:
-            trace = self._empty(max(1, n_steps // trace_every), self.n_bodies, 9)
+            trace = self._empty(n_steps // trace_every, self.n_bodies, 9)
         L.check(self._lib.h2o_rollout_persistent(self._h, int(n_steps), float(dt), float(gravity), int(trace_every),
                                                  ctypes.c_void_p(trace.data_ptr()) if trace is not None else None,
                                                  _stream_ptr(self.device)))
