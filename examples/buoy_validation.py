@@ -9,9 +9,12 @@ factor is reported like its BenchmarkRtf (benchmark_rtf.py:37-71).
 
 With --wave-amplitude > 0 the buoy floats in a regular deep-water wave of that amplitude and --wave-period,
 evaluated by the engine at the buoy on every step; the CSV then has one more column, the surface
-elevation at the buoy.
+elevation at the buoy.  --wave-slope also tests the buoy against the wave surface's local tangent plane
+(h2o_set_wave_slope), so that the waves roll and pitch it; the CSV then also logs the buoy's roll and pitch angles
+(degrees, xyz Euler angles of its orientation).
 
     python examples/buoy_validation.py [--steps 6000] [--n 1] [--csv /tmp/buoy.csv] [--wave-amplitude 0.2 --wave-period 8]
+                                       [--wave-slope]
 """
 import argparse
 import os
@@ -30,7 +33,19 @@ ap.add_argument("--n", type=int, default=1, help="identical buoys stepped side b
 ap.add_argument("--csv", default="/tmp/buoy_velocity_log.csv")
 ap.add_argument("--wave-amplitude", type=float, default=0.0, help="regular deep-water wave amplitude (m); 0 = still water")
 ap.add_argument("--wave-period", type=float, default=8.0, help="wave period (s)")
+ap.add_argument("--wave-slope", action="store_true", help="test the buoy against the waves' local tangent plane")
 args = ap.parse_args()
+if args.wave_slope and not args.wave_amplitude > 0:
+    ap.error("--wave-slope needs --wave-amplitude > 0")
+
+
+def roll_pitch(q):
+    """Roll and pitch (degrees) of an xyzw quaternion: the x and y angles of its xyz Euler decomposition."""
+    x, y, z, s = (float(c) for c in q)
+    roll = np.degrees(np.arctan2(2 * (s * x + y * z), 1 - 2 * (x * x + y * y)))
+    pitch = np.degrees(np.arcsin(np.clip(2 * (s * y - z * x), -1.0, 1.0)))
+    return roll, pitch
+
 
 dev = torch.device("cuda:0")
 wl = W.readme_buoy()
@@ -44,18 +59,26 @@ eng.set_rollout_mode(free_bodies=True, gravity=wl.g)   # every captured step: fo
 in_waves = args.wave_amplitude > 0
 if in_waves:
     eng.set_wave_field(waves.regular(args.wave_amplitude, args.wave_period))
+    eng.set_wave_slope(args.wave_slope)
 
 GRAPH = 100
 eng.capture_rollout(GRAPH, wl.dt)
-trace = VelocityTrace(args.csv, extra_columns=("surface_elevation",) if in_waves else ())
+columns = (("surface_elevation",) if in_waves else ()) + (("roll_deg", "pitch_deg") if args.wave_slope else ())
+trace = VelocityTrace(args.csv, extra_columns=columns)
+max_tilt = 0.0
 rtf = RtfMeter(report_every=1000)
 for k in range(args.steps // GRAPH):
     eng.launch_rollout()
     torch.cuda.synchronize()
     rtf.on_physics_step(wl.dt, GRAPH)
     extra = (float(eng.sample_waves(pos[:1])[0, 0]),) if in_waves else ()   # elevation at the buoy, current clock
+    if args.wave_slope:
+        extra += roll_pitch(quat[0].cpu())
+        max_tilt = max(max_tilt, abs(extra[1]), abs(extra[2]))
     trace.sample(pos.cpu(), v.cpu(), w.cpu(), extra=extra)  # one row per replayed graph
 r = rtf.report()
 z = float(pos[0, 2])
 print(f"{args.n} buoy(s), {r['steps']} steps of {wl.dt * 1e3:.2f} ms: RTF {r['rtf']:.1f}x, {r['steps_per_s']:.0f} steps/s; "
       f"final height of the centre {z:+.4f} m (half submerged = 0), |v| {float(v[0].norm()):.2e} m/s; trace: {args.csv}")
+if args.wave_slope:
+    print(f"largest logged roll / pitch angle: {max_tilt:.2f} deg")

@@ -143,6 +143,27 @@ H2O_API int h2o_wave_time_read(h2o_handle h, double* t, h2o_stream stream);
  * points is a DEVICE array (m,3) in the handle dtype (world positions; the velocity depth is measured from
  * surface_z), out a DEVICE array (m,4) float64 of rows [eta, ux, uy, uz] (zeros without a field). */
 H2O_API int h2o_wave_sample(h2o_handle h, const void* points, int64_t m, double* out, h2o_stream stream);
+/* Wave-slope submersion: enable != 0 tests each body against the wave surface's local tangent plane instead of the
+ * horizontal plane through its waterline W (the reference's model at the same level of approximation: its surface is
+ * a plane, numba_hydrodynamics.py:59-105).  For a body at env-local (X, Y) and env time T (the theta_j of eta):
+ *   sx = s sum_j (-a_j kx_j sin theta_j),   sy = s sum_j (-a_j ky_j sin theta_j)
+ * with s the env's wave scale (1 without env conditions).  fp64 mode evaluates it in double; fp32 mode takes the
+ * sine in float, as for u_z, and keeps the sums in double.  The slope is (0, 0) with the mode off, without a wave
+ * field; the current grid, dz and a caller height array (h2o_set_surface_heights) contribute none.
+ * A keypoint's height above the waterline becomes (p_z - W) + e . k, k its body-frame offset and
+ *   e_c = (R_2c - sx R_0c) - sy R_1c          (double in both modes, c = x, y, z)
+ * with R the rotation the mode uses (R(q), or R(q) + 2 dq I under Warp compatibility).  In the world frame: keypoint w
+ * is wet iff w_z - W - sx (w_x - p_x) - sy (w_y - p_y) < 0.  z_min, z_max, the strict wet mask, the submersion ratio
+ * and its cuts, the wetted faces (face-centre keypoints) and the centre of buoyancy (the mean of the wet keypoints)
+ * are formed from these heights exactly as without slope.  The normal (-sx, -sy, 1) is deliberately not normalised:
+ * every sign test and the ratio -z_min / (z_max - z_min) are invariant to its length.  The forces keep the
+ * reference's formulas (buoyancy along +z, drag, lift, added mass); no fluid-acceleration term is added.
+ * Default 0.  With no wave field the call changes nothing: steps and rollouts are bit-identical to a handle without
+ * it.  With a field whose amplitudes are all zero, steps are bit-identical to the mode off; h2o_rollout_persistent
+ * runs its own slope instantiation there, whose multiply-add contraction may differ: to rounding.  Every step path
+ * that takes a wave field honours the mode (eager, bound, captured, host-buffer, h2o_rollout_persistent);
+ * h2o_components ignores it, as it ignores the field.  Like every h2o_set_* call this drops a captured rollout. */
+H2O_API int h2o_set_wave_slope(h2o_handle h, int enable);
 
 /* Per-env water conditions for vectorised scenes (SURVEY.md 8(f4)).  Envs are contiguous, equal runs of bodies:
  * body i (global index) belongs to env e = i / bodies_per_env, and E = n_bodies / bodies_per_env.  cond_dev is a
@@ -221,6 +242,12 @@ H2O_API int h2o_set_current_grid(h2o_handle h, const double* grid_dev, const int
  * none; an index outside [0, E) gives a NaN row.  H2O_ERR_NOT_CONFIGURED for env_index without env conditions. */
 H2O_API int h2o_water_sample(h2o_handle h, const void* points, const int32_t* env_index, int64_t m, double* out,
                              h2o_stream stream);
+/* The surface slope a step uses at given points and the clock's current value (h2o_set_wave_slope): points as for
+ * h2o_water_sample, out a DEVICE array (m,2) float64 of rows [sx, sy]; zero rows with the mode off or without a wave
+ * field.  env_index as for h2o_water_sample: a NaN row for an index outside [0, E), H2O_ERR_NOT_CONFIGURED for
+ * env_index without env conditions. */
+H2O_API int h2o_water_slope_sample(h2o_handle h, const void* points, const int32_t* env_index, int64_t m, double* out,
+                                   h2o_stream stream);
 
 /* Same twelve scalars, same order as the reference wrapper ctor
  * (numba_hydrodynamics_wrapper.py:9-10): width, depth, height, linear_drag_coefficient,

@@ -80,6 +80,7 @@ struct h2o_engine {
     double* wave_clock = nullptr;  // the wave field's clock (one double, device)
     int n_waves = 0;               // 0 = no wave field
     double wave_depth = INFINITY;
+    int wave_slope = 0;            // 1: with a wave field, bodies are tested against the surface's tangent plane
     const double* env_cond = nullptr;  // (n / bodies_per_env, ENV_STRIDE) per-env conditions, borrowed, or nullptr
     long long bodies_per_env = 0;
     GridArgs grid{};  // current grid (borrowed values, dims and geometry); grid.vals == nullptr = none
@@ -295,6 +296,9 @@ static int launch_tile(h2o_engine* e, StepArgs& a, cudaStream_t stream)
     return H2O_OK;
 }
 
+// Wave-slope submersion is in effect: the mode is on and there is a wave field to take the slope of.
+static bool slope_on(const h2o_engine* e) { return e->wave_slope && e->n_waves; }
+
 template <typename S, int kLayout, int kParam, bool kStats>
 static int launch_direct(h2o_engine* e, const StepArgs& a, long long body_begin, cudaStream_t stream)
 {
@@ -321,7 +325,13 @@ static int launch_direct(h2o_engine* e, const StepArgs& a, long long body_begin,
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, step_direct_kernel<S, kLayout, kParam, kStats>, a, body_begin, wv, ev, gv));
+        if (slope_on(e))
+            CUDA_TRY(cudaLaunchKernelEx(&cfg, step_direct_kernel<S, kLayout, kParam, kStats, true>, a, body_begin, wv, ev,
+                                        gv));
+        else
+            CUDA_TRY(cudaLaunchKernelEx(&cfg, step_direct_kernel<S, kLayout, kParam, kStats>, a, body_begin, wv, ev, gv));
+    } else if (slope_on(e)) {
+        step_direct_kernel<S, kLayout, kParam, kStats, true><<<grid, 256, smem, stream>>>(a, body_begin, wv, ev, gv);
     } else {
         step_direct_kernel<S, kLayout, kParam, kStats><<<grid, 256, smem, stream>>>(a, body_begin, wv, ev, gv);
     }
@@ -680,6 +690,15 @@ int h2o_set_wave_field(h2o_handle h, int n_components, const double* comps, doub
     return H2O_OK;
 }
 
+int h2o_set_wave_slope(h2o_handle h, int enable)
+{
+    h2o_engine* e = check(h);
+    if (!e) return H2O_ERR_BAD_HANDLE;
+    { DeviceGuard gi(e->device); invalidate_graph(e); }
+    e->wave_slope = enable != 0;
+    return H2O_OK;
+}
+
 int h2o_wave_time_write(h2o_handle h, double t, h2o_stream stream)
 {
     h2o_engine* e = check(h);
@@ -854,6 +873,33 @@ int h2o_water_sample(h2o_handle h, const void* points, const int32_t* env_index,
         water_sample_kernel<double><<<grid, 256, smem, s>>>(wave_args(e), env_args(e), e->grid, n_envs, c[0], c[1],
                                                             c[2], e->surface_z, static_cast<const double*>(points),
                                                             env_index, m, out);
+    CUDA_TRY(cudaGetLastError());
+    return H2O_OK;
+}
+
+int h2o_water_slope_sample(h2o_handle h, const void* points, const int32_t* env_index, int64_t m, double* out,
+                           h2o_stream stream)
+{
+    h2o_engine* e = check(h);
+    if (!e) return H2O_ERR_BAD_HANDLE;
+    if (env_index && !e->env_cond) return fail(H2O_ERR_NOT_CONFIGURED, "no env conditions set (h2o_set_env_conditions)");
+    if (m < 0) return fail(H2O_ERR_BAD_ARGUMENT, "m must be >= 0");
+    if (m == 0) return H2O_OK;
+    if (!points || !out) return fail(H2O_ERR_BAD_ARGUMENT, "NULL points / out");
+    DeviceGuard g(e->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int grid = int((m + 255) / 256);
+    // the slope a step uses: none unless the mode is on and there is a wave field
+    WaveArgs wv = wave_args(e);
+    if (!slope_on(e)) wv.n = 0;
+    const size_t smem = (size_t(wv.n) * WAVE_STRIDE + 1) * sizeof(double);
+    const long long n_envs = e->env_cond ? e->n / e->bodies_per_env : 0;
+    if (e->dtype == H2O_F32)
+        water_slope_sample_kernel<float><<<grid, 256, smem, s>>>(wv, env_args(e), n_envs, e->surface_z,
+                                                                 static_cast<const float*>(points), env_index, m, out);
+    else
+        water_slope_sample_kernel<double><<<grid, 256, smem, s>>>(wv, env_args(e), n_envs, e->surface_z,
+                                                                  static_cast<const double*>(points), env_index, m, out);
     CUDA_TRY(cudaGetLastError());
     return H2O_OK;
 }
@@ -1455,17 +1501,21 @@ int h2o_rollout_persistent(h2o_handle h, int n_steps, double dt, double gravity,
     const bool st = e->stats_on;
     const bool env = e->env_cond != nullptr;
     const bool cg = e->grid.vals != nullptr;
-#define H2O_ROLLOUT(S, ST, ENV, CG) \
-    if (st == ST && env == ENV && cg == CG) rollout_persistent_kernel<S, ST, ENV, CG><<<grid, block, smem, s>>>(a)
-#define H2O_ROLLOUTS(S) \
-    H2O_ROLLOUT(S, true, true, false); H2O_ROLLOUT(S, true, false, false);   \
-    H2O_ROLLOUT(S, false, true, false); H2O_ROLLOUT(S, false, false, false); \
-    H2O_ROLLOUT(S, true, true, true); H2O_ROLLOUT(S, true, false, true);     \
-    H2O_ROLLOUT(S, false, true, true); H2O_ROLLOUT(S, false, false, true)
+    const bool sl = slope_on(e);
+#define H2O_ROLLOUT(S, ST, ENV, CG, SL)              \
+    if (st == ST && env == ENV && cg == CG && sl == SL) \
+    rollout_persistent_kernel<S, ST, ENV, CG, SL><<<grid, block, smem, s>>>(a)
+#define H2O_ROLLOUTS(S, SL) \
+    H2O_ROLLOUT(S, true, true, false, SL); H2O_ROLLOUT(S, true, false, false, SL);   \
+    H2O_ROLLOUT(S, false, true, false, SL); H2O_ROLLOUT(S, false, false, false, SL); \
+    H2O_ROLLOUT(S, true, true, true, SL); H2O_ROLLOUT(S, true, false, true, SL);     \
+    H2O_ROLLOUT(S, false, true, true, SL); H2O_ROLLOUT(S, false, false, true, SL)
     if (e->dtype == H2O_F32) {
-        H2O_ROLLOUTS(float);
+        H2O_ROLLOUTS(float, false);
+        H2O_ROLLOUTS(float, true);
     } else {
-        H2O_ROLLOUTS(double);
+        H2O_ROLLOUTS(double, false);
+        H2O_ROLLOUTS(double, true);
     }
 #undef H2O_ROLLOUTS
 #undef H2O_ROLLOUT

@@ -359,9 +359,75 @@ H2O_HD void waterline(H pz, H r20h, H r21h, H r22h, H dxh, H dyh, H dzh, Waterli
     w.partial = partial;
 }
 
+// Separately rounded products and sums that the compiler neither contracts nor merges with other arithmetic
+// (slope_rows: a kernel's remaining code must compile as it does without the slope).
+H2O_HD double h2o_mul_rn(double a, double b)
+{
+#if defined(__CUDA_ARCH__)
+    return __dmul_rn(a, b);
+#else
+    volatile double r = a * b;
+    return r;
+#endif
+}
+H2O_HD double h2o_add_rn(double a, double b)
+{
+#if defined(__CUDA_ARCH__)
+    return __dadd_rn(a, b);
+#else
+    volatile double r = a + b;
+    return r;
+#endif
+}
+H2O_HD float h2o_mul_rn(float a, float b)
+{
+#if defined(__CUDA_ARCH__)
+    return __fmul_rn(a, b);
+#else
+    volatile float r = a * b;
+    return r;
+#endif
+}
+H2O_HD float h2o_add_rn(float a, float b)
+{
+#if defined(__CUDA_ARCH__)
+    return __fadd_rn(a, b);
+#else
+    volatile float r = a + b;
+    return r;
+#endif
+}
+
+// Wave-slope submersion (h2o_set_wave_slope): the keypoints are tested against the plane through the waterline with
+// normal n = (-sx, -sy, 1) instead of the horizontal one.  Keypoint k (body frame) has height
+// (p_z - W) + n . (R k) = (p_z - W) + e . k with e = R^T n, i.e. e_c = (R_2c - sx R_0c) - sy R_1c, formed in H;
+// waterline() then takes e in place of row 2 of R.  Rows 0 and 1 of R (plus diag_shift on the diagonal: the Warp
+// twin's R + 2 dq I) are formed here from q = (x, y, z, w) with the reference's formula, every operation separately
+// rounded, so that nothing is shared with the caller's own rotation and the rest of the caller is unchanged.
+// n is not normalised: every sign test and the ratio -z_min / (z_max - z_min) are invariant to its length.
+// sx = sy = 0 gives e = row 2 (up to the sign of a zero, which no test sees).
+template <typename H>
+H2O_HD void slope_rows(H sx, H sy, H qx, H qy, H qz, H qw, H diag_shift, H& e0, H& e1, H& e2)
+{
+    const H x2 = h2o_add_rn(qx, qx), y2 = h2o_add_rn(qy, qy), z2 = h2o_add_rn(qz, qz);
+    const H xx = h2o_mul_rn(qx, x2), xy = h2o_mul_rn(qx, y2), xz = h2o_mul_rn(qx, z2);
+    const H yy = h2o_mul_rn(qy, y2), yz = h2o_mul_rn(qy, z2), zz = h2o_mul_rn(qz, z2);
+    const H wx = h2o_mul_rn(qw, x2), wy = h2o_mul_rn(qw, y2), wz = h2o_mul_rn(qw, z2);
+    const H r00 = h2o_add_rn(h2o_add_rn(H(1), -h2o_add_rn(yy, zz)), diag_shift), r01 = h2o_add_rn(xy, -wz),
+            r02 = h2o_add_rn(xz, wy);
+    const H r10 = h2o_add_rn(xy, wz), r11 = h2o_add_rn(h2o_add_rn(H(1), -h2o_add_rn(xx, zz)), diag_shift),
+            r12 = h2o_add_rn(yz, -wx);
+    e0 = h2o_add_rn(h2o_add_rn(e0, -h2o_mul_rn(sx, r00)), -h2o_mul_rn(sy, r10));
+    e1 = h2o_add_rn(h2o_add_rn(e1, -h2o_mul_rn(sx, r01)), -h2o_mul_rn(sy, r11));
+    e2 = h2o_add_rn(h2o_add_rn(e2, -h2o_mul_rn(sx, r02)), -h2o_mul_rn(sy, r12));
+}
+
 // One body, branch-free.  kExactTrig: asin/sin as the reference vs 2d*sqrt(1-d^2).
-template <typename H, typename L, bool kExactTrig>
-H2O_HD void body_terms(const BodyIn<H, L>& in, Terms<H, L>& t, const uint32_t* given_mask = nullptr)
+// kSlope: the waterline is the local tangent plane of slope (sx, sy) (slope_rows); everything after the waterline
+// uses the real R.
+template <typename H, typename L, bool kExactTrig, bool kSlope = false>
+H2O_HD void body_terms(const BodyIn<H, L>& in, Terms<H, L>& t, const uint32_t* given_mask = nullptr, H sx = H(0),
+                       H sy = H(0))
 {
     // ---- rotation (numba_hydrodynamics.py:14-49).  Row 2 in H for the waterline.
     const H hx2 = in.qx + in.qx, hy2 = in.qy + in.qy, hz2 = in.qz + in.qz;
@@ -374,12 +440,14 @@ H2O_HD void body_terms(const BodyIn<H, L>& in, Terms<H, L>& t, const uint32_t* g
     const H r22h = (H(1) - (in.qx * hx2 + in.qy * hy2)) + diag_shift;
 
     const H dxh = H(in.dimx), dyh = H(in.dimy), dzh = H(in.dimz);
+    H e0 = r20h, e1 = r21h, e2 = r22h;  // the waterline rows
+    if (kSlope) slope_rows<H>(sx, sy, in.qx, in.qy, in.qz, in.qw, diag_shift, e0, e1, e2);
     Waterline<H> wl;
     if (given_mask) {  // a caller that has run the identical 27 H compares already (body_wrench_fast)
         wl.mask = *given_mask;
-        waterline<H, false>(in.pz, r20h, r21h, r22h, dxh, dyh, dzh, wl);
+        waterline<H, false>(in.pz, e0, e1, e2, dxh, dyh, dzh, wl);
     } else {
-        waterline<H>(in.pz, r20h, r21h, r22h, dxh, dyh, dzh, wl);
+        waterline<H>(in.pz, e0, e1, e2, dxh, dyh, dzh, wl);
     }
     const uint32_t mask = wl.mask;
     const H ratio = wl.ratio;
@@ -615,9 +683,11 @@ H2O_HD void net_wrench(const Terms<H, L>& t, L mass, L F[3], L T[3], bool& clamp
 // fp64 mode, which keeps the world-frame formulation above.  The one place where dq matters
 // even in fp32 (the cancelling cop x F_d, see body_terms) keeps its first-order dq term.
 // ---------------------------------------------------------------------------
-template <typename H, typename L, bool kWarpSkip = false>
+// kSlope: as body_terms (the tangent-plane waterline of slope (sx, sy)).
+template <typename H, typename L, bool kWarpSkip = false, bool kSlope = false>
 H2O_HD void body_wrench_fast(const BodyIn<H, L>& in, L mass, L F[3], L T[3], bool& clamped, H& ratio_out,
-                             bool& still, bool& suspect, uint32_t& mask_out, L* diag = nullptr)
+                             bool& still, bool& suspect, uint32_t& mask_out, L* diag = nullptr, H sx = H(0),
+                             H sy = H(0))
 {
     // ---- waterline in H (the same function body_terms calls)
     const H hx2 = in.qx + in.qx, hy2 = in.qy + in.qy, hz2 = in.qz + in.qz;
@@ -630,7 +700,13 @@ H2O_HD void body_wrench_fast(const BodyIn<H, L>& in, L mass, L F[3], L T[3], boo
     const H dqh = ((in.qx * in.qx + in.qy * in.qy) + (in.qz * in.qz + in.qw * in.qw)) - H(1);
     const H dxh = H(in.dimx), dyh = H(in.dimy), dzh = H(in.dimz);
     Waterline<H> wl;
-    waterline<H, true, kWarpSkip>(in.pz, r20h, r21h, r22h, dxh, dyh, dzh, wl);
+    if (kSlope) {
+        H e0 = r20h, e1 = r21h, e2 = r22h;
+        slope_rows<H>(sx, sy, in.qx, in.qy, in.qz, in.qw, H(0), e0, e1, e2);
+        waterline<H, true, kWarpSkip>(in.pz, e0, e1, e2, dxh, dyh, dzh, wl);
+    } else {
+        waterline<H, true, kWarpSkip>(in.pz, r20h, r21h, r22h, dxh, dyh, dzh, wl);
+    }
     const uint32_t mask = wl.mask;
     const H ratio = wl.ratio;
     const bool partial = wl.partial;

@@ -32,6 +32,14 @@ enum : int {
 struct WaveSample {
     double eta, ux, uy, uz;
 };
+// What a slope instantiation (h2o_set_wave_slope) returns: the field and the surface slope (sx, sy).  The result type
+// carries the slope, so that instantiations without it keep their signatures.
+struct WaveSlopeSample {
+    WaveSample field;
+    double sx, sy;
+};
+template <bool kSlope> struct WaveResult { using type = WaveSample; };
+template <> struct WaveResult<true> { using type = WaveSlopeSample; };
 
 // theta is formed with separately rounded products and sums, in the order written above, on every
 // platform (no FMA contraction), so that it is the same double the NumPy reference forms: at t ~ 1e5 s
@@ -80,13 +88,17 @@ H2O_HD void wave_table_row(const double comp[5], double depth, double row[WAVE_S
 // the depth decay are then evaluated in float (device: MUFU approximations, |error| < 2^-21 on [-pi, pi]), and
 // the sums are kept in float64.  The field then stays within 2e-6 of sum a_j (elevation) and of
 // sum a_j omega_j (velocity) of the float64 values (tests/test_waves.py).
-template <bool kF32>
-H2O_HD WaveSample wave_eval(const double* tab, int n, double depth, double px, double py, double z_rel, double t)
+// kSlope: also the surface gradient sum_j -a_j (kx_j, ky_j) sin theta_j, from the same sine as u_z (float in the fp32
+// policy) with float64 sums (WaveSlopeSample).  Without it nothing of the gradient is formed.
+template <bool kF32, bool kSlope = false>
+H2O_HD typename WaveResult<kSlope>::type wave_eval(const double* tab, int n, double depth, double px, double py,
+                                                  double z_rel, double t)
 {
     const bool deep = !(depth < INFINITY);
     double z = z_rel < 0.0 ? z_rel : 0.0;
     if (!deep && z < -depth) z = -depth;
     WaveSample s{0.0, 0.0, 0.0, 0.0};
+    double gx = 0.0, gy = 0.0;
     for (int j = 0; j < n; ++j) {
         const double* c = tab + WAVE_STRIDE * j;
         const double th = wave_add(wave_add(wave_add(wave_mul(c[WAVE_KX], px), wave_mul(c[WAVE_KY], py)),
@@ -118,8 +130,14 @@ H2O_HD WaveSample wave_eval(const double* tab, int n, double depth, double px, d
         s.ux += uh * c[WAVE_KHAT_X];
         s.uy += uh * c[WAVE_KHAT_Y];
         s.uz += c[WAVE_A_OMEGA] * S * sn;
+        if constexpr (kSlope) {
+            const double as = c[WAVE_A] * sn;
+            gx -= as * c[WAVE_KX];
+            gy -= as * c[WAVE_KY];
+        }
     }
-    return s;
+    if constexpr (kSlope) return WaveSlopeSample{s, gx, gy};
+    else return s;
 }
 
 // ---------------------------------------------------------------------------
@@ -244,6 +262,15 @@ struct Water {
     double surface_z, cx, cy, cz;
     WaveSample field;
 };
+// water_at's slope instantiation: the same, plus the surface slope (sx, sy) the body is tested against
+// (h2o_set_wave_slope): s * the gradient of eta, (0, 0) without a wave field.  The grid, dz and the env's current
+// contribute none.
+struct WaterSlope {
+    Water water;
+    double sx, sy;
+};
+template <bool kSlope> struct WaterResult { using type = Water; };
+template <> struct WaterResult<true> { using type = WaterSlope; };
 
 // The one composition of the global environment (current, surface_z), the env row (has_row), the current grid
 // (grid, or nullptr), the wave table and the clock value t for a body at p, used by every step kernel, the samplers
@@ -254,11 +281,13 @@ struct Water {
 //   waterline = L + s eta,  flow = ((current + c) + g) + s u.
 // The identity row [0,0,0,0,1,0,0,0] makes each row operation exact, so it reproduces the row-less result bit for
 // bit; a grid of zeros does the same for the grid.
-template <bool kF32>
-H2O_HD Water water_at(const double current[3], double surface_z, bool has_row, const EnvRow& row, const double* tab,
-                      int n_waves, double depth, double t, double px, double py, double pz,
-                      const GridArgs* grid = nullptr)
+template <bool kF32, bool kSlope = false>
+H2O_HD typename WaterResult<kSlope>::type water_at(const double current[3], double surface_z, bool has_row,
+                                                   const EnvRow& row, const double* tab, int n_waves, double depth,
+                                                   double t, double px, double py, double pz,
+                                                   const GridArgs* grid = nullptr)
 {
+    double sx = 0.0, sy = 0.0;
     Water w{surface_z, current[0], current[1], current[2], {0.0, 0.0, 0.0, 0.0}};
     const double* c = row.c;
     if (has_row) {
@@ -279,18 +308,30 @@ H2O_HD Water water_at(const double current[3], double surface_z, bool has_row, c
         w.cz = wave_add(w.cz, g[2]);
     }
     if (n_waves) {
-        w.field = wave_eval<kF32>(tab, n_waves, depth, px, py, z_rel, t);  // the one call site
+        if constexpr (kSlope) {
+            const WaveSlopeSample ws = wave_eval<kF32, true>(tab, n_waves, depth, px, py, z_rel, t);
+            w.field = ws.field;
+            sx = ws.sx;
+            sy = ws.sy;
+        } else {
+            w.field = wave_eval<kF32>(tab, n_waves, depth, px, py, z_rel, t);  // the one call site without slope
+        }
         if (has_row) {
             const double s = c[ENV_SCALE];
             w.field = WaveSample{wave_mul(s, w.field.eta), wave_mul(s, w.field.ux), wave_mul(s, w.field.uy),
                                  wave_mul(s, w.field.uz)};
+            if constexpr (kSlope) {
+                sx = wave_mul(s, sx);
+                sy = wave_mul(s, sy);
+            }
         }
         w.surface_z = wave_add(w.surface_z, w.field.eta);
         w.cx = wave_add(w.cx, w.field.ux);
         w.cy = wave_add(w.cy, w.field.uy);
         w.cz = wave_add(w.cz, w.field.uz);
     }
-    return w;
+    if constexpr (kSlope) return WaterSlope{w, sx, sy};
+    else return w;
 }
 
 }  // namespace h2o

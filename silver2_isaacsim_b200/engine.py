@@ -75,6 +75,7 @@ class HydroEngine:
         self.water_density, self.gravity = float(water_density), float(gravity)
         self.quat_order = quat_order
         self._bound = None
+        self._wave_slope = False
 
     # ------------------------------------------------------------------ lifecycle
     def close(self):
@@ -140,6 +141,35 @@ class HydroEngine:
         comps = np.ascontiguousarray(field.components, dtype=np.float64)
         L.check(self._lib.h2o_set_wave_field(self._h, int(comps.shape[0]),
                                              comps.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), float(field.depth)))
+
+    def set_wave_slope(self, enable: bool = True):
+        """Wave-slope submersion: with a wave field, test each body's keypoints and face centres against the wave
+        surface's local tangent plane (slope ``-sum a k sin theta``, scaled per env) instead of the horizontal plane
+        through its waterline, so that buoyancy and drag see a body tilted against the wave flank (semantics in
+        include/h2o.h, h2o_set_wave_slope).  Off by default; without a wave field it changes nothing.  Drops a
+        captured rollout; ``components`` ignores it."""
+        L.check(self._lib.h2o_set_wave_slope(self._h, int(bool(enable))))
+        self._wave_slope = bool(enable)
+
+    @property
+    def wave_slope(self) -> bool:
+        """Whether wave-slope submersion is on (``set_wave_slope``)."""
+        return self._wave_slope
+
+    def sample_surface_slope(self, points, env=None) -> torch.Tensor:
+        """The surface slope a step uses at ``points`` (m,3) world positions and the current clock: a (m,2) float64
+        CUDA tensor of rows ``sx, sy`` (``waves.slope`` / ``waves.slope_env``), zeros with the mode off or without a
+        wave field.  ``env`` as for ``sample_water``: an index outside ``[0, E)`` gives a NaN row."""
+        pts = self._as_dev(points)
+        if pts.ndim != 2 or pts.shape[1] != 3:
+            raise ValueError(f"points must be (m,3), got {tuple(pts.shape)}")
+        out = torch.empty(pts.shape[0], 2, dtype=torch.float64, device=self.device)
+        idx = None if env is None else self._env_index(env, pts.shape[0])
+        L.check(self._lib.h2o_water_slope_sample(self._h, ctypes.c_void_p(pts.data_ptr()),
+                                                 None if idx is None else ctypes.c_void_p(idx.data_ptr()),
+                                                 int(pts.shape[0]), ctypes.c_void_p(out.data_ptr()),
+                                                 _stream_ptr(self.device)))
+        return out
 
     @property
     def wave_time(self) -> float:

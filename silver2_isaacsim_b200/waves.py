@@ -151,6 +151,22 @@ def evaluate(field: WaveField, points, t, surface_z=0.0) -> np.ndarray:
     return out
 
 
+def slope(field: WaveField, points, t) -> np.ndarray:
+    """Float64 reference of the surface slope at ``points`` (m, 3) (only x, y matter) and clock ``t`` (scalar or one
+    per point): (m, 2) rows ``sx, sy`` = the gradient of ``eta``, ``sum_j -a_j (kx_j, ky_j) sin theta_j`` with the
+    ``theta_j`` of ``evaluate`` (include/h2o.h, h2o_set_wave_slope)."""
+    p = np.asarray(points, dtype=np.float64).reshape(-1, 3)
+    t = _per_point(t, len(p))
+    c = field.components
+    a, kx, ky, w, ph = (c[:, j][None, :] for j in range(5))
+    th = ((kx * p[:, 0:1] + ky * p[:, 1:2]) - w * t) + ph
+    asn = a * np.sin(th)
+    out = np.empty((len(p), 2))
+    out[:, 0] = -(asn * kx).sum(axis=1)
+    out[:, 1] = -(asn * ky).sum(axis=1)
+    return out
+
+
 # Columns of a per-env conditions row (HydroEngine.set_env_conditions, h2o_set_env_conditions)
 COND_CX, COND_CY, COND_CZ, COND_DZ, COND_SCALE, COND_TAU, COND_X0, COND_Y0 = range(8)
 COND_COLS = 8
@@ -202,3 +218,19 @@ def evaluate_env(field: WaveField, points, t: float, cond, env_index, surface_z:
     p[:, 1] = p[:, 1] - r[:, COND_Y0]
     out = evaluate(field, p, t + r[:, COND_TAU], surface_z + r[:, COND_DZ])
     return r[:, COND_SCALE:COND_SCALE + 1] * out
+
+
+def slope_env(field: WaveField, points, t: float, cond, env_index) -> np.ndarray:
+    """Float64 reference of the slope env ``env_index[k]`` sees at ``points[k]`` and clock ``t``:
+    ``s * slope(field, p - origin, t + tau)`` with the env's row of ``cond`` (E, 8), as ``evaluate_env`` forms it
+    (``HydroEngine.sample_surface_slope(points, env)`` with the mode on)."""
+    p = np.array(points, dtype=np.float64).reshape(-1, 3)
+    cond = np.asarray(cond, dtype=np.float64)
+    if cond.ndim != 2 or cond.shape[1] != COND_COLS:
+        raise ValueError(f"cond must be (E, {COND_COLS}), got {cond.shape}")
+    r = cond[np.asarray(env_index, dtype=np.int64).reshape(-1)]
+    if len(r) != len(p):
+        raise ValueError("need one env index per point")
+    p[:, 0] = p[:, 0] - r[:, COND_X0]
+    p[:, 1] = p[:, 1] - r[:, COND_Y0]
+    return r[:, COND_SCALE:COND_SCALE + 1] * slope(field, p, t + r[:, COND_TAU])
