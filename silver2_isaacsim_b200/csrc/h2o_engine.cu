@@ -9,7 +9,9 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <mutex>
 #include <string>
+#include <unordered_map>
 #include <vector>
 
 #include "../../include/h2o_dlpack.h"
@@ -89,10 +91,10 @@ struct h2o_engine {
     int max_ctas_per_sm = 0;   // 0 = as many as fit
     int warp_compat = 0;       // components entry point reproduces the Warp twin's deviations
     int robot_cfg = -1;        // -1 = pick the CTA size by lane utilisation (tuning override: 0,1,2)
-    bool use_pdl = false;      // programmatic dependent launch of the tile kernel
     int rollout_free_bodies = 0;  // 1: rollouts integrate the bound state between steps (free bodies)
     double rollout_gravity = 9.81;
     int last_ctas_per_sm = 0;
+    int last_overlap = 0;      // 1: the last tile launch was captured to start while the previous grid drains
     // bound tensors
     bool bound = false;
     int b_layout = LAYOUT_SPLIT;
@@ -243,6 +245,126 @@ static int tile_bodies_for(int threads, size_t esz, int bodies_per_robot)
     return int(threads / l * l);
 }
 
+// ---------------------------------------------------------------------------
+// launch overlap of consecutive tile kernels
+// ---------------------------------------------------------------------------
+// A tile kernel launched with overlap = 1 loads, computes and stores its first tile before it waits for the previous
+// grid of its stream (h2o_kernels.cuh, step_tile_kernel).  The host allows that only for two tile launches of the
+// library that are adjacent in one stream capture and whose memory accesses do not conflict.  Eager launches always
+// wait first: a kernel launched by someone else between two library launches cannot be seen there.
+
+struct Span {  // bytes [lo, hi) of device memory
+    uintptr_t lo, hi;
+};
+
+struct TileAccess {  // what one tile-kernel launch reads and writes
+    Span rd[8];
+    Span wr[6];
+    int n_rd = 0, n_wr = 0;
+};
+
+static void add_span(Span* s, int& n, const void* p, size_t bytes)
+{
+    if (!p || bytes == 0) return;
+    const uintptr_t lo = reinterpret_cast<uintptr_t>(p);
+    s[n++] = Span{lo, lo + bytes};
+}
+
+static bool spans_meet(const Span* a, int na, const Span* b, int nb)
+{
+    for (int i = 0; i < na; ++i)
+        for (int j = 0; j < nb; ++j)
+            if (a[i].lo < b[j].hi && b[j].lo < a[i].hi) return true;
+    return false;
+}
+
+// The later launch may start before the earlier one has finished: it reads nothing the earlier one writes, writes
+// nothing the earlier one writes, and writes nothing the earlier one reads.
+static bool accesses_commute(const TileAccess& earlier, const TileAccess& later)
+{
+    return !spans_meet(earlier.wr, earlier.n_wr, later.rd, later.n_rd) &&
+           !spans_meet(earlier.wr, earlier.n_wr, later.wr, later.n_wr) &&
+           !spans_meet(later.wr, later.n_wr, earlier.rd, earlier.n_rd);
+}
+
+// Every byte a tile launch of `a` (tile_bodies / n_tiles set) may touch, deferred float64 re-evaluation included.
+template <typename S, int kLayout, int kParam, bool kRobot>
+static TileAccess tile_access(const StepArgs& a)
+{
+    using TL = TileLayout<S, kLayout, kParam>;
+    const size_t rows = size_t(a.n_tiles) * size_t(a.tile_bodies);
+    const size_t col = rows * sizeof(S);
+    TileAccess t;
+    add_span(t.rd, t.n_rd, a.pos, col * TL::E_POS);
+    if (TL::E_QUAT) add_span(t.rd, t.n_rd, a.quat, col * TL::E_QUAT);
+    add_span(t.rd, t.n_rd, a.lin, col * TL::E_LIN);
+    if (TL::E_ANG) add_span(t.rd, t.n_rd, a.ang, col * TL::E_ANG);
+    add_span(t.rd, t.n_rd, a.prev, col * TL::E_PREV);
+    if (kParam == PARAM_PER_BODY) {
+        add_span(t.rd, t.n_rd, a.coeff, col * N_COEFF);
+    } else {
+        add_span(t.rd, t.n_rd, a.coeff, size_t(a.n_types) * N_COEFF * sizeof(S));
+        add_span(t.rd, t.n_rd, a.slot_type, size_t(a.n_slots) * sizeof(int32_t));
+    }
+    add_span(t.wr, t.n_wr, a.out_force, col * 3);
+    add_span(t.wr, t.n_wr, a.out_torque, col * 3);
+    add_span(t.wr, t.n_wr, a.prev, col * TL::E_PREV);
+    if (kRobot && a.bodies_per_robot > 0)
+        add_span(t.wr, t.n_wr, a.out_wrench, rows / size_t(a.bodies_per_robot) * 6 * sizeof(S));
+    add_span(t.wr, t.n_wr, a.stats, N_STATS * sizeof(double));
+    if (rows > 0) {  // the bitmap words of bodies first_body .. first_body + rows - 1
+        const size_t w0 = size_t(a.first_body) >> 5, w1 = (size_t(a.first_body) + rows - 1) >> 5;
+        add_span(t.wr, t.n_wr, a.redo_bitmap + w0, (w1 - w0 + 1) * sizeof(uint32_t));
+    }
+    return t;
+}
+
+// The library's last tile launch per stream, kept while that stream is being captured.
+struct LastTile {
+    unsigned long long capture_id;
+    cudaGraphNode_t node;
+    TileAccess access;
+};
+static std::mutex g_last_tile_mu;
+static std::unordered_map<cudaStream_t, LastTile> g_last_tile;
+
+// Any other library kernel on the stream: the next tile launch there waits first.
+static void forget_last_tile(cudaStream_t s)
+{
+    std::lock_guard<std::mutex> lk(g_last_tile_mu);
+    g_last_tile.erase(s);
+}
+
+struct CaptureState {
+    bool capturing = false;
+    unsigned long long id = 0;
+    cudaGraphNode_t only_dep = nullptr;  // the single node the next captured work depends on, or nullptr
+};
+
+static CaptureState capture_state(cudaStream_t s)
+{
+    CaptureState c;
+    cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
+    const cudaGraphNode_t* deps = nullptr;
+    const cudaGraphEdgeData* edges = nullptr;
+    size_t n_deps = 0;
+    if (cudaStreamGetCaptureInfo_v3(s, &st, &c.id, nullptr, &deps, &edges, &n_deps) != cudaSuccess) {
+        cudaGetLastError();  // not an error of the launch: it then simply waits first
+        return CaptureState{};
+    }
+    c.capturing = st == cudaStreamCaptureStatusActive;
+    if (c.capturing && n_deps == 1) c.only_dep = deps[0];
+    return c;
+}
+
+// The overlap decision for a tile launch with access record `acc` after `last` (nullptr = none) in a stream in
+// capture state `c`.
+static bool may_start_early(const LastTile* last, const CaptureState& c, const TileAccess& acc)
+{
+    return c.capturing && last && last->capture_id == c.id && c.only_dep && c.only_dep == last->node &&
+           accesses_commute(last->access, acc);
+}
+
 template <typename S, int kLayout, int kParam, bool kRobot, bool kStats, typename C>
 static int launch_tile(h2o_engine* e, StepArgs& a, cudaStream_t stream)
 {
@@ -269,30 +391,40 @@ static int launch_tile(h2o_engine* e, StepArgs& a, cudaStream_t stream)
     a.tile_bodies = tb_max;
     a.n_tiles = int(std::min<long long>(a.n / tb_max, 0x7fffffff));
     const int grid = int(std::max<long long>(1, std::min<long long>(a.n_tiles, slots)));
+    a.overlap = 0;
     if (e->dry_run) {
         e->launches += 1;
         e->last_ctas_per_sm = cps;
         return H2O_OK;
     }
-    if (e->use_pdl) {
-        cudaLaunchConfig_t cfg;
-        memset(&cfg, 0, sizeof cfg);
-        cfg.gridDim = dim3(grid);
-        cfg.blockDim = dim3(C::kThreads);
-        cfg.dynamicSmemBytes = TLn::smem();
-        cfg.stream = stream;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, TLn::kernel(), a));
-    } else {
-        TLn::kernel()<<<grid, C::kThreads, TLn::smem(), stream>>>(a);
-    }
+    // Programmatic stream serialisation on every launch: after a tile launch of the library the kernel may start
+    // as the previous grid drains (it waits or not as a.overlap says); after any other node it is an ordinary
+    // dependency, since the kernel then waits before touching global memory.
+    const TileAccess acc = tile_access<S, kLayout, kParam, kRobot>(a);
+    std::lock_guard<std::mutex> lk(g_last_tile_mu);
+    const CaptureState before = capture_state(stream);
+    auto it = g_last_tile.find(stream);
+    a.overlap = may_start_early(it == g_last_tile.end() ? nullptr : &it->second, before, acc) ? 1 : 0;
+    cudaLaunchConfig_t cfg;
+    memset(&cfg, 0, sizeof cfg);
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(C::kThreads);
+    cfg.dynamicSmemBytes = TLn::smem();
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    const cudaError_t err = cudaLaunchKernelEx(&cfg, TLn::kernel(), a);
+    const CaptureState after = err == cudaSuccess && before.capturing ? capture_state(stream) : CaptureState{};
+    if (after.capturing && after.only_dep) g_last_tile[stream] = LastTile{after.id, after.only_dep, acc};
+    else if (it != g_last_tile.end()) g_last_tile.erase(it);
+    CUDA_TRY(err);
     CUDA_TRY(cudaGetLastError());
     e->launches += 1;
     e->last_ctas_per_sm = cps;
+    e->last_overlap = a.overlap;
     return H2O_OK;
 }
 
@@ -313,24 +445,8 @@ static int launch_direct(h2o_engine* e, const StepArgs& a, long long body_begin,
         e->launches += 1;
         return H2O_OK;
     }
-    if (e->use_pdl) {
-        cudaLaunchConfig_t cfg;
-        memset(&cfg, 0, sizeof cfg);
-        cfg.gridDim = dim3(grid);
-        cfg.blockDim = dim3(256);
-        cfg.dynamicSmemBytes = smem;
-        cfg.stream = stream;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        if (slope_on(e))
-            CUDA_TRY(cudaLaunchKernelEx(&cfg, step_direct_kernel<S, kLayout, kParam, kStats, true>, a, body_begin, wv, ev,
-                                        gv));
-        else
-            CUDA_TRY(cudaLaunchKernelEx(&cfg, step_direct_kernel<S, kLayout, kParam, kStats>, a, body_begin, wv, ev, gv));
-    } else if (slope_on(e)) {
+    forget_last_tile(stream);
+    if (slope_on(e)) {
         step_direct_kernel<S, kLayout, kParam, kStats, true><<<grid, 256, smem, stream>>>(a, body_begin, wv, ev, gv);
     } else {
         step_direct_kernel<S, kLayout, kParam, kStats><<<grid, 256, smem, stream>>>(a, body_begin, wv, ev, gv);
@@ -351,6 +467,7 @@ static int launch_robot_wrench(h2o_engine* e, const StepArgs& a, long long robot
         e->launches += 1;
         return H2O_OK;
     }
+    forget_last_tile(stream);
     robot_wrench_kernel<S, kLayout><<<grid, 256, 0, stream>>>(a, robot_begin);
     CUDA_TRY(cudaGetLastError());
     e->launches += 1;
@@ -470,6 +587,7 @@ static int advance_clock(h2o_engine* e, double dt, int n, cudaStream_t stream)
         e->launches += 1;
         return H2O_OK;
     }
+    forget_last_tile(stream);
     advance_clock_kernel<<<1, 1, 0, stream>>>(e->wave_clock, dt, n);
     CUDA_TRY(cudaGetLastError());
     e->launches += 1;
@@ -513,6 +631,7 @@ static int step_device(h2o_engine* e, int layout, const void* pos, const void* q
     a.no_fallback = e->no_fallback;
     a.warp_compat = e->warp_compat;
     a.redo_bitmap = e->redo_bitmap;
+    e->last_overlap = 0;
     a.surface_eta = e->surface_eta ? static_cast<const char*>(e->surface_eta) + size_t(first_body) * e->esz : nullptr;
     const int rc = e->dtype == H2O_F32 ? step_typed<float>(e, layout, a, stream) : step_typed<double>(e, layout, a, stream);
     if (rc || !clock_runs(e) || !tick) return rc;
@@ -572,7 +691,6 @@ int h2o_create(h2o_handle* out, int64_t n_bodies, int dtype, int device)
     e->esz = dtype == H2O_F32 ? 4 : 8;
     e->sm_count = prop.multiProcessorCount;
     if (const char* v = getenv("H2O_MAX_CTAS_PER_SM")) e->max_ctas_per_sm = atoi(v);
-    if (const char* v = getenv("H2O_PDL")) e->use_pdl = atoi(v) != 0;
     if (const char* v = getenv("H2O_NO_FALLBACK")) e->no_fallback = std::max(0, atoi(v));
     if (const char* v = getenv("H2O_ROBOT_CFG")) e->robot_cfg = std::max(-1, std::min(2, atoi(v)));
     const size_t bitmap_bytes = (size_t(n_bodies) / 32 + 2) * sizeof(uint32_t);
@@ -705,6 +823,7 @@ int h2o_wave_time_write(h2o_handle h, double t, h2o_stream stream)
     if (!e) return H2O_ERR_BAD_HANDLE;
     if (!std::isfinite(t)) return fail(H2O_ERR_BAD_ARGUMENT, "wave time must be finite");
     DeviceGuard g(e->device);
+    forget_last_tile(static_cast<cudaStream_t>(stream));
     set_clock_kernel<<<1, 1, 0, static_cast<cudaStream_t>(stream)>>>(e->wave_clock, t);
     CUDA_TRY(cudaGetLastError());
     return H2O_OK;
@@ -1355,6 +1474,7 @@ static int integrate_device(h2o_engine* e, void* pos, void* quat, void* lin, voi
         e->launches += 1;
         return H2O_OK;
     }
+    forget_last_tile(s);
     if (e->dtype == H2O_F32) free_body_kernel<float><<<grid, 256, 0, s>>>(a);
     else free_body_kernel<double><<<grid, 256, 0, s>>>(a);
     CUDA_TRY(cudaGetLastError());
@@ -1622,7 +1742,10 @@ static int step_host_impl(h2o_engine* e, int layout, const void* const in[4], vo
     // device-wide host synchronisation.
     if (!e->hp_event) CUDA_TRY(cudaEventCreateWithFlags(&e->hp_event, cudaEventDisableTiming));
     CUDA_TRY(cudaEventRecord(e->hp_event, cudaStreamLegacy));
-    for (int i = 0; i < HOST_PIPE_STREAMS; ++i) CUDA_TRY(cudaStreamWaitEvent(e->hp_stream[i], e->hp_event, 0));
+    for (int i = 0; i < HOST_PIPE_STREAMS; ++i) {
+        CUDA_TRY(cudaStreamWaitEvent(e->hp_stream[i], e->hp_event, 0));
+        forget_last_tile(e->hp_stream[i]);
+    }
 
     // ---- zero-copy path
     {
@@ -2063,6 +2186,49 @@ int h2o_export_prev_dl(h2o_handle h, DLManagedTensor** out)
     x->mt.deleter = prev_export_deleter;
     *out = &x->mt;
     return H2O_OK;
+}
+
+// ---------------------------------------------------------------------------
+// Diagnostics of the launch overlap for the test suite; not part of the public ABI (include/h2o.h).
+// ---------------------------------------------------------------------------
+#define H2O_DIAG __attribute__((visibility("default")))
+
+// 1 if the handle's last tile launch was captured to start while the previous grid of its stream drained.
+H2O_DIAG int h2o_diag_last_overlap(h2o_handle h)
+{
+    h2o_engine* e = check(h);
+    return e ? e->last_overlap : -1;
+}
+
+// The overlap decision of launch_tile, made without a device, for two fp32 split-layout per-body tile launches
+// (robot mode when bodies_per_robot > 0) over n bodies each.  ptrs: pos, quat, lin, ang, prev, coeff, force, torque,
+// wrench, stats, redo bitmap.  relation: 0 = eager, 1 = same capture and the later launch depends on the earlier one
+// alone, 2 = same capture with other dependencies, 3 = another capture.  Returns 1 = start early, 0 = wait first.
+H2O_DIAG int h2o_diag_overlap_decision(const void* const earlier[11], int64_t earlier_n, const void* const later[11],
+                                       int64_t later_n, int bodies_per_robot, int relation)
+{
+    auto access = [&](const void* const p[11], int64_t n) {
+        StepArgs a;
+        memset(&a, 0, sizeof a);
+        a.pos = p[0]; a.quat = p[1]; a.lin = p[2]; a.ang = p[3]; a.prev = const_cast<void*>(p[4]); a.coeff = p[5];
+        a.out_force = const_cast<void*>(p[6]); a.out_torque = const_cast<void*>(p[7]);
+        a.out_wrench = const_cast<void*>(p[8]);
+        a.stats = static_cast<double*>(const_cast<void*>(p[9]));
+        a.redo_bitmap = static_cast<uint32_t*>(const_cast<void*>(p[10]));
+        a.n = n;
+        a.bodies_per_robot = bodies_per_robot;
+        a.tile_bodies = tile_bodies_for(128, sizeof(float), bodies_per_robot);
+        a.n_tiles = a.tile_bodies > 0 ? int(n / a.tile_bodies) : 0;
+        return bodies_per_robot > 0 ? tile_access<float, LAYOUT_SPLIT, PARAM_PER_BODY, true>(a)
+                                    : tile_access<float, LAYOUT_SPLIT, PARAM_PER_BODY, false>(a);
+    };
+    const cudaGraphNode_t node = reinterpret_cast<cudaGraphNode_t>(uintptr_t(0x1000));
+    const LastTile last{7, node, access(earlier, earlier_n)};
+    CaptureState c;
+    c.capturing = relation != 0;
+    c.id = relation == 3 ? 8 : 7;
+    c.only_dep = relation == 1 || relation == 3 ? node : nullptr;
+    return may_start_early(&last, c, access(later, later_n)) ? 1 : 0;
 }
 
 }  // extern "C"

@@ -91,6 +91,8 @@ struct StepArgs {
                              // Numba path: every body through the float64 world-frame formulation, direct kernel only
     int no_fallback;         // study knob H2O_NO_FALLBACK: 1 = keep the fast-path result of flagged bodies,
                              // k = 2^j > 1 = re-evaluate exactly every k-th body instead (cost measurements)
+    int overlap;             // tile kernel: 1 = the host proved that this launch touches nothing the previous launch in
+                             // the stream writes, and nothing it writes is read there: start before waiting for it
 };
 
 // Optional built-in wave field (h2o_set_wave_field): n rows of WAVE_STRIDE doubles, the water depth (+inf = deep)
@@ -176,8 +178,10 @@ template <int N> __device__ __forceinline__ void bulk_wait_all()
 {
     asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory");
 }
-// Programmatic dependent launch (PDL): let the next kernel in the stream become resident while
-// this one drains, and make this one wait for its predecessor before touching global memory.
+// Programmatic dependent launch (PDL).  griddepcontrol.wait returns once the previous grid of the stream has completed
+// and its writes are visible; launch_dependents lets the next grid start once every CTA of this one has executed it (or
+// exited).  Invariant of every kernel here: no thread executes launch_dependents before its own wait has returned.  So
+// when a grid starts early, only the one grid before it can still be running -- the launch the host checked it against.
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait_prerequisites() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void prefetch_l2_keep(const void* p)
@@ -738,7 +742,6 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) step_tile_kernel(const _
                    o_coeff = o_prev + b_prev;
     const uint32_t oo_t = 3u * TB * sizeof(S), oo_prev = 2 * oo_t;
 
-    pdl_launch_dependents();  // no-op unless launched with the PDL attribute
     if (tid == 0) {
         for (int s = 0; s < kStagesIn; ++s) mbar_init(&full_bar[s], 1);
         mbar_fence_init();
@@ -746,13 +749,21 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) step_tile_kernel(const _
         redo_count[0] = 0;  // deferred entries
         redo_count[1] = 0;  // overflow in the current tile
     }
-    pdl_wait_prerequisites();  // everything below reads / writes global memory
 
     // Tile schedule: full tiles dealt round-robin (tile = cta + it*grid).  At any moment the resident
     // CTAs stream one compact window of every array, which is what DRAM pages and the TLB like.
     // Measured alternatives (profiles/r01_sweep_schedules.log): one contiguous share per CTA costs
     // ~10 % of the bandwidth; splitting the ragged last round evenly over all CTAs is ~0.8 us slower.
+    // The ragged extra tiles go to the lowest blockIdx values: those CTAs become resident first when this grid
+    // starts in the slots of a draining predecessor (overlap mode), so the extra round evens out.
     const int n_it = (a.n_tiles > int(blockIdx.x)) ? (a.n_tiles - int(blockIdx.x) + int(gridDim.x) - 1) / int(gridDim.x) : 0;
+    // Overlap mode: the first tile is loaded, computed and stored while the previous grid may still run; the wait
+    // (and only then the trigger for the next grid) follows it.  Otherwise wait before the first global access.
+    const bool early = a.overlap && n_it > 0;
+    if (!early) {
+        pdl_wait_prerequisites();
+        pdl_launch_dependents();
+    }
     const long long round_stride = (long long)gridDim.x * TB;
     const long long first_begin = (long long)blockIdx.x * TB;
     auto tile_start = [&](int it) -> long long { return first_begin + it * round_stride; };
@@ -949,6 +960,10 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) step_tile_kernel(const _
                 reinterpret_cast<S*>(a.out_wrench)[(tile_begin / bpr) * 6 + idx] = sum;
             }
         }
+        if (early && it == 0) {
+            pdl_wait_prerequisites();
+            pdl_launch_dependents();
+        }
     }
     if (sizeof(S) == 4 && !kCopyOnly) {
         __syncthreads();  // every tile done: the list is complete, every bulk store has been issued
@@ -1056,8 +1071,8 @@ __global__ void __launch_bounds__(256) step_direct_kernel(const __grid_constant_
     __shared__ S table[(kParam == PARAM_TABLE) ? MAX_TABLE_TYPES * N_COEFF : 1];
     __shared__ unsigned char slot_map[(kParam == PARAM_TABLE) ? MAX_TABLE_SLOTS : 1];
     extern __shared__ double wave_smem[];
-    pdl_launch_dependents();   // no-ops unless launched with the PDL attribute
-    pdl_wait_prerequisites();
+    pdl_wait_prerequisites();  // returns at once (plain launch); the trigger lets a following tile launch start early
+    pdl_launch_dependents();
     if (wv.n) {
         stage_waves(wave_smem, wv.tab, wv.clock, wv.n);
         __syncthreads();

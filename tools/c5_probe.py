@@ -18,4 +18,4 @@ for free in (False, True):
     ms_e = timeit(lambda: [e.step_bound(wl.dt) for _ in range(1000)]) if not free else float("nan")
     e.capture_rollout(1000, wl.dt)
     ms_g = timeit(e.launch_rollout)
-    print(f"N={wl.n} free_bodies={free} PDL={os.environ.get('H2O_PDL','0')}: eager {ms_e:.2f} us/step, graph {ms_g:.2f} us/step, kernel {e.last_kernel}")
+    print(f"N={wl.n} free_bodies={free}: eager {ms_e:.2f} us/step, graph {ms_g:.2f} us/step, kernel {e.last_kernel}")
