@@ -164,6 +164,36 @@ H2O_API int h2o_wave_sample(h2o_handle h, const void* points, int64_t m, double*
  * that takes a wave field honours the mode (eager, bound, captured, host-buffer, h2o_rollout_persistent);
  * h2o_components ignores it, as it ignores the field.  Like every h2o_set_* call this drops a captured rollout. */
 H2O_API int h2o_set_wave_slope(h2o_handle h, int enable);
+/* Fluid-acceleration loads: enable != 0 adds the inertia part of Morison's equation, which dominates the wave loads
+ * on bodies much smaller than the wavelength.  The fluid acceleration a_f is evaluated at the body centre, at the
+ * (X, Y, Z, T) the flow is evaluated at (env-local position, depth below the env's mean level, env time):
+ *   waves: a_w = sum_j a_j omega_j^2 (C_j sin theta_j khat_j, -S_j cos theta_j), the time derivative of the orbital
+ *          velocity, with its theta_j, C_j, S_j and z clamp (fp32 mode: the same float sine, cosine and decay, double
+ *          sums; within 2e-6 of sum a_j omega_j^2)
+ *   grid:  a_g = (G_{f+1} - G_f) / ht for nt > 1 and T inside [t0, t0 + (nt - 1) ht], G_f and G_{f+1} the spatial
+ *          interpolations of the two frames the interpolation in time blends (separately rounded float64
+ *          operations); 0 where the grid is held in time, and for nt == 1
+ *   a_f = a_g + s a_w, s the env's wave scale (1 without env conditions), every operation separately rounded.
+ * The global and env currents are constant and the caller height array (h2o_set_surface_heights) moves no water:
+ * they contribute nothing.  The convective term (u . grad) u is omitted (second order for linear waves), and so is
+ * the rotation of the flow (Airy waves are irrotational).
+ * With r the submersion ratio, V = dimx dimy dimz and rho = waterDensity, two terms join the net wrench before the
+ * safety clamp:
+ *   Froude-Krylov  F_FK = rho r V a_f at the centre of buoyancy: the torque gains (cob - p) x F_FK
+ *   added mass     its linear part sees a_b - a_f in place of a_b: with the wrapper's diagonal (isotropic C_a rho V)
+ *                  this adds C_a rho r V a_f at the body origin (no arm, like the added-mass force itself); with dense
+ *                  matrices (h2o_set_added_mass_dense) it is M [R^T (a_b - a_f); R^T alpha_b], so the coupling block
+ *                  turns a_f into a torque.  The angular part is unchanged.
+ * Dry bodies (r = 0) get nothing.  a_b stays the reference's backward difference of body velocities
+ * (hydrodynamics_behavior.py:196-202), half a step behind a_f.  fp32 mode counts both groups in the force and torque
+ * conditioning checks, so bodies where they cancel drag or buoyancy are re-evaluated in float64.
+ * Default 0.  With the mode off, or with no wave field and no grid with nt > 1, steps and rollouts run the code
+ * without the mode and are bit-identical to a handle without it.  Every step path that takes a wave field honours the
+ * mode (eager, bound, captured, host-buffer, h2o_rollout_persistent; h2o_reset_envs with restart_waves restarts an
+ * env's a_f with its sea); h2o_components ignores it, as it ignores the field.  H2O_ERR_NOT_CONFIGURED when Warp
+ * compatibility is on (and h2o_set_warp_compat refuses to turn it on while this mode is on): the Warp twin has no such
+ * term.  Like every h2o_set_* call this drops a captured rollout; a refused call leaves it intact. */
+H2O_API int h2o_set_fluid_inertia(h2o_handle h, int enable);
 
 /* Per-env water conditions for vectorised scenes (SURVEY.md 8(f4)).  Envs are contiguous, equal runs of bodies:
  * body i (global index) belongs to env e = i / bodies_per_env, and E = n_bodies / bodies_per_env.  cond_dev is a
@@ -248,6 +278,12 @@ H2O_API int h2o_water_sample(h2o_handle h, const void* points, const int32_t* en
  * env_index without env conditions. */
 H2O_API int h2o_water_slope_sample(h2o_handle h, const void* points, const int32_t* env_index, int64_t m, double* out,
                                    h2o_stream stream);
+/* The fluid acceleration a_f a step uses at given points and the clock's current value (h2o_set_fluid_inertia):
+ * points as for h2o_water_sample, out a DEVICE array (m,3) float64 of rows [ax, ay, az]; zero rows with the mode off
+ * or with neither a wave field nor a grid with nt > 1.  env_index as for h2o_water_sample: a NaN row for an index
+ * outside [0, E), H2O_ERR_NOT_CONFIGURED for env_index without env conditions. */
+H2O_API int h2o_fluid_accel_sample(h2o_handle h, const void* points, const int32_t* env_index, int64_t m, double* out,
+                                   h2o_stream stream);
 
 /* Same twelve scalars, same order as the reference wrapper ctor
  * (numba_hydrodynamics_wrapper.py:9-10): width, depth, height, linear_drag_coefficient,
@@ -296,7 +332,8 @@ H2O_API int h2o_set_kernel(h2o_handle h, int choice);
  * when fully submerged (:57-58), cob = cop = position for a dry body (:59-61, :290).  Applies to h2o_components
  * and to the fused step entry points (the production behaviour script evaluates forces through the Warp wrapper,
  * hydrodynamics_behavior.py:19, :155); the step then runs every body through the float64 formulation on the
- * per-body kernel (a compatibility mode, not a fast path).  Default 0 = the Numba semantics (north star). */
+ * per-body kernel (a compatibility mode, not a fast path).  Default 0 = the Numba semantics (north star).
+ * H2O_ERR_NOT_CONFIGURED for enable != 0 while h2o_set_fluid_inertia is on. */
 H2O_API int h2o_set_warp_compat(h2o_handle h, int enable);
 /* fp32 mode only.  1 (default): every body meets the fp32-mode bound of the parity criterion (|dF|, |dtau| <=
  * max(1e-5 |.|_inf, 1e-6) against the float64 Numba path): the fused step flags the few bodies per 10 000 whose

@@ -55,12 +55,14 @@ SIGNATURES = {
     "h2o_wave_time_read": (c_int, [_P, POINTER(c_double), _P]),
     "h2o_wave_sample": (c_int, [_P, _P, c_int64, _P, _P]),
     "h2o_set_wave_slope": (c_int, [_P, c_int]),
+    "h2o_set_fluid_inertia": (c_int, [_P, c_int]),
     "h2o_set_env_conditions": (c_int, [_P, c_int64, _P]),
     "h2o_reset_envs": (c_int, [_P, _P, c_int, _P]),
     "h2o_wave_sample_env": (c_int, [_P, _P, _P, c_int64, _P, _P]),
     "h2o_set_current_grid": (c_int, [_P, _P, POINTER(c_int64), POINTER(c_double)]),
     "h2o_water_sample": (c_int, [_P, _P, _P, c_int64, _P, _P]),
     "h2o_water_slope_sample": (c_int, [_P, _P, _P, c_int64, _P, _P]),
+    "h2o_fluid_accel_sample": (c_int, [_P, _P, _P, c_int64, _P, _P]),
     "h2o_set_added_mass_dense": (c_int, [_P, c_int, POINTER(c_double), c_int, POINTER(c_int32)]),
     "h2o_set_params_uniform": (c_int, [_P, POINTER(c_double), c_double]),
     "h2o_set_part_table": (c_int, [_P, c_int, POINTER(c_double), c_int, POINTER(c_int32)]),

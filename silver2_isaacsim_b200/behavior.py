@@ -49,7 +49,8 @@ class BatchedHydrodynamicsBehavior:
     def __init__(self, prim_names: Sequence[str], view, device: str = "cuda:0",
                  config_path: Optional[str] = None, dtype: torch.dtype = torch.float32,
                  bodies_per_robot: int = 0, robot_offsets: Optional[Sequence[int]] = None,
-                 warp_compat: bool = False, waves: Optional[WaveField] = None, wave_slope: bool = False):
+                 warp_compat: bool = False, waves: Optional[WaveField] = None, wave_slope: bool = False,
+                 fluid_inertia: bool = False):
         self.prim_names = list(prim_names)
         self._view = view
         self._device = device
@@ -59,6 +60,7 @@ class BatchedHydrodynamicsBehavior:
         self._warp_compat = bool(warp_compat)
         self._waves = waves  # built-in wave field, installed by _setup with its clock at 0
         self._wave_slope = bool(wave_slope)  # test the prims against the wave surface's tangent plane (needs waves)
+        self._fluid_inertia = bool(fluid_inertia)  # Froude-Krylov + added mass on the fluid-relative acceleration
         # robots of unequal size, e.g. [0, 19, 20] for one SILVER2 + the Obsea buoy (the main scene)
         self._robot_offsets = None if robot_offsets is None else [int(o) for o in robot_offsets]
         self._engine: Optional[HydroEngine] = None
@@ -118,6 +120,8 @@ class BatchedHydrodynamicsBehavior:
             self._engine.set_wave_time(0.0)
             if self._wave_slope:
                 self._engine.set_wave_slope(True)
+            if self._fluid_inertia:
+                self._engine.set_fluid_inertia(True)
         if self._robot_offsets is not None:
             self._engine.set_articulation_offsets(self._robot_offsets)
         else:

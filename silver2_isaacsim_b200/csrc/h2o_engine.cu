@@ -83,6 +83,7 @@ struct h2o_engine {
     int n_waves = 0;               // 0 = no wave field
     double wave_depth = INFINITY;
     int wave_slope = 0;            // 1: with a wave field, bodies are tested against the surface's tangent plane
+    int fluid_inertia = 0;         // 1: Froude-Krylov force and added mass on the fluid-relative acceleration
     const double* env_cond = nullptr;  // (n / bodies_per_env, ENV_STRIDE) per-env conditions, borrowed, or nullptr
     long long bodies_per_env = 0;
     GridArgs grid{};  // current grid (borrowed values, dims and geometry); grid.vals == nullptr = none
@@ -430,6 +431,9 @@ static int launch_tile(h2o_engine* e, StepArgs& a, cudaStream_t stream)
 
 // Wave-slope submersion is in effect: the mode is on and there is a wave field to take the slope of.
 static bool slope_on(const h2o_engine* e) { return e->wave_slope && e->n_waves; }
+// Fluid-inertia loads are in effect: the mode is on and something accelerates the water (a wave field, or a grid with
+// more than one frame).  Otherwise the instantiations without the mode run, so that results stay bit-identical.
+static bool inertia_on(const h2o_engine* e) { return e->fluid_inertia && clock_runs(e); }
 
 template <typename S, int kLayout, int kParam, bool kStats>
 static int launch_direct(h2o_engine* e, const StepArgs& a, long long body_begin, cudaStream_t stream)
@@ -446,7 +450,12 @@ static int launch_direct(h2o_engine* e, const StepArgs& a, long long body_begin,
         return H2O_OK;
     }
     forget_last_tile(stream);
-    if (slope_on(e)) {
+    if (inertia_on(e)) {
+        if (slope_on(e))
+            step_direct_kernel<S, kLayout, kParam, kStats, true, true><<<grid, 256, smem, stream>>>(a, body_begin, wv, ev, gv);
+        else
+            step_direct_kernel<S, kLayout, kParam, kStats, false, true><<<grid, 256, smem, stream>>>(a, body_begin, wv, ev, gv);
+    } else if (slope_on(e)) {
         step_direct_kernel<S, kLayout, kParam, kStats, true><<<grid, 256, smem, stream>>>(a, body_begin, wv, ev, gv);
     } else {
         step_direct_kernel<S, kLayout, kParam, kStats><<<grid, 256, smem, stream>>>(a, body_begin, wv, ev, gv);
@@ -817,6 +826,18 @@ int h2o_set_wave_slope(h2o_handle h, int enable)
     return H2O_OK;
 }
 
+int h2o_set_fluid_inertia(h2o_handle h, int enable)
+{
+    h2o_engine* e = check(h);
+    if (!e) return H2O_ERR_BAD_HANDLE;
+    if (enable && e->warp_compat)  // checked before the captured rollout is dropped: a refused call leaves it intact
+        return fail(H2O_ERR_NOT_CONFIGURED,
+                    "fluid-inertia loads follow the Numba semantics: turn Warp compatibility off first");
+    { DeviceGuard gi(e->device); invalidate_graph(e); }
+    e->fluid_inertia = enable != 0;
+    return H2O_OK;
+}
+
 int h2o_wave_time_write(h2o_handle h, double t, h2o_stream stream)
 {
     h2o_engine* e = check(h);
@@ -1018,6 +1039,37 @@ int h2o_water_slope_sample(h2o_handle h, const void* points, const int32_t* env_
                                                                  static_cast<const float*>(points), env_index, m, out);
     else
         water_slope_sample_kernel<double><<<grid, 256, smem, s>>>(wv, env_args(e), n_envs, e->surface_z,
+                                                                  static_cast<const double*>(points), env_index, m, out);
+    CUDA_TRY(cudaGetLastError());
+    return H2O_OK;
+}
+
+int h2o_fluid_accel_sample(h2o_handle h, const void* points, const int32_t* env_index, int64_t m, double* out,
+                           h2o_stream stream)
+{
+    h2o_engine* e = check(h);
+    if (!e) return H2O_ERR_BAD_HANDLE;
+    if (env_index && !e->env_cond) return fail(H2O_ERR_NOT_CONFIGURED, "no env conditions set (h2o_set_env_conditions)");
+    if (m < 0) return fail(H2O_ERR_BAD_ARGUMENT, "m must be >= 0");
+    if (m == 0) return H2O_OK;
+    if (!points || !out) return fail(H2O_ERR_BAD_ARGUMENT, "NULL points / out");
+    DeviceGuard g(e->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int grid = int((m + 255) / 256);
+    // the a_f a step uses: none unless the mode is in effect
+    WaveArgs wv = wave_args(e);
+    GridArgs gv = e->grid;
+    if (!inertia_on(e)) {
+        wv.n = 0;
+        gv.vals = nullptr;
+    }
+    const size_t smem = (size_t(wv.n) * WAVE_STRIDE + 1) * sizeof(double);
+    const long long n_envs = e->env_cond ? e->n / e->bodies_per_env : 0;
+    if (e->dtype == H2O_F32)
+        fluid_accel_sample_kernel<float><<<grid, 256, smem, s>>>(wv, env_args(e), gv, n_envs, e->surface_z,
+                                                                 static_cast<const float*>(points), env_index, m, out);
+    else
+        fluid_accel_sample_kernel<double><<<grid, 256, smem, s>>>(wv, env_args(e), gv, n_envs, e->surface_z,
                                                                   static_cast<const double*>(points), env_index, m, out);
     CUDA_TRY(cudaGetLastError());
     return H2O_OK;
@@ -1281,6 +1333,9 @@ int h2o_set_warp_compat(h2o_handle h, int enable)
 {
     h2o_engine* e = check(h);
     if (!e) return H2O_ERR_BAD_HANDLE;
+    if (enable && e->fluid_inertia)  // checked before the captured rollout is dropped: a refused call leaves it intact
+        return fail(H2O_ERR_NOT_CONFIGURED,
+                    "Warp compatibility has no fluid-inertia loads: turn h2o_set_fluid_inertia off first");
     { DeviceGuard gi(e->device); invalidate_graph(e); }
     e->warp_compat = enable != 0;
     return H2O_OK;
@@ -1622,21 +1677,37 @@ int h2o_rollout_persistent(h2o_handle h, int n_steps, double dt, double gravity,
     const bool env = e->env_cond != nullptr;
     const bool cg = e->grid.vals != nullptr;
     const bool sl = slope_on(e);
+    const bool in = inertia_on(e);
 #define H2O_ROLLOUT(S, ST, ENV, CG, SL)              \
-    if (st == ST && env == ENV && cg == CG && sl == SL) \
+    if (st == ST && env == ENV && cg == CG && sl == SL && !in) \
     rollout_persistent_kernel<S, ST, ENV, CG, SL><<<grid, block, smem, s>>>(a)
 #define H2O_ROLLOUTS(S, SL) \
     H2O_ROLLOUT(S, true, true, false, SL); H2O_ROLLOUT(S, true, false, false, SL);   \
     H2O_ROLLOUT(S, false, true, false, SL); H2O_ROLLOUT(S, false, false, false, SL); \
     H2O_ROLLOUT(S, true, true, true, SL); H2O_ROLLOUT(S, true, false, true, SL);     \
     H2O_ROLLOUT(S, false, true, true, SL); H2O_ROLLOUT(S, false, false, true, SL)
+// the inertia instantiations: only launched with a wave field or a time-varying grid
+#define H2O_ROLLOUT_IN(S, ST, ENV, CG, SL)           \
+    if (st == ST && env == ENV && cg == CG && sl == SL && in) \
+    rollout_persistent_kernel<S, ST, ENV, CG, SL, true><<<grid, block, smem, s>>>(a)
+#define H2O_ROLLOUTS_IN(S, SL) \
+    H2O_ROLLOUT_IN(S, true, true, false, SL); H2O_ROLLOUT_IN(S, true, false, false, SL);   \
+    H2O_ROLLOUT_IN(S, false, true, false, SL); H2O_ROLLOUT_IN(S, false, false, false, SL); \
+    H2O_ROLLOUT_IN(S, true, true, true, SL); H2O_ROLLOUT_IN(S, true, false, true, SL);     \
+    H2O_ROLLOUT_IN(S, false, true, true, SL); H2O_ROLLOUT_IN(S, false, false, true, SL)
     if (e->dtype == H2O_F32) {
         H2O_ROLLOUTS(float, false);
         H2O_ROLLOUTS(float, true);
+        H2O_ROLLOUTS_IN(float, false);
+        H2O_ROLLOUTS_IN(float, true);
     } else {
         H2O_ROLLOUTS(double, false);
         H2O_ROLLOUTS(double, true);
+        H2O_ROLLOUTS_IN(double, false);
+        H2O_ROLLOUTS_IN(double, true);
     }
+#undef H2O_ROLLOUTS_IN
+#undef H2O_ROLLOUT_IN
 #undef H2O_ROLLOUTS
 #undef H2O_ROLLOUT
     CUDA_TRY(cudaGetLastError());

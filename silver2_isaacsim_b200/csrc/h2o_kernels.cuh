@@ -310,12 +310,14 @@ struct ExactStepOut {
     int flags;  // bit 0 clamped, bit 1 still
 };
 // Core (inlined into its noinline carriers below): the fp64-mode arithmetic on one fp32-stored body.  kSlope: the
-// waterline is the tangent plane of slope (sx, sy) (h2o_set_wave_slope).
-template <bool kSlope = false>
+// waterline is the tangent plane of slope (sx, sy) (h2o_set_wave_slope).  kInertia: the fluid-acceleration loads for
+// a_f = (afx, afy, afz) (h2o_set_fluid_inertia).
+template <bool kSlope = false, bool kInertia = false>
 __device__ __forceinline__ ExactStepOut exact_eval_f32(const RawBody<float>& r, const float* c, int quat_wxyz, double rho,
                                                         double grav, double inv_dt, double surface_z, float cx, float cy,
                                                         float cz, const float* am_dense, bool warp_compat = false,
-                                                        double sx = 0.0, double sy = 0.0)
+                                                        double sx = 0.0, double sy = 0.0, double afx = 0.0,
+                                                        double afy = 0.0, double afz = 0.0)
 {
     BodyIn<double, double> g;
     g.pz = double(r.pz) - surface_z;
@@ -341,10 +343,10 @@ __device__ __forceinline__ ExactStepOut exact_eval_f32(const RawBody<float>& r, 
         g.am_dense = md;
     }
     Terms<double, double> t;
-    body_terms<double, double, false, kSlope>(g, t, nullptr, sx, sy);
+    body_terms<double, double, false, kSlope, kInertia>(g, t, nullptr, sx, sy, afx, afy, afz);
     double F[3], T[3];
     bool clamped;
-    net_wrench<double, double>(t, double(c[10]), F, T, clamped);
+    net_wrench<double, double, kInertia>(t, double(c[10]), F, T, clamped);
     ExactStepOut o;
 #pragma unroll
     for (int j = 0; j < 3; ++j) {
@@ -370,6 +372,17 @@ __device__ __noinline__ ExactStepOut body_step_exact_f32_slope(const RawBody<flo
                                                                bool warp_compat = false)
 {
     return exact_eval_f32<true>(r, c, quat_wxyz, rho, grav, inv_dt, surface_z, cx, cy, cz, nullptr, warp_compat, sx, sy);
+}
+// The same with the fluid-acceleration loads for a_f (and the slope when kSlope): carriers of their own, so that kernels
+// without the mode keep their call sites.
+template <bool kSlope>
+__device__ __noinline__ ExactStepOut body_step_exact_f32_inertia(const RawBody<float>& r, const float* c, int quat_wxyz,
+                                                                 double rho, double grav, double inv_dt, double surface_z,
+                                                                 float cx, float cy, float cz, double sx, double sy,
+                                                                 double afx, double afy, double afz)
+{
+    return exact_eval_f32<kSlope, true>(r, c, quat_wxyz, rho, grav, inv_dt, surface_z, cx, cy, cz, nullptr, false, sx, sy,
+                                        afx, afy, afz);
 }
 // Step kernels: re-read the flagged body's inputs from global memory (they are L2-resident: the tile was
 // streamed in microseconds ago), so the hot path keeps no input alive for this.  Scalars cross the call by
@@ -407,6 +420,25 @@ __device__ __noinline__ ExactStepOut body_step_exact_from_global_slope(
     for (int j = 0; j < N_COEFF; ++j) cl[j] = c[j];
     return exact_eval_f32<true>(r, cl, quat_wxyz, rho, grav, inv_dt, surface_z, cx, cy, cz, am_dense, false, sx, sy);
 }
+// The same with the fluid-acceleration loads (step_direct_kernel's inertia instantiations).
+template <int kLayout, int kParam, bool kSlope>
+__device__ __noinline__ ExactStepOut body_step_exact_from_global_inertia(
+    const float* pos, const float* quat, const float* lin, const float* ang, const float* prev, const float* coeff,
+    const int32_t* slot_type, long long i, long long first_body, int n_slots, int quat_wxyz, double rho, double grav,
+    double inv_dt, double surface_z, float cx, float cy, float cz, const float* am_dense, double sx, double sy,
+    double afx, double afy, double afz)
+{
+    BodyPtrs<float> bp;
+    bp.pos = pos; bp.quat = quat; bp.lin = lin; bp.ang = ang; bp.prev = prev; bp.coeff = coeff;
+    RawBody<float> r;
+    load_raw<float, kLayout, false>(bp, i, r);
+    const float* c = coeff + N_COEFF * (kParam == PARAM_PER_BODY ? i : (long long)slot_type[(first_body + i) % n_slots]);
+    float cl[N_COEFF];
+#pragma unroll
+    for (int j = 0; j < N_COEFF; ++j) cl[j] = c[j];
+    return exact_eval_f32<kSlope, true>(r, cl, quat_wxyz, rho, grav, inv_dt, surface_z, cx, cy, cz, am_dense, false, sx,
+                                        sy, afx, afy, afz);
+}
 // prev_row: nullptr = the body's row of a.prev (still the OLD velocities), else a saved copy of that row.
 // surface_z, cx, cy, cz: the waterline and the flow (rounded to float) the fast path saw for this body.
 template <int kLayout, int kParam>
@@ -436,6 +468,18 @@ __device__ __forceinline__ ExactStepOut redo_exact_slope(const StepArgs& a, long
         reinterpret_cast<const float*>(a.pos), reinterpret_cast<const float*>(a.quat), reinterpret_cast<const float*>(a.lin),
         reinterpret_cast<const float*>(a.ang), reinterpret_cast<const float*>(a.prev), reinterpret_cast<const float*>(a.coeff),
         a.slot_type, i, a.first_body, a.n_slots, a.quat_wxyz, a.rho, a.grav, a.inv_dt, surface_z, cx, cy, cz, am, sx, sy);
+}
+template <int kLayout, int kParam, bool kSlope>
+__device__ __forceinline__ ExactStepOut redo_exact_inertia(const StepArgs& a, long long i, double surface_z, float cx,
+                                                           float cy, float cz, double sx, double sy, const double af[3])
+{
+    const float* am = a.am_dense ? reinterpret_cast<const float*>(a.am_dense) + 36 * a.am_slot_type[(a.first_body + i) % a.am_n_slots]
+                                 : nullptr;
+    return body_step_exact_from_global_inertia<kLayout, kParam, kSlope>(
+        reinterpret_cast<const float*>(a.pos), reinterpret_cast<const float*>(a.quat), reinterpret_cast<const float*>(a.lin),
+        reinterpret_cast<const float*>(a.ang), reinterpret_cast<const float*>(a.prev), reinterpret_cast<const float*>(a.coeff),
+        a.slot_type, i, a.first_body, a.n_slots, a.quat_wxyz, a.rho, a.grav, a.inv_dt, surface_z, cx, cy, cz, am, sx, sy,
+        af[0], af[1], af[2]);
 }
 
 // Deferred re-evaluation at the end of a tile-kernel CTA: one saved body per lane, and the float64 model split
@@ -534,20 +578,23 @@ __device__ __noinline__ ExactStepOut combine_roles(const double* p)
 
 // fp32 mode: body-frame fast path (returns true when the body must be re-evaluated, see above);
 // fp64 mode: the world-frame formulation (exact in dq).  kSlope: the tangent-plane waterline of slope (sx, sy).
-template <typename S, bool kWarpSkip = false, bool kSlope = false>
+// kInertia: the fluid-acceleration loads for a_f = af (h2o_set_fluid_inertia).
+template <typename S, bool kWarpSkip = false, bool kSlope = false, bool kInertia = false>
 __device__ __forceinline__ bool body_step(const BodyIn<double, S>& in, S mass, S F[3], S T[3], bool& clamped,
-                                          bool& still, double& ratio, uint32_t& mask, double sx = 0.0, double sy = 0.0)
+                                          bool& still, double& ratio, uint32_t& mask, double sx = 0.0, double sy = 0.0,
+                                          const double* af = nullptr)
 {
+    const double afx = kInertia ? af[0] : 0.0, afy = kInertia ? af[1] : 0.0, afz = kInertia ? af[2] : 0.0;
     if (sizeof(S) == 4) {
         bool suspect;
-        body_wrench_fast<double, S, kWarpSkip, kSlope>(in, mass, F, T, clamped, ratio, still, suspect, mask, nullptr, sx,
-                                                       sy);
+        body_wrench_fast<double, S, kWarpSkip, kSlope, kInertia>(in, mass, F, T, clamped, ratio, still, suspect, mask,
+                                                                 nullptr, sx, sy, afx, afy, afz);
         return suspect;
     } else {
         mask = 0;
         Terms<double, S> t;
-        body_terms<double, S, false, kSlope>(in, t, nullptr, sx, sy);
-        net_wrench<double, S>(t, mass, F, T, clamped);
+        body_terms<double, S, false, kSlope, kInertia>(in, t, nullptr, sx, sy, afx, afy, afz);
+        net_wrench<double, S, kInertia>(t, mass, F, T, clamped);
         ratio = t.ratio;
         still = t.still;
         return false;
@@ -575,20 +622,24 @@ __device__ __forceinline__ void accumulate_stats(ThreadStats& st, double fx, dou
 // re-evaluation; kDefer = false does it on the spot (redo_exact), kDefer = true leaves it to the caller.
 // `i` = body index inside the launch (a.pos etc. are the launch's base pointers).
 // kSlope (direct kernel only, kDefer = false): the tangent-plane waterline of slope (sx, sy), re-evaluation included.
-template <typename S, int kLayout, int kParam, bool kStats, bool kDefer, bool kWarpSkip = false, bool kSlope = false>
+// kInertia (likewise): the fluid-acceleration loads for a_f = af, re-evaluation included.
+template <typename S, int kLayout, int kParam, bool kStats, bool kDefer, bool kWarpSkip = false, bool kSlope = false,
+          bool kInertia = false>
 __device__ __forceinline__ bool step_one_body(const StepArgs& a, long long i, const BodyIn<double, S>& in, S mass,
                                               const Env& env, S F[3], S T[3], ThreadStats& st, uint32_t& mask,
-                                              double sx = 0.0, double sy = 0.0)
+                                              double sx = 0.0, double sy = 0.0, const double* af = nullptr)
 {
     bool clamped, still;
     double ratio;
-    bool redo = body_step<S, kWarpSkip, kSlope>(in, mass, F, T, clamped, still, ratio, mask, sx, sy);
+    bool redo = body_step<S, kWarpSkip, kSlope, kInertia>(in, mass, F, T, clamped, still, ratio, mask, sx, sy, af);
     if (sizeof(S) == 4) {
         redo = redo && a.no_fallback != 1;
         if (a.no_fallback > 1) redo = ((a.first_body + i) & (long long)(a.no_fallback - 1)) == 0;  // study knob: every k-th body, k = 2^j
         if (redo && !kDefer) {
             const ExactStepOut o =
-                kSlope ? redo_exact_slope<kLayout, kParam>(a, i, env.surface_z, float(env.cx), float(env.cy),
+                kInertia ? redo_exact_inertia<kLayout, kParam, kSlope>(a, i, env.surface_z, float(env.cx), float(env.cy),
+                                                                       float(env.cz), sx, sy, af)
+                : kSlope ? redo_exact_slope<kLayout, kParam>(a, i, env.surface_z, float(env.cx), float(env.cy),
                                                            float(env.cz), sx, sy)
                        : redo_exact<kLayout, kParam>(a, i, env.surface_z, float(env.cx), float(env.cy), float(env.cz));
 #pragma unroll
@@ -1062,7 +1113,9 @@ __device__ __forceinline__ void stage_waves(double* dst, const double* tab, cons
 
 // kSlope (h2o_set_wave_slope, launched only with a wave field): every body is tested against the tangent plane of the
 // wave surface at its position (body_terms / body_wrench_fast), on every path below.
-template <typename S, int kLayout, int kParam, bool kStats, bool kSlope = false>
+// kInertia (h2o_set_fluid_inertia, launched only with a wave field or a grid with nt > 1, never with Warp
+// compatibility): the fluid-acceleration loads for the a_f water_at forms at the body centre, on every path below.
+template <typename S, int kLayout, int kParam, bool kStats, bool kSlope = false, bool kInertia = false>
 __global__ void __launch_bounds__(256) step_direct_kernel(const __grid_constant__ StepArgs a, long long body_begin,
                                                           const __grid_constant__ WaveArgs wv,
                                                           const __grid_constant__ EnvArgs ev,
@@ -1108,12 +1161,21 @@ __global__ void __launch_bounds__(256) step_direct_kernel(const __grid_constant_
         BodyIn<double, S> bin;
         Env env{a.current[0], a.current[1], a.current[2], a.surface_z};
         double slope[2] = {0.0, 0.0};
+        double af[3] = {0.0, 0.0, 0.0};
         if (wv.n || ev.cond || gv.vals) {
             EnvRow row{};
             if (ev.cond) row = env_row(ev.cond, (a.first_body + i) / ev.bodies_per_env);
             // the clock: staged with the wave table, else read directly when only the grid needs it
             const double t = wv.n ? wave_smem[wv.n * WAVE_STRIDE] : (gv.vals ? *wv.clock : 0.0);
-            if constexpr (kSlope) {
+            if constexpr (kInertia) {
+                const WaterAccel wa = water_at<sizeof(S) == 4, kSlope, true>(
+                    a.current, a.surface_z, ev.cond != nullptr, row, wave_smem, wv.n, wv.depth, t, double(r.px),
+                    double(r.py), double(r.pz), gv.vals ? &gv : nullptr);
+                env = Env{wa.water.cx, wa.water.cy, wa.water.cz, wa.water.surface_z};
+                slope[0] = wa.sx;
+                slope[1] = wa.sy;
+                af[0] = wa.ax; af[1] = wa.ay; af[2] = wa.az;
+            } else if constexpr (kSlope) {
                 const WaterSlope ws = water_at<sizeof(S) == 4, true>(a.current, a.surface_z, ev.cond != nullptr, row,
                                                                      wave_smem, wv.n, wv.depth, t, double(r.px),
                                                                      double(r.py), double(r.pz), gv.vals ? &gv : nullptr);
@@ -1134,7 +1196,7 @@ __global__ void __launch_bounds__(256) step_direct_kernel(const __grid_constant_
         S F[3], T[3];
         uint32_t kp_mask;
         bin.warp_compat = a.warp_compat != 0;  // fp64 mode: body_terms honours it
-        if (sizeof(S) == 4 && a.warp_compat) {
+        if (!kInertia && sizeof(S) == 4 && a.warp_compat) {
             // fp32 mode, Warp-twin semantics: the float64 world-frame formulation for every body (compatibility
             // mode, not a fast path: body_wrench_fast knows only the Numba semantics)
             RawBody<float> rf;
@@ -1160,8 +1222,8 @@ __global__ void __launch_bounds__(256) step_direct_kernel(const __grid_constant_
             if (kStats) accumulate_stats(st, double(F[0]), double(F[1]), double(F[2]), double(o.ratio), (o.flags & 1) != 0,
                                          (o.flags & 2) != 0, true);
         } else {
-            step_one_body<S, kLayout, kParam, kStats, false, false, kSlope>(a, i, bin, cl[10], env, F, T, st, kp_mask,
-                                                                            slope[0], slope[1]);
+            step_one_body<S, kLayout, kParam, kStats, false, false, kSlope, kInertia>(a, i, bin, cl[10], env, F, T, st,
+                                                                                      kp_mask, slope[0], slope[1], af);
         }
         S* of = reinterpret_cast<S*>(a.out_force) + 3 * i;
         S* ot = reinterpret_cast<S*>(a.out_torque) + 3 * i;
@@ -1400,8 +1462,9 @@ struct RolloutArgs {
 // Dynamic shared memory: wave_smem_bytes(a.waves.n).  kEnv: a.envs.cond is set (a separate instantiation, so that
 // the env row held in registers costs nothing without conditions).  kGrid: a.grid.vals is set (likewise: rollouts
 // without a grid compile as they did before the grid existed).  kSlope: wave-slope submersion (h2o_set_wave_slope),
-// instantiated for rollouts with a wave field only.
-template <typename S, bool kStats, bool kEnv, bool kGrid, bool kSlope = false>
+// instantiated for rollouts with a wave field only.  kInertia: the fluid-acceleration loads (h2o_set_fluid_inertia),
+// launched only with a wave field or a grid with nt > 1.
+template <typename S, bool kStats, bool kEnv, bool kGrid, bool kSlope = false, bool kInertia = false>
 __global__ void rollout_persistent_kernel(const __grid_constant__ RolloutArgs a)
 {
     extern __shared__ double wave_smem[];
@@ -1437,8 +1500,17 @@ __global__ void rollout_persistent_kernel(const __grid_constant__ RolloutArgs a)
         for (int step = 0; step < a.n_steps; ++step) {
             Env env{a.current[0], a.current[1], a.current[2], a.surface_z};
             double slope[2] = {0.0, 0.0};
+            double af[3] = {0.0, 0.0, 0.0};
             if (wv.n || kEnv || kGrid) {
-                if constexpr (kSlope) {
+                if constexpr (kInertia) {
+                    const WaterAccel wa = water_at<sizeof(S) == 4, kSlope, true>(
+                        a.current, a.surface_z, kEnv, row, wave_smem, wv.n, wv.depth, t, double(r.px), double(r.py),
+                        double(r.pz), kGrid ? &a.grid : nullptr);
+                    env = Env{wa.water.cx, wa.water.cy, wa.water.cz, wa.water.surface_z};
+                    slope[0] = wa.sx;
+                    slope[1] = wa.sy;
+                    af[0] = wa.ax; af[1] = wa.ay; af[2] = wa.az;
+                } else if constexpr (kSlope) {
                     const WaterSlope ws = water_at<sizeof(S) == 4, true>(a.current, a.surface_z, kEnv, row, wave_smem,
                                                                          wv.n, wv.depth, t, double(r.px), double(r.py),
                                                                          double(r.pz), kGrid ? &a.grid : nullptr);
@@ -1458,7 +1530,8 @@ __global__ void rollout_persistent_kernel(const __grid_constant__ RolloutArgs a)
             bool clamped, still;
             double ratio;
             uint32_t kp_mask;
-            bool redo = body_step<S, false, kSlope>(bin, cl[10], F, T, clamped, still, ratio, kp_mask, slope[0], slope[1]);
+            bool redo = body_step<S, false, kSlope, kInertia>(bin, cl[10], F, T, clamped, still, ratio, kp_mask, slope[0],
+                                                              slope[1], af);
             if (sizeof(S) == 4) {
                 redo = redo && a.no_fallback != 1;
                 if (redo) {
@@ -1473,7 +1546,11 @@ __global__ void rollout_persistent_kernel(const __grid_constant__ RolloutArgs a)
 #pragma unroll
                     for (int k = 0; k < N_COEFF; ++k) cf[k] = float(cl[k]);
                     const ExactStepOut o =
-                        kSlope ? body_step_exact_f32_slope(rf, cf, a.quat_wxyz, a.rho, a.grav, 1.0 / a.dt, env.surface_z,
+                        kInertia ? body_step_exact_f32_inertia<kSlope>(rf, cf, a.quat_wxyz, a.rho, a.grav, 1.0 / a.dt,
+                                                                      env.surface_z, float(env.cx), float(env.cy),
+                                                                      float(env.cz), slope[0], slope[1], af[0], af[1],
+                                                                      af[2])
+                        : kSlope ? body_step_exact_f32_slope(rf, cf, a.quat_wxyz, a.rho, a.grav, 1.0 / a.dt, env.surface_z,
                                                            float(env.cx), float(env.cy), float(env.cz), slope[0],
                                                            slope[1])
                                : body_step_exact_f32(rf, cf, a.quat_wxyz, a.rho, a.grav, 1.0 / a.dt, env.surface_z,
@@ -1648,6 +1725,41 @@ __global__ void __launch_bounds__(256) water_slope_sample_kernel(const __grid_co
                                                          wv.depth, wave_smem[wv.n * WAVE_STRIDE], double(p[0]),
                                                          double(p[1]), double(p[2]));
     o[0] = ws.sx; o[1] = ws.sy;
+}
+
+// Fluid-acceleration sampling (h2o_fluid_accel_sample): point k -> out row [ax, ay, az], the a_f a step with
+// h2o_set_fluid_inertia on forms at the clock's value (env row of env_index[k] when env_index is set; grid, or
+// nullptr, and waves); an index outside [0, n_envs) gives a NaN row.  Dynamic shared memory: (wv.n * WAVE_STRIDE + 1)
+// doubles.
+template <typename S>
+__global__ void __launch_bounds__(256) fluid_accel_sample_kernel(const __grid_constant__ WaveArgs wv,
+                                                                 const __grid_constant__ EnvArgs ev,
+                                                                 const __grid_constant__ GridArgs gv, long long n_envs,
+                                                                 double surface_z, const S* points,
+                                                                 const int32_t* env_index, long long m, double* out)
+{
+    extern __shared__ double wave_smem[];
+    stage_waves(wave_smem, wv.tab, wv.clock, wv.n);
+    __syncthreads();
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    double* o = out + 3 * i;
+    EnvRow row{};
+    if (env_index) {
+        const long long e = env_index[i];
+        if (e < 0 || e >= n_envs) {
+            o[0] = o[1] = o[2] = __longlong_as_double(0x7ff8000000000000ll);
+            return;
+        }
+        row = env_row(ev.cond, e);
+    }
+    const S* p = points + 3 * i;
+    const double zero[3] = {0.0, 0.0, 0.0};
+    const WaterAccel wa = water_at<sizeof(S) == 4, false, true>(zero, surface_z, env_index != nullptr, row, wave_smem,
+                                                                wv.n, wv.depth, wave_smem[wv.n * WAVE_STRIDE],
+                                                                double(p[0]), double(p[1]), double(p[2]),
+                                                                gv.vals ? &gv : nullptr);
+    o[0] = wa.ax; o[1] = wa.ay; o[2] = wa.az;
 }
 
 // Masked env reset (h2o_reset_envs), one thread per body: the carried [v, omega] of every body of a masked env

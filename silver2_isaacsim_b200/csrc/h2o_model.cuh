@@ -279,6 +279,7 @@ template <typename H, typename L> struct Terms {
     L cob[3];             // centre of buoyancy - p   (body-relative lever arm, world axes)
     L cop[3];             // centre of pressure - p
     L tarm[3];            // (cop - p) x drag force, evaluated without cancellation
+    L ffk[3];             // Froude-Krylov force rho r V a_f at the centre of buoyancy (kInertia only)
     uint32_t kp_mask;     // 27-bit submerged-keypoint mask (diagnostic)
     bool still;           // wet and speed <= 1e-6: the reference raises here (SURVEY.md A.8)
     bool lift_undefined;  // moving, but the flow is along the body z axis: the Numba path returns zero lift
@@ -425,9 +426,12 @@ H2O_HD void slope_rows(H sx, H sy, H qx, H qy, H qz, H qw, H diag_shift, H& e0, 
 // One body, branch-free.  kExactTrig: asin/sin as the reference vs 2d*sqrt(1-d^2).
 // kSlope: the waterline is the local tangent plane of slope (sx, sy) (slope_rows); everything after the waterline
 // uses the real R.
-template <typename H, typename L, bool kExactTrig, bool kSlope = false>
+// kInertia: fluid-acceleration loads for the world-frame fluid acceleration (afx, afy, afz) (h2o_set_fluid_inertia):
+// the added mass sees a - a_f in place of a, and t.ffk holds the Froude-Krylov force rho r V a_f (net_wrench applies
+// it at the centre of buoyancy).
+template <typename H, typename L, bool kExactTrig, bool kSlope = false, bool kInertia = false>
 H2O_HD void body_terms(const BodyIn<H, L>& in, Terms<H, L>& t, const uint32_t* given_mask = nullptr, H sx = H(0),
-                       H sy = H(0))
+                       H sy = H(0), H afx = H(0), H afy = H(0), H afz = H(0))
 {
     // ---- rotation (numba_hydrodynamics.py:14-49).  Row 2 in H for the waterline.
     const H hx2 = in.qx + in.qx, hy2 = in.qy + in.qy, hz2 = in.qz + in.qz;
@@ -603,9 +607,12 @@ H2O_HD void body_terms(const BodyIn<H, L>& in, Terms<H, L>& t, const uint32_t* g
     //      numba_hydrodynamics_wrapper.py:101-112): -R diag(M) R^T acc * ratio
     {
         const bool fwd = in.warp_compat;  // Numba: R^T a (numba_hydrodynamics.py:229-230); Warp twin: R a
-        const L lx = fwd ? r00 * in.ax + r01 * in.ay + r02 * in.az : r00 * in.ax + r10 * in.ay + r20 * in.az;
-        const L ly = fwd ? r10 * in.ax + r11 * in.ay + r12 * in.az : r01 * in.ax + r11 * in.ay + r21 * in.az;
-        const L lz = fwd ? r20 * in.ax + r21 * in.ay + r22 * in.az : r02 * in.ax + r12 * in.ay + r22 * in.az;
+        // kInertia: the fluid-relative acceleration a - a_f
+        const L ax = kInertia ? in.ax - L(afx) : in.ax, ay = kInertia ? in.ay - L(afy) : in.ay,
+                az = kInertia ? in.az - L(afz) : in.az;
+        const L lx = fwd ? r00 * ax + r01 * ay + r02 * az : r00 * ax + r10 * ay + r20 * az;
+        const L ly = fwd ? r10 * ax + r11 * ay + r12 * az : r01 * ax + r11 * ay + r21 * az;
+        const L lz = fwd ? r20 * ax + r21 * ay + r22 * az : r02 * ax + r12 * ay + r22 * az;
         const L gx = fwd ? r00 * in.bx + r01 * in.by + r02 * in.bz : r00 * in.bx + r10 * in.by + r20 * in.bz;
         const L gy = fwd ? r10 * in.bx + r11 * in.by + r12 * in.bz : r01 * in.bx + r11 * in.by + r21 * in.bz;
         const L gz = fwd ? r20 * in.bx + r21 * in.by + r22 * in.bz : r02 * in.bx + r12 * in.by + r22 * in.bz;
@@ -637,23 +644,39 @@ H2O_HD void body_terms(const BodyIn<H, L>& in, Terms<H, L>& t, const uint32_t* g
 
     t.cob[0] = cobx; t.cob[1] = coby; t.cob[2] = cobz;
     t.cop[0] = copx; t.cop[1] = copy; t.cop[2] = copz;
+    if (kInertia) {  // Froude-Krylov: rho r V a_f (0 for a dry body)
+        const L rv = in.rho * (rl * vol);
+        t.ffk[0] = rv * L(afx); t.ffk[1] = rv * L(afy); t.ffk[2] = rv * L(afz);
+    }
 }
 
 // Net wrench + safety clamp (hydrodynamics_behavior.py:212-226).
 // Lever arms are already body-relative, so  (cob - p) x F_b  =  cob_rel x (0,0,fbz).
 // Only F_z mixes the H-precision buoyancy with the L terms.
-template <typename H, typename L>
+// kInertia: the Froude-Krylov force t.ffk joins the force, and (cob - p) x t.ffk the torque, before the clamp.
+template <typename H, typename L, bool kInertia = false>
 H2O_HD void net_wrench(const Terms<H, L>& t, L mass, L F[3], L T[3], bool& clamped)
 {
     F[0] = (t.fd[0] + t.fl[0]) + t.fam[0];
     F[1] = (t.fd[1] + t.fl[1]) + t.fam[1];
-    F[2] = L(t.fbz + H((t.fd[2] + t.fl[2]) + t.fam[2]));
+    if (kInertia) {
+        F[0] = F[0] + t.ffk[0];
+        F[1] = F[1] + t.ffk[1];
+        F[2] = L(t.fbz + H(((t.fd[2] + t.fl[2]) + t.fam[2]) + t.ffk[2]));
+    } else {
+        F[2] = L(t.fbz + H((t.fd[2] + t.fl[2]) + t.fam[2]));
+    }
 
     const L fb = L(t.fbz);
     const L cx = t.cop[0], cy = t.cop[1], cz = t.cop[2];
     T[0] = ((t.cob[1] * fb + t.tarm[0]) + (cy * t.fl[2] - cz * t.fl[1])) + (t.td[0] + t.tam[0]);
     T[1] = ((t.tarm[1] - t.cob[0] * fb) + (cz * t.fl[0] - cx * t.fl[2])) + (t.td[1] + t.tam[1]);
     T[2] = (t.tarm[2] + (cx * t.fl[1] - cy * t.fl[0])) + (t.td[2] + t.tam[2]);
+    if (kInertia) {
+        T[0] = T[0] + (t.cob[1] * t.ffk[2] - t.cob[2] * t.ffk[1]);
+        T[1] = T[1] + (t.cob[2] * t.ffk[0] - t.cob[0] * t.ffk[2]);
+        T[2] = T[2] + (t.cob[0] * t.ffk[1] - t.cob[1] * t.ffk[0]);
+    }
 
     // scale = min(1, m*500 / (|F| + 1e-6)); the division only matters when the clamp bites.
     const L max_force = mass * L(500.0);
@@ -684,10 +707,14 @@ H2O_HD void net_wrench(const Terms<H, L>& t, L mass, L F[3], L T[3], bool& clamp
 // even in fp32 (the cancelling cop x F_d, see body_terms) keeps its first-order dq term.
 // ---------------------------------------------------------------------------
 // kSlope: as body_terms (the tangent-plane waterline of slope (sx, sy)).
-template <typename H, typename L, bool kWarpSkip = false, bool kSlope = false>
+// kInertia: as body_terms (fluid acceleration (afx, afy, afz), world frame).  The isotropic diagonal added mass on a_f
+// and the Froude-Krylov force join the world-frame force as rho r V (1 + C_a) a_f (rho r V a_f with a dense matrix,
+// whose a_f part M [R^T a_f; 0] is formed in the body frame); the Froude-Krylov torque (cob - p) x rho r V R^T a_f is
+// formed in the body frame.  Both groups are counted by the conditioning check.
+template <typename H, typename L, bool kWarpSkip = false, bool kSlope = false, bool kInertia = false>
 H2O_HD void body_wrench_fast(const BodyIn<H, L>& in, L mass, L F[3], L T[3], bool& clamped, H& ratio_out,
                              bool& still, bool& suspect, uint32_t& mask_out, L* diag = nullptr, H sx = H(0),
-                             H sy = H(0))
+                             H sy = H(0), H afx = H(0), H afy = H(0), H afz = H(0))
 {
     // ---- waterline in H (the same function body_terms calls)
     const H hx2 = in.qx + in.qx, hy2 = in.qy + in.qy, hz2 = in.qz + in.qz;
@@ -838,6 +865,15 @@ H2O_HD void body_wrench_fast(const BodyIn<H, L>& in, L mass, L F[3], L T[3], boo
     L ml, ffx, ffy, ffz, tbx, tby, tbz;
     L ai0, ai1, ai2;  // added-inertia torque, body frame
     const L cfx = army * flz - armz * fly, cfy = armz * flx - armx * flz, cfz = armx * fly - army * flx;  // arm x F_l
+    // kInertia: a_f in the world and body frames, rho r V, and the magnitudes of the groups it forms
+    const L afw0 = L(afx), afw1 = L(afy), afw2 = L(afz);
+    L afb0 = L(0), afb1 = L(0), afb2 = L(0), ri = L(0), mfi = L(0), mti = L(0);
+    if (kInertia) {
+        afb0 = r00 * afw0 + r10 * afw1 + r20 * afw2;
+        afb1 = r01 * afw0 + r11 * afw1 + r21 * afw2;
+        afb2 = r02 * afw0 + r12 * afw1 + r22 * afw2;
+        ri = vol * in.rho * rl;
+    }
     if (in.am_dense) {
         const L a6[6] = {r00 * in.ax + r10 * in.ay + r20 * in.az, r01 * in.ax + r11 * in.ay + r21 * in.az,
                          r02 * in.ax + r12 * in.ay + r22 * in.az, bbx, bby, bbz};
@@ -847,6 +883,12 @@ H2O_HD void body_wrench_fast(const BodyIn<H, L>& in, L mass, L F[3], L T[3], boo
             L acc = L(0);
             for (int j = 0; j < 6; ++j) acc += in.am_dense[6 * i + j] * a6[j];
             f6[i] = acc * sc;
+            if (kInertia) {  // M [R^T (a - a_f); R^T alpha]: the a_f part, counted by the conditioning check
+                const L fa = ((in.am_dense[6 * i] * afb0 + in.am_dense[6 * i + 1] * afb1) + in.am_dense[6 * i + 2] * afb2) * rl;
+                f6[i] = f6[i] - fa;
+                if (i < 3) mfi += h2o_abs(fa);
+                else mti += h2o_abs(fa);
+            }
         }
         ml = L(0);
         ffx = flx - f6[0]; ffy = fly - f6[1]; ffz = flz - f6[2];
@@ -863,6 +905,19 @@ H2O_HD void body_wrench_fast(const BodyIn<H, L>& in, L mass, L F[3], L T[3], boo
     tby = psi * tdy + (cfy - ai1);
     tbz = psi * tdz + (cfz - ai2);
     mt += ((h2o_abs(cfx) + h2o_abs(cfy)) + h2o_abs(cfz)) + ((h2o_abs(ai0) + h2o_abs(ai1)) + h2o_abs(ai2));
+    // kInertia, world-frame force coefficient of a_f: Froude-Krylov, plus the isotropic diagonal added mass
+    L kfi = L(0);
+    if (kInertia) {
+        kfi = in.am_dense ? ri : ri * (L(1) + in.c_am);
+        // Froude-Krylov torque, body frame: cob x rho r V R^T a_f
+        const L fk0 = ri * afb0, fk1 = ri * afb1, fk2 = ri * afb2;
+        const L tf0 = cby * fk2 - cbz * fk1, tf1 = cbz * fk0 - cbx * fk2, tf2 = cbx * fk1 - cby * fk0;
+        tbx = tbx + tf0;
+        tby = tby + tf1;
+        tbz = tbz + tf2;
+        mt += ((h2o_abs(tf0) + h2o_abs(tf1)) + h2o_abs(tf2)) + mti;
+        mfi += h2o_abs(kfi) * ((h2o_abs(afw0) + h2o_abs(afw1)) + h2o_abs(afw2));
+    }
 
     // ---- angular drag (world): -(0.5 rho |w| C V + k min(1, 5|w|)) ratio * w
     const L as2 = in.wx * in.wx + in.wy * in.wy + in.wz * in.wz;
@@ -880,7 +935,13 @@ H2O_HD void body_wrench_fast(const BodyIn<H, L>& in, L mass, L F[3], L T[3], boo
     // buoyancy joins in L: its rounding (6e-8 fbz) reaches the bound only where |F| < 0.6 % of fbz, and those
     // bodies are flagged below (|F| < FLAG_KAPPA_F fbz)
     const L fbl = L(fbz);
-    F[2] = fbl + ((r20 * ffx + r21 * ffy + r22 * ffz) - (gam * in.vz + ml * in.az));
+    if (kInertia) {
+        F[0] = F[0] + kfi * afw0;
+        F[1] = F[1] + kfi * afw1;
+        F[2] = fbl + (((r20 * ffx + r21 * ffy + r22 * ffz) - (gam * in.vz + ml * in.az)) + kfi * afw2);
+    } else {
+        F[2] = fbl + ((r20 * ffx + r21 * ffy + r22 * ffz) - (gam * in.vz + ml * in.az));
+    }
 
     // ---- conditioning check.  L arithmetic carries ~1e-7 relative error per TERM; the result meets the
     // fp32-mode bound (1e-5 relative per vector, SURVEY.md 8(d)) unless that error is amplified:
@@ -894,12 +955,14 @@ H2O_HD void body_wrench_fast(const BodyIn<H, L>& in, L mass, L F[3], L T[3], boo
         const L t1 = (h2o_abs(T[0]) + h2o_abs(T[1])) + h2o_abs(T[2]);
         const L f1 = (h2o_abs(F[0]) + h2o_abs(F[1])) + h2o_abs(F[2]);
         // (b): buoyancy is the only force group that does not vanish with the velocities, so a cancelled net
-        // force means |F| << F_buoyancy
-        flag_kt = t1 / h2o_max(mt, L(1e-30)); flag_kf = f1 / h2o_max(fbl, L(1e-30));
+        // force means |F| << F_buoyancy.  kInertia: the fluid-acceleration groups do not vanish with the velocities
+        // either (and cancel drag exactly in the Morison case): |F| << F_buoyancy + their magnitude
+        const L fs = kInertia ? fbl + mfi : fbl;
+        flag_kt = t1 / h2o_max(mt, L(1e-30)); flag_kf = f1 / h2o_max(fs, L(1e-30));
 #if defined(H2O_NO_FLAGS)  // cost experiment only: no conditioning check (the dq check stays)
         suspect = h2o_abs(dqh) > H(FAST_PATH_MAX_DQ);
 #else
-        suspect = (t1 < L(FLAG_KAPPA_T) * mt) | (f1 < L(FLAG_KAPPA_F) * fbl) | (h2o_abs(dqh) > H(FAST_PATH_MAX_DQ));
+        suspect = (t1 < L(FLAG_KAPPA_T) * mt) | (f1 < L(FLAG_KAPPA_F) * fs) | (h2o_abs(dqh) > H(FAST_PATH_MAX_DQ));
 #endif
     }
 

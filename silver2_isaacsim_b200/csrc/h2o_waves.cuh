@@ -38,8 +38,16 @@ struct WaveSlopeSample {
     WaveSample field;
     double sx, sy;
 };
-template <bool kSlope> struct WaveResult { using type = WaveSample; };
-template <> struct WaveResult<true> { using type = WaveSlopeSample; };
+// What an acceleration instantiation (h2o_set_fluid_inertia) returns: the field, the slope (zero without kSlope) and
+// the time derivative (ax, ay, az) of the orbital velocity.
+struct WaveAccelSample {
+    WaveSample field;
+    double sx, sy;
+    double ax, ay, az;
+};
+template <bool kSlope, bool kAccel = false> struct WaveResult { using type = WaveSample; };
+template <> struct WaveResult<true, false> { using type = WaveSlopeSample; };
+template <bool kSlope> struct WaveResult<kSlope, true> { using type = WaveAccelSample; };
 
 // theta is formed with separately rounded products and sums, in the order written above, on every
 // platform (no FMA contraction), so that it is the same double the NumPy reference forms: at t ~ 1e5 s
@@ -90,15 +98,18 @@ H2O_HD void wave_table_row(const double comp[5], double depth, double row[WAVE_S
 // sum a_j omega_j (velocity) of the float64 values (tests/test_waves.py).
 // kSlope: also the surface gradient sum_j -a_j (kx_j, ky_j) sin theta_j, from the same sine as u_z (float in the fp32
 // policy) with float64 sums (WaveSlopeSample).  Without it nothing of the gradient is formed.
-template <bool kF32, bool kSlope = false>
-H2O_HD typename WaveResult<kSlope>::type wave_eval(const double* tab, int n, double depth, double px, double py,
-                                                  double z_rel, double t)
+// kAccel: also the time derivative of the orbital velocity, sum_j a_j omega_j^2 (C_j sin theta_j khat_j,
+// -S_j cos theta_j), from the same sine, cosine and depth decay with float64 sums (WaveAccelSample).
+template <bool kF32, bool kSlope = false, bool kAccel = false>
+H2O_HD typename WaveResult<kSlope, kAccel>::type wave_eval(const double* tab, int n, double depth, double px,
+                                                          double py, double z_rel, double t)
 {
     const bool deep = !(depth < INFINITY);
     double z = z_rel < 0.0 ? z_rel : 0.0;
     if (!deep && z < -depth) z = -depth;
     WaveSample s{0.0, 0.0, 0.0, 0.0};
     double gx = 0.0, gy = 0.0;
+    double dx = 0.0, dy = 0.0, dz = 0.0;
     for (int j = 0; j < n; ++j) {
         const double* c = tab + WAVE_STRIDE * j;
         const double th = wave_add(wave_add(wave_add(wave_mul(c[WAVE_KX], px), wave_mul(c[WAVE_KY], py)),
@@ -135,8 +146,16 @@ H2O_HD typename WaveResult<kSlope>::type wave_eval(const double* tab, int n, dou
             gx -= as * c[WAVE_KX];
             gy -= as * c[WAVE_KY];
         }
+        if constexpr (kAccel) {
+            const double aw2 = c[WAVE_A_OMEGA] * c[WAVE_OMEGA];
+            const double ah = aw2 * C * sn;
+            dx += ah * c[WAVE_KHAT_X];
+            dy += ah * c[WAVE_KHAT_Y];
+            dz -= aw2 * S * cs;
+        }
     }
-    if constexpr (kSlope) return WaveSlopeSample{s, gx, gy};
+    if constexpr (kAccel) return WaveAccelSample{s, gx, gy, dx, dy, dz};
+    else if constexpr (kSlope) return WaveSlopeSample{s, gx, gy};
     else return s;
 }
 
@@ -239,12 +258,18 @@ H2O_HD void grid_xyz(const GridArgs& g, const double* p, double wx, double wy, d
 // The grid's velocity at grid-frame coordinates (X, Y, Z) and time T: multilinear, along x, then y, then z, then t,
 // held at the boundary outside the lattice and before the first / after the last frame.  Any NaN coordinate gives
 // NaN, with no read.
-H2O_HD void grid_eval(const GridArgs& g, double X, double Y, double Z, double T, double v[3])
+// kDiff: also dv = (G_{f+1} - G_f) / ht, the time derivative of the interpolation (G_f, G_{f+1} the spatial
+// interpolations of the two frames it blends), for nt > 1 and T inside [t0, t0 + (nt - 1) ht]; 0 where the grid is
+// held and for nt = 1 (h2o_set_fluid_inertia).
+template <bool kDiff = false>
+H2O_HD void grid_eval(const GridArgs& g, double X, double Y, double Z, double T, double v[3], double* dv = nullptr)
 {
     if (X != X || Y != Y || Z != Z || T != T) {  // NaN
         v[0] = v[1] = v[2] = nan("");
+        if constexpr (kDiff) dv[0] = dv[1] = dv[2] = nan("");
         return;
     }
+    if constexpr (kDiff) dv[0] = dv[1] = dv[2] = 0.0;
     const GridAxis ax = grid_axis(X, g.nx, g.gx, g.hx), ay = grid_axis(Y, g.ny, g.gy, g.hy);
     const GridAxis az = grid_axis(Z, g.nz, g.gz, g.hz), at = grid_axis(T, g.nt, g.t0, g.ht);
     const double* p = g.vals + 3 * (((at.i * g.nz + az.i) * g.ny + ay.i) * g.nx + ax.i);
@@ -252,6 +277,11 @@ H2O_HD void grid_eval(const GridArgs& g, double X, double Y, double Z, double T,
     if (g.nt > 1) {
         double b[3];
         grid_xyz(g, p + 3 * g.nx * g.ny * g.nz, ax.w, ay.w, az.w, b);
+        if constexpr (kDiff) {
+            const double u = wave_div(wave_add(T, -g.t0), g.ht);  // grid_axis's unclamped coordinate
+            if (u >= 0.0 && u <= double(g.nt - 1))
+                for (int c = 0; c < 3; ++c) dv[c] = wave_div(wave_add(b[c], -v[c]), g.ht);
+        }
         grid_lerp(v, b, at.w);
     }
 }
@@ -269,8 +299,18 @@ struct WaterSlope {
     Water water;
     double sx, sy;
 };
-template <bool kSlope> struct WaterResult { using type = Water; };
-template <> struct WaterResult<true> { using type = WaterSlope; };
+// water_at's acceleration instantiation (h2o_set_fluid_inertia): the same, the slope (zero without kSlope) and the
+// fluid acceleration a_f = a_g + s a_w at the body centre (ax, ay, az): a_g the grid's time derivative (grid_eval
+// kDiff), a_w the waves' (wave_eval kAccel).  The global and env currents, dz and a caller height array contribute
+// none; the convective term (u . grad) u is not formed.
+struct WaterAccel {
+    Water water;
+    double sx, sy;
+    double ax, ay, az;
+};
+template <bool kSlope, bool kAccel = false> struct WaterResult { using type = Water; };
+template <> struct WaterResult<true, false> { using type = WaterSlope; };
+template <bool kSlope> struct WaterResult<kSlope, true> { using type = WaterAccel; };
 
 // The one composition of the global environment (current, surface_z), the env row (has_row), the current grid
 // (grid, or nullptr), the wave table and the clock value t for a body at p, used by every step kernel, the samplers
@@ -281,13 +321,15 @@ template <> struct WaterResult<true> { using type = WaterSlope; };
 //   waterline = L + s eta,  flow = ((current + c) + g) + s u.
 // The identity row [0,0,0,0,1,0,0,0] makes each row operation exact, so it reproduces the row-less result bit for
 // bit; a grid of zeros does the same for the grid.
-template <bool kF32, bool kSlope = false>
-H2O_HD typename WaterResult<kSlope>::type water_at(const double current[3], double surface_z, bool has_row,
-                                                   const EnvRow& row, const double* tab, int n_waves, double depth,
-                                                   double t, double px, double py, double pz,
-                                                   const GridArgs* grid = nullptr)
+// kAccel: also a_f = a_g + s a_w (WaterAccel), every operation separately rounded.
+template <bool kF32, bool kSlope = false, bool kAccel = false>
+H2O_HD typename WaterResult<kSlope, kAccel>::type water_at(const double current[3], double surface_z, bool has_row,
+                                                           const EnvRow& row, const double* tab, int n_waves,
+                                                           double depth, double t, double px, double py, double pz,
+                                                           const GridArgs* grid = nullptr)
 {
     double sx = 0.0, sy = 0.0;
+    double ag[3] = {0.0, 0.0, 0.0}, aw[3] = {0.0, 0.0, 0.0};
     Water w{surface_z, current[0], current[1], current[2], {0.0, 0.0, 0.0, 0.0}};
     const double* c = row.c;
     if (has_row) {
@@ -302,13 +344,20 @@ H2O_HD typename WaterResult<kSlope>::type water_at(const double current[3], doub
     const double z_rel = pz - w.surface_z;
     if (grid) {
         double g[3];
-        grid_eval(*grid, px, py, z_rel, t, g);
+        if constexpr (kAccel) grid_eval<true>(*grid, px, py, z_rel, t, g, ag);
+        else grid_eval(*grid, px, py, z_rel, t, g);
         w.cx = wave_add(w.cx, g[0]);
         w.cy = wave_add(w.cy, g[1]);
         w.cz = wave_add(w.cz, g[2]);
     }
     if (n_waves) {
-        if constexpr (kSlope) {
+        if constexpr (kAccel) {
+            const WaveAccelSample wa = wave_eval<kF32, kSlope, true>(tab, n_waves, depth, px, py, z_rel, t);
+            w.field = wa.field;
+            sx = wa.sx;
+            sy = wa.sy;
+            aw[0] = wa.ax; aw[1] = wa.ay; aw[2] = wa.az;
+        } else if constexpr (kSlope) {
             const WaveSlopeSample ws = wave_eval<kF32, true>(tab, n_waves, depth, px, py, z_rel, t);
             w.field = ws.field;
             sx = ws.sx;
@@ -324,13 +373,17 @@ H2O_HD typename WaterResult<kSlope>::type water_at(const double current[3], doub
                 sx = wave_mul(s, sx);
                 sy = wave_mul(s, sy);
             }
+            if constexpr (kAccel)
+                for (int k = 0; k < 3; ++k) aw[k] = wave_mul(s, aw[k]);
         }
         w.surface_z = wave_add(w.surface_z, w.field.eta);
         w.cx = wave_add(w.cx, w.field.ux);
         w.cy = wave_add(w.cy, w.field.uy);
         w.cz = wave_add(w.cz, w.field.uz);
     }
-    if constexpr (kSlope) return WaterSlope{w, sx, sy};
+    if constexpr (kAccel)
+        return WaterAccel{w, sx, sy, wave_add(ag[0], aw[0]), wave_add(ag[1], aw[1]), wave_add(ag[2], aw[2])};
+    else if constexpr (kSlope) return WaterSlope{w, sx, sy};
     else return w;
 }
 

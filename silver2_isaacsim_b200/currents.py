@@ -124,13 +124,25 @@ def evaluate(grid: CurrentGrid, x, y, z, t) -> np.ndarray:
     x, y, z, t = np.broadcast_arrays(*(np.asarray(q, dtype=np.float64).reshape(-1) for q in (x, y, z, t)))
     nan = np.isnan(x) | np.isnan(y) | np.isnan(z) | np.isnan(t)
     x, y, z, t = (np.where(nan, 0.0, q) for q in (x, y, z, t))
+    it, wt = _axis(t, grid.dims[0], grid.t0, grid.frame_dt)
+    along_z = _spatial(grid, x, y, z)
+    out = along_z(it)
+    if grid.dims[0] > 1:
+        out = _lerp(out, along_z(it + 1), wt)
+    out = np.array(out, dtype=np.float64)
+    out[nan] = np.nan
+    return out
+
+
+def _spatial(grid: CurrentGrid, x, y, z):
+    """The spatial interpolation at points x, y, z (without NaN): f -> (m, 3) values of frames f, along x, then y,
+    then z."""
     v = grid.values
-    nt, nz, ny, nx = grid.dims
+    _, nz, ny, nx = grid.dims
     (gx, gy, gz), (hx, hy, hz) = grid.origin, grid.spacing
     ix, wx = _axis(x, nx, gx, hx)
     iy, wy = _axis(y, ny, gy, hy)
     iz, wz = _axis(z, nz, gz, hz)
-    it, wt = _axis(t, nt, grid.t0, grid.frame_dt)
 
     def along_x(f, k, j):
         a = v[f, k, j, ix]
@@ -144,9 +156,26 @@ def evaluate(grid: CurrentGrid, x, y, z, t) -> np.ndarray:
         a = along_y(f, iz)
         return _lerp(a, along_y(f, iz + 1), wz) if nz > 1 else a
 
-    out = along_z(it)
+    return along_z
+
+
+def time_derivative(grid: CurrentGrid, x, y, z, t) -> np.ndarray:
+    """Float64 reference of the grid's time derivative at grid-frame points ``x, y, z`` and times ``t`` (scalars or one
+    value per point): (m, 3) rows ``(G_{f+1} - G_f) / frame_dt``, with ``G_f``, ``G_{f+1}`` the spatial interpolations
+    of the two frames ``evaluate`` blends at ``t``, for ``nt > 1`` and ``t`` inside ``[t0, t0 + (nt - 1) frame_dt]``;
+    zero rows where the grid is held in time and for one frame; NaN rows where a coordinate is NaN (include/h2o.h,
+    h2o_set_fluid_inertia)."""
+    x, y, z, t = np.broadcast_arrays(*(np.asarray(q, dtype=np.float64).reshape(-1) for q in (x, y, z, t)))
+    nan = np.isnan(x) | np.isnan(y) | np.isnan(z) | np.isnan(t)
+    x, y, z, t = (np.where(nan, 0.0, q) for q in (x, y, z, t))
+    out = np.zeros((len(x), 3))
+    nt = grid.dims[0]
     if nt > 1:
-        out = _lerp(out, along_z(it + 1), wt)
-    out = np.array(out, dtype=np.float64)
+        it, _ = _axis(t, nt, grid.t0, grid.frame_dt)
+        u = (t - grid.t0) / grid.frame_dt
+        inside = (u >= 0.0) & (u <= float(nt - 1))
+        along_z = _spatial(grid, x, y, z)
+        out = np.where(inside[:, None], (along_z(it + 1) - along_z(it)) / grid.frame_dt, 0.0)
     out[nan] = np.nan
     return out
+

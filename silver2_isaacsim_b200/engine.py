@@ -76,6 +76,7 @@ class HydroEngine:
         self.quat_order = quat_order
         self._bound = None
         self._wave_slope = False
+        self._fluid_inertia = False
 
     # ------------------------------------------------------------------ lifecycle
     def close(self):
@@ -166,6 +167,37 @@ class HydroEngine:
         out = torch.empty(pts.shape[0], 2, dtype=torch.float64, device=self.device)
         idx = None if env is None else self._env_index(env, pts.shape[0])
         L.check(self._lib.h2o_water_slope_sample(self._h, ctypes.c_void_p(pts.data_ptr()),
+                                                 None if idx is None else ctypes.c_void_p(idx.data_ptr()),
+                                                 int(pts.shape[0]), ctypes.c_void_p(out.data_ptr()),
+                                                 _stream_ptr(self.device)))
+        return out
+
+    def set_fluid_inertia(self, enable: bool = True):
+        """Fluid-acceleration loads: the Froude-Krylov force ``rho r V a_f`` at the centre of buoyancy, and the added
+        mass on the fluid-relative acceleration ``a_b - a_f``, with ``a_f`` the water's acceleration at each body's
+        centre (waves, and a current grid with more than one frame; semantics in include/h2o.h,
+        h2o_set_fluid_inertia).  Off by default; with still water it changes nothing.  Refused with Warp
+        compatibility on (and ``set_warp_compat(True)`` is refused while it is on).  Drops a captured rollout;
+        ``components`` ignores it."""
+        L.check(self._lib.h2o_set_fluid_inertia(self._h, int(bool(enable))))
+        self._fluid_inertia = bool(enable)
+
+    @property
+    def fluid_inertia(self) -> bool:
+        """Whether fluid-acceleration loads are on (``set_fluid_inertia``)."""
+        return self._fluid_inertia
+
+    def sample_fluid_accel(self, points, env=None) -> torch.Tensor:
+        """The fluid acceleration a step uses at ``points`` (m,3) world positions and the current clock: a (m,3)
+        float64 CUDA tensor of rows ``ax, ay, az`` (``waves.acceleration`` plus ``currents.time_derivative``), zeros
+        with the mode off or when nothing accelerates the water.  ``env`` as for ``sample_water``: an index outside
+        ``[0, E)`` gives a NaN row."""
+        pts = self._as_dev(points)
+        if pts.ndim != 2 or pts.shape[1] != 3:
+            raise ValueError(f"points must be (m,3), got {tuple(pts.shape)}")
+        out = torch.empty(pts.shape[0], 3, dtype=torch.float64, device=self.device)
+        idx = None if env is None else self._env_index(env, pts.shape[0])
+        L.check(self._lib.h2o_fluid_accel_sample(self._h, ctypes.c_void_p(pts.data_ptr()),
                                                  None if idx is None else ctypes.c_void_p(idx.data_ptr()),
                                                  int(pts.shape[0]), ctypes.c_void_p(out.data_ptr()),
                                                  _stream_ptr(self.device)))

@@ -167,6 +167,35 @@ def slope(field: WaveField, points, t) -> np.ndarray:
     return out
 
 
+def acceleration(field: WaveField, points, t, surface_z=0.0) -> np.ndarray:
+    """Float64 reference of the water's acceleration at ``points`` (m, 3) and clock ``t``: (m, 3) rows ``ax, ay, az``,
+    the time derivative of ``evaluate``'s orbital velocity, ``sum_j a_j omega_j^2 (C_j sin theta_j khat_j,
+    -S_j cos theta_j)`` with the ``theta_j``, ``C_j``, ``S_j`` and depth clamp of ``evaluate`` (include/h2o.h,
+    h2o_set_fluid_inertia).  ``t`` and ``surface_z`` are scalars or one value per point."""
+    p = np.asarray(points, dtype=np.float64).reshape(-1, 3)
+    t, surface_z = _per_point(t, len(p)), _per_point(surface_z, len(p))
+    c = field.components
+    a, kx, ky, w, ph = (c[:, j][None, :] for j in range(5))
+    k = np.hypot(kx, ky)
+    h = field.depth
+    z = np.minimum(p[:, 2:3] - surface_z, 0.0)
+    if math.isinf(h):
+        C = S = np.exp(k * z)
+    else:
+        z = np.maximum(z, -h)
+        inv = -1.0 / np.expm1(-2.0 * k * h)
+        e0, e1 = np.exp(k * z), np.exp(-k * (z + 2.0 * h))
+        C, S = (e0 + e1) * inv, (e0 - e1) * inv
+    th = ((kx * p[:, 0:1] + ky * p[:, 1:2]) - w * t) + ph
+    aw2 = (a * w) * w
+    ah = aw2 * C * np.sin(th)
+    out = np.empty((len(p), 3))
+    out[:, 0] = (ah * (kx / k)).sum(axis=1)
+    out[:, 1] = (ah * (ky / k)).sum(axis=1)
+    out[:, 2] = -(aw2 * S * np.cos(th)).sum(axis=1)
+    return out
+
+
 # Columns of a per-env conditions row (HydroEngine.set_env_conditions, h2o_set_env_conditions)
 COND_CX, COND_CY, COND_CZ, COND_DZ, COND_SCALE, COND_TAU, COND_X0, COND_Y0 = range(8)
 COND_COLS = 8
@@ -234,3 +263,20 @@ def slope_env(field: WaveField, points, t: float, cond, env_index) -> np.ndarray
     p[:, 0] = p[:, 0] - r[:, COND_X0]
     p[:, 1] = p[:, 1] - r[:, COND_Y0]
     return r[:, COND_SCALE:COND_SCALE + 1] * slope(field, p, t + r[:, COND_TAU])
+
+
+def acceleration_env(field: WaveField, points, t: float, cond, env_index, surface_z: float = 0.0) -> np.ndarray:
+    """Float64 reference of the water's acceleration env ``env_index[k]`` sees at ``points[k]`` and clock ``t``:
+    ``s * acceleration(field, p - origin, t + tau, surface_z + dz)`` with the env's row of ``cond`` (E, 8), as
+    ``evaluate_env`` forms it."""
+    p = np.array(points, dtype=np.float64).reshape(-1, 3)
+    cond = np.asarray(cond, dtype=np.float64)
+    if cond.ndim != 2 or cond.shape[1] != COND_COLS:
+        raise ValueError(f"cond must be (E, {COND_COLS}), got {cond.shape}")
+    r = cond[np.asarray(env_index, dtype=np.int64).reshape(-1)]
+    if len(r) != len(p):
+        raise ValueError("need one env index per point")
+    p[:, 0] = p[:, 0] - r[:, COND_X0]
+    p[:, 1] = p[:, 1] - r[:, COND_Y0]
+    out = acceleration(field, p, t + r[:, COND_TAU], surface_z + r[:, COND_DZ])
+    return r[:, COND_SCALE:COND_SCALE + 1] * out
